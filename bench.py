@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/s of the batched StrikeForce tick on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload = "squad5v5"): Squad 5v5 with NPC spawns under the reference's
@@ -195,6 +195,31 @@ def load_peaks():
     return 6650.0, "fallback (B200_PROFILING.md)"
 
 
+DUMP_LIMIT = 64 * 10 ** 6 - 4096  # array bytes of --dump-outputs: under 64 MB with the .npy headers
+
+
+def step_outputs(sim):
+    """What the caller of sim.step reads back after a step, on the host as float64 (exact for int32 and
+    for each uint32 half of the 64-bit state hash): per arena its sf_step_out row and its state hash.
+    Arenas beyond DUMP_LIMIT are sampled with a fixed seed; `env_ids` says which ones were kept."""
+    import numpy as np
+    n = sim.n_envs
+    keep = np.arange(n)
+    per_row = (1 + 8 + 2) * 8
+    if n * per_row > DUMP_LIMIT:
+        keep = np.sort(np.random.default_rng(0).choice(n, DUMP_LIMIT // per_row, replace=False))
+    out = sim.step_out().cpu().numpy()[keep]
+    h = sim.state_hash().cpu().numpy()[keep].view(np.uint32).reshape(-1, 2)  # little-endian: low half first
+    return {"env_ids": keep.astype(np.float64), "step_out": out.astype(np.float64), "state_hash_lo_hi": h.astype(np.float64)}
+
+
+def write_outputs(directory, arrays):
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -260,6 +285,7 @@ def run_ours(args):
     ms_dev = e0.elapsed_time(e1)
     launches = sim.launches - l0
     st1 = sim.stats_tensor().clone()
+    dumped = step_outputs(sim) if args.dump_outputs and rank == 0 else None  # the last timed step's results
     t += K
     # ---- end-to-end timing: host actions in, step results out, every step
     acts_h = [a.cpu().pin_memory() for a in
@@ -381,6 +407,8 @@ def run_ours(args):
                                  "traffic": load_traffic("sf_observe_kernel_nhwc", E)}}}
         if world == 1 and not args.no_cpu:
             line["cpu_baseline"] = cpu_reference(args.cpu_steps, overhead=True)
+        if dumped is not None:
+            write_outputs(args.dump_outputs, dumped)
         print(json.dumps(line))
     sim.close()
     if world > 1:
@@ -572,7 +600,12 @@ def main():
     ap.add_argument("--strict-fp32", action="store_true", help="royale16: convolutions without TF32 (8x slower)")
     ap.add_argument("--nchw", action="store_true", help="royale16: observations in the reference's [32][31][31] layout "
                                                         "(default: channel innermost, SF_OBS_NHWC)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="squad5v5: after the timed steps, write what the last one computed (rank 0's sf_step_out rows "
+                         "and state hashes) as DIR/<name>.npy, float64")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "squad5v5"):
+        ap.error("--dump-outputs records the squad5v5 workload of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "royale16":

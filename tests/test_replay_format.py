@@ -10,12 +10,13 @@ import sfref
 from strikeforce_b200 import config as sfcfg
 from strikeforce_b200 import replay
 
-pytestmark = pytest.mark.skipif(not sfref.available(), reason="oracle/_ref/libsfref.so not built")
+needs_reference = pytest.mark.skipif(not sfref.available(), reason="oracle/_ref/libsfref.so not built")
 
 CAPS = [sfcfg.DEFAULT_CAPS[k] for k in ("cap_humans", "cap_zombies", "cap_bullets", "cap_chests", "cap_built",
                                         "cap_portals")]
 
 
+@needs_reference
 def test_writer_matches_the_reference_logger(arena_data, tmp_path):
     """The reference logs a Solo match; our writer reproduces the file byte for byte, our reader
     recovers seeds, sheet and commands."""
@@ -36,6 +37,7 @@ def test_writer_matches_the_reference_logger(arena_data, tmp_path):
     assert (log.sheet == replay.logged_sheet(arena_data.player_sheet("account1"))).all()
 
 
+@needs_reference
 @pytest.mark.parametrize("mode,level,agents", [(sfcfg.MODE_SOLO, 1, False), (sfcfg.MODE_SQUAD, 2, True)])
 def test_reference_replays_our_file_like_the_oracle(arena_data, tmp_path, mode, level, agents):
     """A file written by us is replayed by the reference's own reader; the oracle, fed by our reader,
