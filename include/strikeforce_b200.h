@@ -173,7 +173,11 @@ int sf_step(sf_handle *h, const uint8_t *actions, void *stream);
    sf_step_b that closes the first is SF_ERR_ARG), for callers that need the P2 observation point
    (get_command -> bot() inside human_action, gameplay.hpp:933): sf_step_a runs the spawns and
    half-tick A (gameplay.hpp:1444-1461), sf_observe(..., SF_OBS_P2, ...) then sees what the
-   squad agents see, and sf_step_b applies the actions and runs half-tick B (:1462-1471). */
+   squad agents see, and sf_step_b applies the actions and runs half-tick B (:1462-1471).
+   sf_step_a then sf_step_b leaves every arena, its sf_step_out and the statistics exactly as sf_step
+   would.  An arena whose episode ends in half A (SF_OVERFLOW, SF_UB_GUARD) keeps its terminal status
+   until sf_step_b, which reports it and, with auto_reset, resets the arena at its end; its P2
+   observation is undefined, as is the state after any abort. */
 int sf_step_a(sf_handle *h, void *stream);
 int sf_step_b(sf_handle *h, const uint8_t *actions, void *stream);
 

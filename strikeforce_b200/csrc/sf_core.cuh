@@ -1731,6 +1731,10 @@ SF_FN void sf_step_body(const SfDev &d, const SfConst &k, const SfTabs &t, int e
         d.out[env] = o;
         if (d.out_mirror) d.out_mirror[env] = o; /* straight into the caller's host buffer, no copy afterwards */
     }
+    /* Auto-reset happens at the end of the whole step: an episode that ends in half A (an overflow or
+       guard abort) is stored as it ended, half B runs on it with nothing to do, keeps its terminal status
+       in d.out and resets it.  With auto-reset no arena waits for sf_reset, so an arena that is terminal
+       when half B starts ended in this step's half A. */
     bool reset = false;
     if (was_on) {
         sd.kills += e.kills - d.kills[env], sd.tkills += e.tkills - d.tkills[env], sd.loot += e.loot - d.loot[env];
@@ -1743,9 +1747,11 @@ SF_FN void sf_step_body(const SfDev &d, const SfConst &k, const SfTabs &t, int e
             sd.wins += e.status == SF_WIN, sd.deaths += e.status == SF_DEAD, sd.timeouts += e.status == SF_TIMEOUT;
             sd.truncated += e.status == SF_TRUNCATED, sd.overflows += e.status == SF_OVERFLOW;
             sd.ub_guards += e.status == SF_UB_GUARD;
-            reset = k.auto_reset != 0;
+            reset = k.auto_reset != 0 && half != SF_HALF_A;
         }
         if (!reset) sf_store_env(d, env, e);
+    } else if (half == SF_HALF_B && valid && k.auto_reset != 0 && e.status != SF_RUNNING) {
+        reset = true;
     }
     if (reset) { /* new behaviour (SURVEY 7.4#10): next episode of the synthetic seed chain */
         e.episode += 1;
