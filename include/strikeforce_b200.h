@@ -208,6 +208,46 @@ int sf_get(sf_handle *h, int32_t field, void *dev_out, void *stream);
    on entry, count on exit.  Synchronises. */
 int sf_export_env(sf_handle *h, int32_t env, int32_t *host_buf, int64_t *n_inout);
 
+/* Arena records: save arenas into a device buffer and put them back later, into the same handle or another
+   one (search and branching, checkpoint and resume, rewind).  A record holds every per-arena word of the
+   device state at the handle's full capacities -- pending random stream, both banks of the stream
+   constants, dead slots, overlay hints and spill bits included -- behind a 64-byte header (magic, format
+   version, record size, a fingerprint of the configuration, the global id env_id_base + env of the arena it
+   was saved from).  The fingerprint covers what gives the state words their meaning (map geometry,
+   capacities, mode, squad_agents, Battle Royale players and ind, templates and item tables, the static map);
+   n_envs, env_id_base, auto_reset, max_steps and the level range are not part of it.  A record does not
+   hold the handle's SF_STAT_* statistics: they stay sums over the steps this handle ran since sf_create.
+   A checkpoint on disk is the records copied to the host as they are.
+
+   Loading a record into an arena of the same global id (in any handle with the same fingerprint) restores
+   it completely: it plays on exactly as its source would have, current episode, auto-resets and later
+   episodes.  Loaded into another global id (a clone), the current episode goes on bit for bit, with the
+   record's level and episode counter, but the seed chain stays with the slot: the pending stream is seeded
+   again with the synthetic seeds (sf_synth.h) of the slot's global id for episode + 1, and from the next reset on the arena follows its own id's
+   level and seeds, as if its previous episode had ended there (that first reset may finish the stream's
+   warm-up in one go, as after sf_reset).  sf_observe, sf_get and sf_export_env of a loaded arena give what
+   they gave for its source when it was saved, and sf_save of it gives back the loaded bytes (but for the
+   header's global id after a clone).
+
+   Host id arrays are checked on the host and staged in the handle; both calls synchronise before they
+   return, and both are SF_ERR_ARG between sf_step_a and sf_step_b. */
+
+/* bytes of one arena record of this handle (a multiple of 128; fixed for a given library build and
+   configuration) */
+int64_t sf_snapshot_bytes(const sf_handle *h);
+
+/* Write the records of arenas env_ids[0..n) (HOST array; NULL = all n_envs in order, n ignored; at most n_envs
+   entries) into the DEVICE buffer records, [n][sf_snapshot_bytes], 16-byte aligned.  Duplicate ids are
+   allowed. */
+int sf_save(sf_handle *h, const int32_t *env_ids, int32_t n, void *records, void *stream);
+
+/* Overwrite arenas env_ids[i] (HOST array; NULL = all n_envs in order) with record rows[i] (HOST array; NULL =
+   row i) of the DEVICE buffer records ([n_records][sf_snapshot_bytes], 16-byte aligned).  Destination ids must
+   be distinct.  All or nothing: if any referenced record is not a record of a compatible handle (magic,
+   version, size, fingerprint), no arena changes and the call returns SF_ERR_ARG. */
+int sf_load(sf_handle *h, const int32_t *env_ids, int32_t n, const void *records, int32_t n_records,
+            const int32_t *rows, void *stream);
+
 /* Replaces Random::_srand + Random::_rand (random.hpp:54-76) for a batch of independent
    streams: seeds stream i with (tb[i], serial[i]) and writes n_draws outputs per stream into
    the HOST buffer out_host[draw * n_streams + i].  Known-answer tests use it. */

@@ -21,6 +21,7 @@
 #include "sf_core.cuh"
 #include "sf_host_setup.h"
 #include "sf_obs.cuh"
+#include "sf_snapshot.cuh"
 
 #ifndef SF_CTA
 #define SF_CTA 896 /* threads per CTA = arenas in flight per SM (one CTA per SM); 28 warps x 148 SMs = 4144 >= the 4096 chunks of 131072 arenas, 72 registers per thread */
@@ -472,6 +473,162 @@ sf_rng_kernel(const SfDev d, const int64_t *tb, const int64_t *serial, int n_str
     }
 }
 
+/* sf_save / sf_load: arena records (sf_snapshot.cuh) to and from a device buffer.
+ *
+ * A pure HBM copy.  The list is cut into tiles of 32 entries and each (tile, work item of the layout) pair
+ * is one turn of a CTA, so even a short list keeps every SM busy.  A block item (overlay, built list,
+ * sf_step_out) is a straight 16-byte (8-byte for an odd built-list tail) vector copy of each arena's
+ * contiguous bytes.  A SoA item covers consecutive [slot][E] sections: row s of the tile's 32 arenas is
+ * read with one lane per arena (coalesced when the ids are consecutive, as in the all-arenas case; scattered
+ * otherwise, by the same code), transposed through shared memory into each arena's contiguous run of the
+ * record, and that run written with vector stores.  A load runs the same steps backwards.  Record-side
+ * stores of a save and record-side loads of a load are streaming (.cs): the records are not read again
+ * soon, the state is. */
+#define SF_SNAP_CTA 256
+#define SF_SNAP_CTAS_PER_SM 8
+#define SF_SNAP_STAGE (SF_SNAP_TILE * (SF_SNAP_STAGE_RUN + 16))
+
+/* stage stride of a run of P bytes per arena: an odd number of 16-byte chunks, so that the arenas of a row
+   do not all fall into the same shared-memory banks */
+__device__ __forceinline__ uint32_t sf_snap_stride(uint32_t P) { return ((P >> 4) | 1u) << 4; }
+
+/* row-by-row transpose of one SoA section between the arenas' columns in the state and the stage */
+template <bool SAVE, class T>
+__device__ __forceinline__ void sf_snap_soa(const SfSnapSeg &g, int E, uint8_t *st, uint32_t S, int nv, const int *s_env)
+{
+    T *dev = reinterpret_cast<T *>(g.dev);
+    /* a save also writes the zero padding at the end of the section (rows beyond g.rows) */
+    const int rows = SAVE ? (int)(sf_snap_seg_bytes(g) / sizeof(T)) : (int)g.rows;
+#pragma unroll 4
+    for (int q = threadIdx.x; q < rows * SF_SNAP_TILE; q += SF_SNAP_CTA) {
+        const int r = q >> 5, j = q & 31;
+        if (j >= nv) continue;
+        T *s = reinterpret_cast<T *>(st + (size_t)j * S) + r;
+        if (SAVE) *s = r < (int)g.rows ? __ldg(dev + (size_t)r * E + s_env[j]) : T(0);
+        else dev[(size_t)r * E + s_env[j]] = *s;
+    }
+}
+
+/* bytes [lo, hi) of the per-arena block g for the tile's arenas; bytes at or beyond g.elem are the record's
+   padding (written as zeros by a save, skipped by a load) */
+template <bool SAVE, class V>
+__device__ __forceinline__ void sf_snap_block(const SfSnapSeg &g, uint32_t lo, uint32_t hi, uint8_t *records, int nv,
+                                              const int *s_env, const size_t *s_rec)
+{
+    const int per = (int)((hi - lo) / sizeof(V));
+    auto one = [&](int j, int c) {
+        const uint32_t b = lo + (uint32_t)c * (uint32_t)sizeof(V);
+        V *dev = reinterpret_cast<V *>(g.dev + (size_t)s_env[j] * g.elem + b);
+        V *rec = reinterpret_cast<V *>(records + s_rec[j] + g.off + b);
+        if (SAVE) {
+            V v;
+            if (b < g.elem) v = __ldg(dev);
+            else memset(&v, 0, sizeof v);
+            __stcs(rec, v);
+        } else if (b < g.elem) {
+            *dev = __ldcs(rec);
+        }
+    };
+    if (per >= SF_SNAP_CTA) { /* large blocks: the CTA walks one arena at a time, fully coalesced */
+#pragma unroll 4
+        for (int j = 0; j < nv; ++j)
+            for (int c = threadIdx.x; c < per; c += SF_SNAP_CTA) one(j, c);
+    } else {
+        for (int q = threadIdx.x; q < nv * per; q += SF_SNAP_CTA) one(q / per, q % per);
+    }
+}
+
+/* SAVE: records[i] = arena ids[i] (ids NULL: arena i).  LOAD: arena ids[i] = records[rows[i]] (rows NULL:
+   row i), unless sf_snap_check_kernel refused a referenced record. */
+template <bool SAVE>
+__global__ void __launch_bounds__(SF_SNAP_CTA)
+sf_snap_kernel(const __grid_constant__ SfSnapLayout L, int64_t env_id_base, const int32_t *__restrict__ ids, int n,
+               uint8_t *records, const int32_t *__restrict__ rows, const int *refused)
+{
+    __shared__ __align__(16) uint8_t stage[SF_SNAP_STAGE];
+    __shared__ int s_env[SF_SNAP_TILE];
+    __shared__ size_t s_rec[SF_SNAP_TILE]; /* byte offset of the entry's record */
+    if (!SAVE && *reinterpret_cast<const volatile int *>(refused)) return;
+    const long n_work = (long)((n + SF_SNAP_TILE - 1) / SF_SNAP_TILE) * L.n_item;
+    for (long w = blockIdx.x; w < n_work; w += gridDim.x) {
+        const int tile = (int)(w / L.n_item), item = (int)(w % L.n_item);
+        const SfSnapItem it = L.item[item];
+        const int nv = min(SF_SNAP_TILE, n - tile * SF_SNAP_TILE);
+        __syncthreads(); /* the last turn is done with the stage and the entry table */
+        if (threadIdx.x < nv) {
+            const int i = tile * SF_SNAP_TILE + threadIdx.x;
+            s_env[threadIdx.x] = ids ? ids[i] : i;
+            s_rec[threadIdx.x] = (size_t)(SAVE || !rows ? i : rows[i]) * L.bytes;
+        }
+        __syncthreads();
+        if (it.first >= L.n_soa) {
+            const SfSnapSeg &g = L.seg[it.first];
+            const uint32_t hi = it.hi == g.elem ? sf_snap_end(L, it.first) - g.off : it.hi; /* the last piece covers the padding */
+            if (g.elem % 16 == 0) sf_snap_block<SAVE, uint4>(g, it.lo, hi, records, nv, s_env, s_rec);
+            else sf_snap_block<SAVE, uint2>(g, it.lo, hi, records, nv, s_env, s_rec);
+            continue;
+        }
+        const uint32_t lo = L.seg[it.first].off;
+        const uint32_t P = sf_snap_end(L, it.last - 1) - lo, S = sf_snap_stride(P);
+        const int chunks = (int)(P / 16);
+        if (!SAVE) {
+            for (int q = threadIdx.x; q < nv * chunks; q += SF_SNAP_CTA) {
+                const int j = q / chunks, c = q - j * chunks;
+                *reinterpret_cast<uint4 *>(stage + (size_t)j * S + 16 * c) =
+                    __ldcs(reinterpret_cast<const uint4 *>(records + s_rec[j] + lo + 16 * c));
+            }
+            __syncthreads();
+        }
+        for (int s = it.first; s < it.last; ++s) {
+            const SfSnapSeg &g = L.seg[s];
+            uint8_t *st = stage + (g.off - lo);
+            switch (g.elem) {
+            case 1: sf_snap_soa<SAVE, uint8_t>(g, L.E, st, S, nv, s_env); break;
+            case 2: sf_snap_soa<SAVE, uint16_t>(g, L.E, st, S, nv, s_env); break;
+            case 4: sf_snap_soa<SAVE, uint32_t>(g, L.E, st, S, nv, s_env); break;
+            default: sf_snap_soa<SAVE, unsigned long long>(g, L.E, st, S, nv, s_env); break;
+            }
+        }
+        if (SAVE) {
+            __syncthreads();
+            for (int q = threadIdx.x; q < nv * chunks; q += SF_SNAP_CTA) {
+                const int j = q / chunks, c = q - j * chunks;
+                __stcs(reinterpret_cast<uint4 *>(records + s_rec[j] + lo + 16 * c),
+                       *reinterpret_cast<const uint4 *>(stage + (size_t)j * S + 16 * c));
+            }
+            if (item == 0 && threadIdx.x < 4 * nv) { /* the header, 4 chunks per record */
+                const int j = threadIdx.x >> 2, c = threadIdx.x & 3;
+                const int64_t ge = env_id_base + s_env[j];
+                __stcs(reinterpret_cast<uint4 *>(records + s_rec[j]) + c,
+                       make_uint4(sf_snap_header_word(L, ge, 4 * c), sf_snap_header_word(L, ge, 4 * c + 1),
+                                  sf_snap_header_word(L, ge, 4 * c + 2), sf_snap_header_word(L, ge, 4 * c + 3)));
+            }
+        }
+    }
+}
+
+/* magic, version, size and fingerprint of every record a load references */
+__global__ void sf_snap_check_kernel(const __grid_constant__ SfSnapLayout L, const uint8_t *records, const int32_t *rows,
+                                     int n, int *refused)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t *w = reinterpret_cast<const uint32_t *>(records + (size_t)(rows ? rows[i] : i) * L.bytes);
+    if (!sf_snap_compatible(w, L)) atomicOr(refused, 1);
+}
+
+/* after the copy: the pending stream of every arena that took a record of another global id */
+__global__ void sf_snap_reseed_kernel(const SfDev d, const __grid_constant__ SfConst k, const uint8_t *records, uint32_t bytes,
+                                      const int32_t *ids, const int32_t *rows, int n, const int *refused)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n || *refused) return;
+    SfTabs t;
+    sf_global_tabs(d, t);
+    const uint32_t *w = reinterpret_cast<const uint32_t *>(records + (size_t)(rows ? rows[i] : i) * bytes);
+    sf_snap_reseed(d, k, t, ids ? ids[i] : i, sf_snap_global_id(w));
+}
+
 /* ====================================================================== host side */
 
 struct sf_handle {
@@ -486,6 +643,9 @@ struct sf_handle {
     long long *d_export_n = nullptr;
     int32_t *d_ids = nullptr;
     int64_t *d_tb = nullptr, *d_serial = nullptr;
+    int32_t *d_rows = nullptr;   /* sf_load: record row of each entry */
+    int *d_refused = nullptr;    /* sf_load: set when a referenced record is not one of this configuration */
+    SfSnapLayout snap;           /* the record layout of sf_save / sf_load (sf_snapshot.cuh) */
     int device = 0, n_sm = 0;
     bool between_halves = false; /* sf_step_a has run, sf_step_b has not: the P2 observation point */
     int lanes_per_warp = 0;      /* 0 = chosen from the batch size; SF_LANES_PER_WARP overrides (measurements) */
@@ -585,6 +745,7 @@ void carve(Carver &c, sf_handle &h)
     c.take(h.d_export, (size_t)SF_EXPORT_CAP);
     c.take(h.d_export_n, (size_t)1);
     c.take(h.d_ids, E), c.take(h.d_tb, E), c.take(h.d_serial, E);
+    c.take(h.d_rows, E), c.take(h.d_refused, (size_t)1);
 }
 } // namespace
 
@@ -659,6 +820,7 @@ int sf_create(const sf_config *cfg, sf_handle **out)
     Carver placer;
     placer.base = static_cast<uint8_t *>(h->arena);
     carve(placer, *h);
+    sf_snap_layout(h->d, h->k, sf_snap_fingerprint(h->k, h->tabs.smap.data(), h->d.cap_t), h->snap);
 #define SF_CREATE_CUDA(call)                                                        \
     do {                                                                            \
         cudaError_t e_ = (call);                                                    \
@@ -937,6 +1099,81 @@ int sf_rng_stream(sf_handle *h, const int64_t *tb, const int64_t *serial, int32_
     h->launches += 1;
     SF_CUDA(h, cudaGetLastError());
     SF_CUDA(h, cudaMemcpy(out_host, d_out, n_out * 4, cudaMemcpyDeviceToHost));
+    return SF_OK;
+}
+
+int64_t sf_snapshot_bytes(const sf_handle *h) { return h ? (int64_t)h->snap.bytes : 0; }
+
+/* the checks sf_save and sf_load share; stages the arena ids in d_ids */
+static int sf_snap_args(sf_handle *h, const char *fn, const int32_t *env_ids, int32_t &n, const void *records,
+                        bool distinct, cudaStream_t s)
+{
+    if (!records) return sf_fail(h, SF_ERR_ARG, std::string(fn) + ": null record buffer");
+    if (h->between_halves) return sf_fail(h, SF_ERR_ARG, std::string(fn) + ": the step opened by sf_step_a is still waiting for sf_step_b");
+    if (reinterpret_cast<uintptr_t>(records) & 15u) return sf_fail(h, SF_ERR_ARG, std::string(fn) + ": records must be 16-byte aligned");
+    if (!env_ids) n = h->d.n_envs;
+    if (n <= 0 || n > h->d.n_envs) return sf_fail(h, SF_ERR_ARG, std::string(fn) + ": bad arena count");
+    if (env_ids) {
+        std::vector<uint8_t> seen(distinct ? (size_t)h->d.n_envs : 0, 0);
+        for (int i = 0; i < n; ++i) {
+            if (env_ids[i] < 0 || env_ids[i] >= h->d.n_envs) return sf_fail(h, SF_ERR_ARG, std::string(fn) + ": arena id out of range");
+            if (distinct && seen[env_ids[i]]++) return sf_fail(h, SF_ERR_ARG, std::string(fn) + ": duplicate destination arena");
+        }
+        SF_CUDA(h, cudaMemcpyAsync(h->d_ids, env_ids, (size_t)n * 4, cudaMemcpyHostToDevice, s));
+    }
+    return SF_OK;
+}
+
+static int sf_snap_grid(const sf_handle *h, int n)
+{
+    const long work = (long)((n + SF_SNAP_TILE - 1) / SF_SNAP_TILE) * h->snap.n_item;
+    const long cap = (long)h->n_sm * SF_SNAP_CTAS_PER_SM;
+    return (int)(work < cap ? work : cap);
+}
+
+int sf_save(sf_handle *h, const int32_t *env_ids, int32_t n, void *records, void *stream)
+{
+    if (!h) return SF_ERR_ARG;
+    SfDeviceGuard guard(h);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    int rc = sf_snap_args(h, "sf_save", env_ids, n, records, false, s);
+    if (rc) return rc;
+    sf_snap_kernel<true><<<sf_snap_grid(h, n), SF_SNAP_CTA, 0, s>>>(h->snap, h->k.env_id_base, env_ids ? h->d_ids : nullptr, n,
+                                                                   static_cast<uint8_t *>(records), nullptr, nullptr);
+    h->launches += 1;
+    SF_CUDA(h, cudaGetLastError());
+    SF_CUDA(h, cudaStreamSynchronize(s)); /* the staging buffers are reused by the next call */
+    return SF_OK;
+}
+
+int sf_load(sf_handle *h, const int32_t *env_ids, int32_t n, const void *records, int32_t n_records, const int32_t *rows,
+            void *stream)
+{
+    if (!h) return SF_ERR_ARG;
+    SfDeviceGuard guard(h);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    int rc = sf_snap_args(h, "sf_load", env_ids, n, records, true, s);
+    if (rc) return rc;
+    if (rows) {
+        for (int i = 0; i < n; ++i)
+            if (rows[i] < 0 || rows[i] >= n_records) return sf_fail(h, SF_ERR_ARG, "sf_load: record row out of range");
+        SF_CUDA(h, cudaMemcpyAsync(h->d_rows, rows, (size_t)n * 4, cudaMemcpyHostToDevice, s));
+    } else if (n_records < n) {
+        return sf_fail(h, SF_ERR_ARG, "sf_load: fewer records than arenas");
+    }
+    const uint8_t *rec = static_cast<const uint8_t *>(records);
+    const int32_t *d_ids = env_ids ? h->d_ids : nullptr, *d_rows = rows ? h->d_rows : nullptr;
+    SF_CUDA(h, cudaMemsetAsync(h->d_refused, 0, sizeof(int), s));
+    sf_snap_check_kernel<<<(n + 255) / 256, 256, 0, s>>>(h->snap, rec, d_rows, n, h->d_refused);
+    sf_snap_kernel<false><<<sf_snap_grid(h, n), SF_SNAP_CTA, 0, s>>>(h->snap, h->k.env_id_base, d_ids, n, const_cast<uint8_t *>(rec),
+                                                                    d_rows, h->d_refused);
+    sf_snap_reseed_kernel<<<(n + 255) / 256, 256, 0, s>>>(h->d, h->k, rec, h->snap.bytes, d_ids, d_rows, n, h->d_refused);
+    h->launches += 3;
+    SF_CUDA(h, cudaGetLastError());
+    int refused = 0;
+    SF_CUDA(h, cudaMemcpyAsync(&refused, h->d_refused, sizeof refused, cudaMemcpyDeviceToHost, s));
+    SF_CUDA(h, cudaStreamSynchronize(s));
+    if (refused) return sf_fail(h, SF_ERR_ARG, "sf_load: a record is not one of this configuration (magic, version, size or fingerprint)");
     return SF_OK;
 }
 

@@ -17,8 +17,8 @@ BUILD_SCRIPT = os.path.join(_HERE, "csrc", "build.sh")
 
 EXPORTS = [
     "sf_abi_version", "sf_last_error", "sf_create", "sf_destroy", "sf_reset", "sf_step", "sf_step_a", "sf_step_b",
-    "sf_step_host", "sf_synth_actions", "sf_observe", "sf_get", "sf_export_env", "sf_rng_stream",
-    "sf_agents_per_env", "sf_num_envs", "sf_launch_count", "sf_device_bytes",
+    "sf_step_host", "sf_synth_actions", "sf_observe", "sf_get", "sf_export_env", "sf_snapshot_bytes", "sf_save",
+    "sf_load", "sf_rng_stream", "sf_agents_per_env", "sf_num_envs", "sf_launch_count", "sf_device_bytes",
 ]
 
 _lib = None
@@ -63,6 +63,10 @@ def lib():
         L.sf_observe.argtypes = [vp, vp, i32, C.c_uint32, vp]
         L.sf_get.argtypes = [vp, i32, vp, vp]
         L.sf_export_env.argtypes = [vp, i32, vp, C.POINTER(i64)]
+        L.sf_snapshot_bytes.argtypes = [vp]
+        L.sf_snapshot_bytes.restype = i64
+        L.sf_save.argtypes = [vp, vp, i32, vp, vp]
+        L.sf_load.argtypes = [vp, vp, i32, vp, i32, vp, vp]
         L.sf_rng_stream.argtypes = [vp, vp, vp, i32, i32, vp]
         L.sf_agents_per_env.argtypes = [vp]
         L.sf_num_envs.argtypes = [vp]

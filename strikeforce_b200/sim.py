@@ -159,6 +159,52 @@ class BatchedArena:
         self._chk(lib().sf_export_env(self._h, env, buf.ctypes.data, C.byref(n)))
         return buf[:n.value].copy()
 
+    # ------------------------------------------------------------------ arena records (sf_save / sf_load)
+    @property
+    def snapshot_bytes(self):
+        """bytes of one arena record of this handle (include/strikeforce_b200.h, sf_snapshot_bytes)"""
+        return int(lib().sf_snapshot_bytes(self._h))
+
+    @staticmethod
+    def _ids(ids):
+        return None if ids is None else np.ascontiguousarray(ids, dtype=np.int32).reshape(-1)
+
+    def save(self, env_ids=None, out=None):
+        """Records of arenas ``env_ids`` (default: all, in order) as a uint8 device tensor
+        [n, snapshot_bytes].  A checkpoint on disk is ``save().cpu().numpy()``."""
+        ids = self._ids(env_ids)
+        n = self.n_envs if ids is None else len(ids)
+        if out is None:
+            out = torch.empty((n, self.snapshot_bytes), dtype=torch.uint8, device=self.device)
+        assert out.is_cuda and out.dtype == torch.uint8 and out.is_contiguous()
+        assert out.numel() == n * self.snapshot_bytes
+        self._chk(lib().sf_save(self._h, None if ids is None else ids.ctypes.data, n, C.c_void_p(out.data_ptr()),
+                                self._stream()))
+        return out
+
+    def load(self, records, env_ids=None, rows=None):
+        """Overwrite arenas ``env_ids`` (default: all, in order; distinct) with the records ``records[rows[i]]``
+        (default: row i).  ``records`` is a uint8 tensor [n_records, snapshot_bytes] (a host array or tensor is
+        copied to the device first).  Raises (and changes no arena) when a record is not of this configuration."""
+        records = torch.as_tensor(records)
+        if not records.is_cuda:
+            records = records.to(self.device)
+        records = records.contiguous().view(-1, self.snapshot_bytes)
+        assert records.dtype == torch.uint8
+        ids, rws = self._ids(env_ids), self._ids(rows)
+        n = self.n_envs if ids is None else len(ids)
+        if rws is not None:
+            assert len(rws) == n
+        self._chk(lib().sf_load(self._h, None if ids is None else ids.ctypes.data, n, C.c_void_p(records.data_ptr()),
+                                records.shape[0], None if rws is None else rws.ctypes.data, self._stream()))
+
+    def clone(self, src_ids, dst_ids):
+        """Arena dst_ids[i] becomes a copy of arena src_ids[i]: one save of the distinct sources, one load.
+        A copy under another global id goes on with the source's episode and then follows its own seeds."""
+        src = self._ids(src_ids)
+        uniq, rows = np.unique(src, return_inverse=True)
+        self.load(self.save(uniq), dst_ids, rows=rows)
+
     def rng_stream(self, tb, serial, n_draws):
         """Random::_srand + n _rand() draws per stream on the device (random.hpp:54-76)."""
         tb = np.ascontiguousarray(tb, dtype=np.int64)
