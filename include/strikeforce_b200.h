@@ -201,6 +201,38 @@ int sf_synth_actions(sf_handle *h, uint8_t *actions, uint64_t t, const char *tab
    sf_step_b, SF_OBS_P1 otherwise (SF_ERR_ARG if it does not). */
 int sf_observe(sf_handle *h, float *obs, int32_t phase, uint32_t agent_mask, void *stream);
 
+/* Final observations and partial resets without the host (DESIGN.md section 7b).  With auto_reset = 0 an arena
+   whose episode ends keeps its terminal state until it is reset, so it can be observed; these three calls find,
+   observe and reset such arenas on the device, in stream order, without a host synchronisation (a loop of
+   step, list, observe and reset can be captured in a CUDA graph).
+
+   auto_reset = 0 with sf_reset_finished right after every step (after sf_step_b for a split step) leaves every
+   arena, its sf_step_out, the statistics and the records of sf_save byte for byte as auto_reset = 1 does,
+   including arenas that ended in half A (SF_OVERFLOW, SF_UB_GUARD).  Between the step and the reset,
+   sf_observe, sf_observe_list, sf_get, sf_export_env and sf_save see the terminal state; the terminal state of
+   an abort is undefined, as always.  Finished means: the arena's state has a status other than SF_RUNNING, as
+   the last column of SF_FIELD_COUNTERS shows (sf_step_out only says what the last step did).
+
+   The ids of the finished arenas that have not been reset since, ascending, into the DEVICE buffer
+   env_ids [n_envs]; their number into the DEVICE int32 *count (both 4-byte aligned).  Allowed anywhere, also
+   between sf_step_a and sf_step_b. */
+int sf_list_finished(sf_handle *h, int32_t *env_ids, int32_t *count, void *stream);
+
+/* Reset, on the device, exactly the arenas sf_list_finished would list now, as auto_reset = 1 would have at the
+   end of the step in which they ended: next episode of the arena's own synthetic seed chain (episode + 1), level
+   from its global id, the pending stream installed.  sf_step_out and the SF_STAT_* statistics stay as they are
+   (the step that ended the episode counted it).  SF_ERR_ARG between sf_step_a and sf_step_b; with
+   auto_reset = 1 it finds nothing to do. */
+int sf_reset_finished(sf_handle *h, void *stream);
+
+/* sf_observe for a DEVICE list of arenas: row i of obs ([n_max][n_selected][32][31][31], or channel-innermost
+   with SF_OBS_NHWC or-ed into phase) is the observation of arena env_ids[i] (DEVICE int32 [n_max]), for
+   i < min(*count, n_max) (count: DEVICE int32, NULL = n_max rows).  Rows from that bound up to n_max are not
+   written.  Duplicate ids are allowed; an id outside [0, n_envs) gives an all-zero row.  1 <= n_max <= n_envs;
+   the phase rule and the 16-byte alignment of obs are those of sf_observe. */
+int sf_observe_list(sf_handle *h, float *obs, int32_t phase, uint32_t agent_mask, const int32_t *env_ids,
+                    const int32_t *count, int32_t n_max, void *stream);
+
 /* Copy a per-arena field into a DEVICE buffer (sizes above). */
 int sf_get(sf_handle *h, int32_t field, void *dev_out, void *stream);
 

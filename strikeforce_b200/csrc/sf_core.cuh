@@ -1691,6 +1691,23 @@ SF_FN void sf_reset_body(const SfDev &d, const SfConst &k, const SfTabs &t, int 
     d.out[env] = o;
 }
 
+/* an arena whose episode has ended and that has not been reset since, from its header word */
+SF_FN bool sf_misc_finished(uint32_t misc) { return ((misc >> 8) & 0xFFu) != SF_RUNNING; }
+
+/* sf_reset_finished for arena `env`: what auto-reset does at the end of the step in which the episode
+ * ended (the tail of sf_step_body), on the state that step stored -- next episode of the arena's own
+ * synthetic seed chain, the pending stream installed.  d.out and the statistics are not touched. */
+SF_FN void sf_reset_finished_body(const SfDev &d, const SfConst &k, const SfTabs &t, int env)
+{
+    SfEnv e;
+    sf_load_env(d, env, e);
+    if (e.status != SF_RUNNING) {
+        e.episode += 1;
+        sf_reset_env(d, k, t, env, e);
+        sf_store_env(d, env, e);
+    }
+}
+
 /* one env-step (or one half of it) for arena `env`; `actions` is the arena's row of the
  * action buffer (NULL for SF_HALF_A).  `valid` is false for the padding lanes of the last
  * warp: they walk through the same code with nothing to do, so that every lane of a warp

@@ -250,10 +250,14 @@ __device__ __forceinline__ void sf_obs_item(int item, int nsel, uint32_t agent_m
     *env = item / nsel, *slot = __ffs(m) - 1;
 }
 
-template <bool NHWC> /* NHWC: the same values with the channel innermost, SF_OBS_NHWC of the header */
+/* NHWC: the same values with the channel innermost, SF_OBS_NHWC of the header.  LIST (sf_observe_list): the
+   arena of row r is env_ids[r / nsel] instead of r / nsel, an id outside [0, n_envs) gives a zero row, and the
+   rows written are min(*list_n, n_items / nsel) (list_n == NULL: all); the launch shape is chosen for n_items. */
+template <bool NHWC, bool LIST>
 __global__ void __launch_bounds__(SF_OBS_CTA, SF_OBS_CTAS_PER_SM)
 sf_observe_kernel(const SfDev d, const __grid_constant__ SfConst k, float *__restrict__ obs, uint32_t agent_mask,
-                  int nsel, int n_items, int rows, int run_len)
+                  int nsel, int n_items, int rows, int run_len, const int32_t *__restrict__ env_ids,
+                  const int32_t *__restrict__ list_n)
 {
     float *feat = reinterpret_cast<float *>(sf_smem);                         /* [row][SF_OBS_PITCH] */
     uint16_t *code = reinterpret_cast<uint16_t *>(feat + SF_OBS_ROWS * SF_OBS_PITCH); /* per window cell */
@@ -273,10 +277,19 @@ sf_observe_kernel(const SfDev d, const __grid_constant__ SfConst k, float *__res
         for (int c = 0; c < SF_OBS_CH; ++c) feat[threadIdx.x * SF_OBS_PITCH + c] = f[c] ? sf_obs_transform(d, f[c], &fb) : 0.f;
     }
     constexpr int PER = (SF_OBS_CELLS + SF_OBS_CTA - 1) / SF_OBS_CTA;
+    if constexpr (LIST) {
+        if (list_n) n_items = min(max(*list_n, 0), n_items / nsel) * nsel; /* CTAs whose runs lie beyond it exit */
+    }
     for (int run = blockIdx.x; run * run_len < n_items; run += gridDim.x)
     for (int item = run * run_len, end = min(n_items, item + run_len); item < end; ++item) {
         int env, slot;
         sf_obs_item(item, nsel, agent_mask, &env, &slot);
+        bool listed = true;
+        if constexpr (LIST) { /* an id outside the handle reads arena 0 and observes nothing: a zero row */
+            const int id = env_ids[env];
+            listed = id >= 0 && id < d.n_envs;
+            env = listed ? id : 0;
+        }
         float *out = obs + (size_t)item * SF_OBS_LEN;
         /* the few header words the features need */
         SfEnv e;
@@ -285,7 +298,7 @@ sf_observe_kernel(const SfDev d, const __grid_constant__ SfConst k, float *__res
         e.mb[0] = SF_AT(d.mb, 0), e.mb[1] = SF_AT(d.mb, 1);
         e.ntemp = d.ntemp[env];
         e.env = env;
-        const bool observer = slot < e.hw_h; /* a slot this episode never used sees nothing */
+        const bool observer = listed && slot < e.hw_h; /* a slot this episode never used sees nothing */
         const int vcell = observer ? (int)(SF_AT(d.h_pw, slot) & POS_CELL) : 0;
         const uint32_t team = observer ? (SF_AT(d.h_sel, slot) & HS_TEAM) : 0u;
         int vf, vr, vc;
@@ -629,6 +642,100 @@ __global__ void sf_snap_reseed_kernel(const SfDev d, const __grid_constant__ SfC
     sf_snap_reseed(d, k, t, ids ? ids[i] : i, sf_snap_global_id(w));
 }
 
+/* sf_list_finished / sf_reset_finished: a stable compaction of the arenas whose state is not SF_RUNNING.
+ *
+ * Tiles of SF_LIST_TILE consecutive arenas, one CTA each, four arenas per thread (one 16-byte load of their
+ * header words).  sf_list_count_kernel writes the number of finished arenas of every tile; sf_list_scatter_kernel
+ * adds up the counts of the tiles before its own, scans its tile and writes the ids, and its last CTA writes the
+ * total.  An id's position is the number of finished arenas below it, so the list is ascending and the same on
+ * every run (no atomics); the header words are read twice, the second time from L2 (512 KB at 131,072 arenas). */
+#define SF_LIST_CTA 256
+#define SF_LIST_TILE (4 * SF_LIST_CTA)
+#define SF_FIN_CTA 32 /* sf_reset_finished_kernel: one warp per CTA, so that a short list spreads over the SMs */
+
+/* bit j: arena tile * SF_LIST_TILE + 4 * thread + j is finished (E is a multiple of 32: the load stays in the array) */
+__device__ __forceinline__ uint32_t sf_list_flags(const SfDev &d, int tile)
+{
+    const int base = tile * SF_LIST_TILE + 4 * (int)threadIdx.x;
+    if (base >= d.n_envs) return 0u;
+    const uint4 m = __ldg(reinterpret_cast<const uint4 *>(d.misc + base));
+    uint32_t f = (sf_misc_finished(m.x) ? 1u : 0u) | (sf_misc_finished(m.y) ? 2u : 0u) | (sf_misc_finished(m.z) ? 4u : 0u) |
+                 (sf_misc_finished(m.w) ? 8u : 0u);
+    const int left = d.n_envs - base;
+    return left >= 4 ? f : f & ((1u << left) - 1u);
+}
+
+/* sum of v over the CTA, in every thread */
+__device__ __forceinline__ int sf_list_sum(int v, int *s_warp)
+{
+    v = (int)__reduce_add_sync(0xffffffffu, (unsigned)v);
+    __syncthreads(); /* s_warp is free */
+    if ((threadIdx.x & 31) == 0) s_warp[threadIdx.x >> 5] = v;
+    __syncthreads();
+    int sum = 0;
+#pragma unroll
+    for (int w = 0; w < SF_LIST_CTA / 32; ++w) sum += s_warp[w];
+    return sum;
+}
+
+__global__ void __launch_bounds__(SF_LIST_CTA) sf_list_count_kernel(const SfDev d, int32_t *__restrict__ tile_n)
+{
+    __shared__ int s_warp[SF_LIST_CTA / 32];
+    const int n = sf_list_sum(__popc(sf_list_flags(d, blockIdx.x)), s_warp);
+    if (threadIdx.x == 0) tile_n[blockIdx.x] = n;
+}
+
+__global__ void __launch_bounds__(SF_LIST_CTA)
+sf_list_scatter_kernel(const SfDev d, const int32_t *__restrict__ tile_n, int32_t *__restrict__ ids, int32_t *__restrict__ count)
+{
+    __shared__ int s_warp[SF_LIST_CTA / 32];
+    int before = 0;
+    for (int i = threadIdx.x; i < (int)blockIdx.x; i += SF_LIST_CTA) before += tile_n[i];
+    const int base = sf_list_sum(before, s_warp); /* finished arenas in the tiles below this one */
+    const uint32_t f = sf_list_flags(d, blockIdx.x);
+    const int c = __popc(f), lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int incl = c; /* inclusive scan over the warp */
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int v = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += v;
+    }
+    __syncthreads(); /* every thread has read s_warp */
+    if (lane == 31) s_warp[warp] = incl;
+    __syncthreads();
+    int pos = base + incl - c, total = base;
+#pragma unroll
+    for (int w = 0; w < SF_LIST_CTA / 32; ++w) {
+        pos += w < warp ? s_warp[w] : 0;
+        total += s_warp[w];
+    }
+    const int env = blockIdx.x * SF_LIST_TILE + 4 * (int)threadIdx.x;
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+        if ((f >> j) & 1u) ids[pos++] = env + j;
+    if (blockIdx.x == gridDim.x - 1 && threadIdx.x == 0) *count = total;
+}
+
+/* sf_reset_finished: the listed arenas (the count is read here, not on the host), lpw consecutive entries of the
+ * list per one-warp CTA.  As in sf_launch_step, lpw is the smallest power of two that still fits the list into one
+ * pass of the grid: a reset is a long serial chain per lane (the 19,968-byte overlay cleared with 16-byte stores,
+ * the rest of the stream warm-up, the digit split of the next seeds), so the few dozen arenas that finish in a
+ * typical step run one per SM, and a long list fills whole warps instead of looping. */
+__global__ void __launch_bounds__(SF_FIN_CTA, 1)
+sf_reset_finished_kernel(const SfDev d, const __grid_constant__ SfConst k, const int32_t *__restrict__ ids,
+                         const int32_t *__restrict__ count)
+{
+    const int n = *count;
+    int lpw = 1;
+    while (lpw < SF_FIN_CTA && (n + lpw - 1) / lpw > (int)gridDim.x) lpw *= 2;
+    SfTabs t;
+    sf_global_tabs(d, t);
+    for (int c = blockIdx.x; c * lpw < n; c += gridDim.x) {
+        const int i = c * lpw + (int)threadIdx.x;
+        if ((int)threadIdx.x < lpw && i < n) sf_reset_finished_body(d, k, t, ids[i]);
+    }
+}
+
 /* ====================================================================== host side */
 
 struct sf_handle {
@@ -645,6 +752,9 @@ struct sf_handle {
     int64_t *d_tb = nullptr, *d_serial = nullptr;
     int32_t *d_rows = nullptr;   /* sf_load: record row of each entry */
     int *d_refused = nullptr;    /* sf_load: set when a referenced record is not one of this configuration */
+    int32_t *d_fin_ids = nullptr; /* sf_reset_finished: the finished arenas, ascending ... */
+    int32_t *d_fin_n = nullptr;   /* ... and their number */
+    int32_t *d_tile_n = nullptr;  /* sf_list_finished / sf_reset_finished: finished arenas per tile of SF_LIST_TILE */
     SfSnapLayout snap;           /* the record layout of sf_save / sf_load (sf_snapshot.cuh) */
     int device = 0, n_sm = 0;
     bool between_halves = false; /* sf_step_a has run, sf_step_b has not: the P2 observation point */
@@ -746,6 +856,7 @@ void carve(Carver &c, sf_handle &h)
     c.take(h.d_export_n, (size_t)1);
     c.take(h.d_ids, E), c.take(h.d_tb, E), c.take(h.d_serial, E);
     c.take(h.d_rows, E), c.take(h.d_refused, (size_t)1);
+    c.take(h.d_fin_ids, E), c.take(h.d_fin_n, (size_t)1), c.take(h.d_tile_n, (E + SF_LIST_TILE - 1) / SF_LIST_TILE);
 }
 } // namespace
 
@@ -844,8 +955,10 @@ int sf_create(const sf_config *cfg, sf_handle **out)
     SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_B>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
     SF_CREATE_CUDA(cudaFuncSetAttribute(sf_reset_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
     SF_CREATE_CUDA(cudaFuncSetAttribute(sf_rng_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
-    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_observe_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_OBS_SMEM));
-    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_observe_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_OBS_SMEM));
+    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_observe_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_OBS_SMEM));
+    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_observe_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_OBS_SMEM));
+    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_observe_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_OBS_SMEM));
+    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_observe_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_OBS_SMEM));
     rc = sf_launch_reset(h, nullptr, h->d.n_envs, nullptr, nullptr, 0);
     if (rc == SF_OK) {
         cudaError_t e_ = cudaDeviceSynchronize();
@@ -990,23 +1103,25 @@ int sf_synth_actions(sf_handle *h, uint8_t *actions, uint64_t t, const char *tab
     return SF_OK;
 }
 
-int sf_observe(sf_handle *h, float *obs, int32_t phase, uint32_t agent_mask, void *stream)
+/* the checks and the launch sf_observe and sf_observe_list share: n_rows rows of observations (arenas 0..n_rows-1,
+   or env_ids[0..n_rows) with *count of them written) */
+static int sf_launch_observe(sf_handle *h, const char *fn, float *obs, int32_t phase, uint32_t agent_mask, int n_rows,
+                             const int32_t *env_ids, const int32_t *count, cudaStream_t s)
 {
-    if (!h || !obs) return h ? sf_fail(h, SF_ERR_ARG, "sf_observe: null buffer") : SF_ERR_ARG;
     const bool nhwc = (phase & SF_OBS_NHWC) != 0;
     phase &= ~SF_OBS_NHWC;
-    if (phase != SF_OBS_P1 && phase != SF_OBS_P2) return sf_fail(h, SF_ERR_ARG, "sf_observe: phase must be SF_OBS_P1 or SF_OBS_P2");
+    if (phase != SF_OBS_P1 && phase != SF_OBS_P2) return sf_fail(h, SF_ERR_ARG, std::string(fn) + ": phase must be SF_OBS_P1 or SF_OBS_P2");
     /* the kernel describes the arena as it stands; the phase says WHERE in the step the caller claims
        to be, and a claim that does not match the handle is an error: P2 is the point between
        sf_step_a and sf_step_b (get_command inside human_action), P1 the loop top */
     if ((phase == SF_OBS_P2) != h->between_halves)
-        return sf_fail(h, SF_ERR_ARG, phase == SF_OBS_P2 ? "sf_observe: SF_OBS_P2 is the point between sf_step_a and sf_step_b"
-                                                         : "sf_observe: between sf_step_a and sf_step_b the observation point is SF_OBS_P2");
+        return sf_fail(h, SF_ERR_ARG, std::string(fn) + (phase == SF_OBS_P2 ? ": SF_OBS_P2 is the point between sf_step_a and sf_step_b"
+                                                                             : ": between sf_step_a and sf_step_b the observation point is SF_OBS_P2"));
     SfDeviceGuard guard(h);
     int nsel = __builtin_popcount(agent_mask);
-    if (nsel == 0) return sf_fail(h, SF_ERR_ARG, "sf_observe: empty agent mask");
-    if (reinterpret_cast<uintptr_t>(obs) & 15u) return sf_fail(h, SF_ERR_ARG, "sf_observe: obs must be 16-byte aligned");
-    int n_items = h->d.n_envs * nsel;
+    if (nsel == 0) return sf_fail(h, SF_ERR_ARG, std::string(fn) + ": empty agent mask");
+    if (reinterpret_cast<uintptr_t>(obs) & 15u) return sf_fail(h, SF_ERR_ARG, std::string(fn) + ": obs must be 16-byte aligned");
+    int n_items = n_rows * nsel;
     /* a CTA writes runs of consecutive observations: HBM takes 1,184 store streams that each run on for
        megabytes better than a front of 123 KB pieces (profiles/r02_obs_run.txt: 73 -> 80% of the peak); the
        longest run of up to 16 that still leaves every CTA four turns */
@@ -1016,12 +1131,70 @@ int sf_observe(sf_handle *h, float *obs, int32_t phase, uint32_t agent_mask, voi
         for (run_len = 16; run_len > 1 && n_items / run_len < 4 * ctas; run_len >>= 1) {}
     int runs = (n_items + run_len - 1) / run_len;
     int grid = runs < ctas ? runs : ctas;
-    if (nhwc)
-        sf_observe_kernel<true><<<grid, SF_OBS_CTA, SF_OBS_SMEM, static_cast<cudaStream_t>(stream)>>>(h->d, h->k, obs, agent_mask,
-                                                                                                    nsel, n_items, h->obs_rows, run_len);
-    else
-        sf_observe_kernel<false><<<grid, SF_OBS_CTA, SF_OBS_SMEM, static_cast<cudaStream_t>(stream)>>>(h->d, h->k, obs, agent_mask,
-                                                                                                     nsel, n_items, h->obs_rows, run_len);
+#define SF_OBS_LAUNCH(NHWC, LIST)                                                                                          \
+    sf_observe_kernel<NHWC, LIST><<<grid, SF_OBS_CTA, SF_OBS_SMEM, s>>>(h->d, h->k, obs, agent_mask, nsel, n_items, h->obs_rows, \
+                                                                        run_len, env_ids, count)
+    if (env_ids) {
+        if (nhwc) SF_OBS_LAUNCH(true, true);
+        else SF_OBS_LAUNCH(false, true);
+    } else {
+        if (nhwc) SF_OBS_LAUNCH(true, false);
+        else SF_OBS_LAUNCH(false, false);
+    }
+#undef SF_OBS_LAUNCH
+    h->launches += 1;
+    SF_CUDA(h, cudaGetLastError());
+    return SF_OK;
+}
+
+int sf_observe(sf_handle *h, float *obs, int32_t phase, uint32_t agent_mask, void *stream)
+{
+    if (!h || !obs) return h ? sf_fail(h, SF_ERR_ARG, "sf_observe: null buffer") : SF_ERR_ARG;
+    return sf_launch_observe(h, "sf_observe", obs, phase, agent_mask, h->d.n_envs, nullptr, nullptr, static_cast<cudaStream_t>(stream));
+}
+
+int sf_observe_list(sf_handle *h, float *obs, int32_t phase, uint32_t agent_mask, const int32_t *env_ids, const int32_t *count,
+                    int32_t n_max, void *stream)
+{
+    if (!h || !obs || !env_ids) return h ? sf_fail(h, SF_ERR_ARG, "sf_observe_list: null buffer") : SF_ERR_ARG;
+    if (n_max < 1 || n_max > h->d.n_envs) return sf_fail(h, SF_ERR_ARG, "sf_observe_list: n_max must be in [1, n_envs]");
+    if ((reinterpret_cast<uintptr_t>(env_ids) | reinterpret_cast<uintptr_t>(count)) & 3u)
+        return sf_fail(h, SF_ERR_ARG, "sf_observe_list: env_ids and count must be 4-byte aligned");
+    return sf_launch_observe(h, "sf_observe_list", obs, phase, agent_mask, n_max, env_ids, count, static_cast<cudaStream_t>(stream));
+}
+
+/* the two launches of the compaction (see sf_list_count_kernel) */
+static int sf_launch_list(sf_handle *h, int32_t *ids, int32_t *count, cudaStream_t s)
+{
+    const int tiles = (h->d.n_envs + SF_LIST_TILE - 1) / SF_LIST_TILE;
+    sf_list_count_kernel<<<tiles, SF_LIST_CTA, 0, s>>>(h->d, h->d_tile_n);
+    sf_list_scatter_kernel<<<tiles, SF_LIST_CTA, 0, s>>>(h->d, h->d_tile_n, ids, count);
+    h->launches += 2;
+    SF_CUDA(h, cudaGetLastError());
+    return SF_OK;
+}
+
+int sf_list_finished(sf_handle *h, int32_t *env_ids, int32_t *count, void *stream)
+{
+    if (!h || !env_ids || !count) return h ? sf_fail(h, SF_ERR_ARG, "sf_list_finished: null buffer") : SF_ERR_ARG;
+    if ((reinterpret_cast<uintptr_t>(env_ids) | reinterpret_cast<uintptr_t>(count)) & 3u)
+        return sf_fail(h, SF_ERR_ARG, "sf_list_finished: env_ids and count must be 4-byte aligned");
+    SfDeviceGuard guard(h);
+    return sf_launch_list(h, env_ids, count, static_cast<cudaStream_t>(stream));
+}
+
+int sf_reset_finished(sf_handle *h, void *stream)
+{
+    if (!h) return SF_ERR_ARG;
+    if (h->between_halves) return sf_fail(h, SF_ERR_ARG, "sf_reset_finished: the step opened by sf_step_a is still waiting for sf_step_b");
+    SfDeviceGuard guard(h);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    int rc = sf_launch_list(h, h->d_fin_ids, h->d_fin_n, s);
+    if (rc) return rc;
+    /* one-warp CTAs, four per SM (see sf_reset_finished_kernel for how the list is spread over them) */
+    int grid = (h->d.n_envs + SF_FIN_CTA - 1) / SF_FIN_CTA;
+    if (grid > 4 * h->n_sm) grid = 4 * h->n_sm;
+    sf_reset_finished_kernel<<<grid, SF_FIN_CTA, 0, s>>>(h->d, h->k, h->d_fin_ids, h->d_fin_n);
     h->launches += 1;
     SF_CUDA(h, cudaGetLastError());
     return SF_OK;

@@ -104,26 +104,68 @@ class BatchedArena:
         return out
 
     # ------------------------------------------------------------------ observation / readback
-    def observe(self, agent_mask=1, phase=sfcfg.OBS_P1, out=None, channels_last=False):
+    def observe(self, agent_mask=1, phase=sfcfg.OBS_P1, out=None, channels_last=False, env_ids=None, count=None):
         """gameplay::bot() up to Agent::predict (bots/bot-0.5/Custom.hpp:137-158): fp32 device
         tensor [n_envs, n_selected, 32, 31, 31].
 
         ``channels_last=True`` returns a tensor of the same shape and values whose MEMORY is
         [n_envs, n_selected, 31, 31, 32] (SF_OBS_NHWC): ``.flatten(0, 1)`` of it is a channels-last batch that
         the policy's first convolution reads without a transpose.  ``out`` is always the plain buffer in memory
-        order."""
+        order.
+
+        ``env_ids`` (an int32 CUDA tensor [n_max], sf_observe_list) observes those arenas instead: the result has
+        n_max rows, row i is arena env_ids[i] (duplicates allowed, an id outside [0, n_envs) gives a zero row).
+        With ``count`` (an int32 CUDA tensor [1], e.g. from ``list_finished``) only the first min(count, n_max)
+        rows are written, with no host synchronisation; rows at and beyond ``count`` are whatever ``out`` held
+        (uninitialised memory when ``out`` is None)."""
         nsel = bin(agent_mask).count("1")
         W, CH = sfcfg.OBS_WIN, sfcfg.OBS_CH
+        rows = self.n_envs
+        if env_ids is not None:
+            assert env_ids.is_cuda and env_ids.dtype == torch.int32 and env_ids.is_contiguous() and env_ids.dim() == 1
+            rows = env_ids.numel()
+            if count is not None:
+                assert count.is_cuda and count.dtype == torch.int32 and count.numel() == 1
+        else:
+            assert count is None, "count goes with env_ids"
         if out is None:
-            out = torch.empty((self.n_envs, nsel, W, W, CH) if channels_last else (self.n_envs, nsel, CH, W, W),
+            out = torch.empty((rows, nsel, W, W, CH) if channels_last else (rows, nsel, CH, W, W),
                               dtype=torch.float32, device=self.device)
         assert out.is_cuda and out.dtype == torch.float32 and out.is_contiguous()
-        assert out.numel() == self.n_envs * nsel * sfcfg.OBS_LEN
-        self._chk(lib().sf_observe(self._h, C.c_void_p(out.data_ptr()), phase | (sfcfg.OBS_NHWC if channels_last else 0),
-                                   agent_mask, self._stream()))
+        assert out.numel() == rows * nsel * sfcfg.OBS_LEN
+        ph = phase | (sfcfg.OBS_NHWC if channels_last else 0)
+        if env_ids is None:
+            self._chk(lib().sf_observe(self._h, C.c_void_p(out.data_ptr()), ph, agent_mask, self._stream()))
+        else:
+            self._chk(lib().sf_observe_list(self._h, C.c_void_p(out.data_ptr()), ph, agent_mask,
+                                            C.c_void_p(env_ids.data_ptr()),
+                                            None if count is None else C.c_void_p(count.data_ptr()), rows,
+                                            self._stream()))
         if channels_last:
-            return out.view(self.n_envs, nsel, W, W, CH).permute(0, 1, 4, 2, 3)
+            return out.view(rows, nsel, W, W, CH).permute(0, 1, 4, 2, 3)
         return out
+
+    # ------------------------------------------------------------------ finished arenas (final observations)
+    def list_finished(self, ids=None, count=None):
+        """sf_list_finished: ``(ids, count)``, device tensors int32 [n_envs] and int32 [1]: the ascending ids of
+        the arenas whose episode has ended and that have not been reset since are ids[:count].  No host
+        synchronisation; pass ``ids`` / ``count`` to reuse buffers (e.g. inside a CUDA graph)."""
+        if ids is None:
+            ids = torch.empty(self.n_envs, dtype=torch.int32, device=self.device)
+        if count is None:
+            count = torch.empty(1, dtype=torch.int32, device=self.device)
+        assert ids.is_cuda and ids.dtype == torch.int32 and ids.is_contiguous() and ids.numel() == self.n_envs
+        assert count.is_cuda and count.dtype == torch.int32 and count.numel() == 1
+        self._chk(lib().sf_list_finished(self._h, C.c_void_p(ids.data_ptr()), C.c_void_p(count.data_ptr()),
+                                         self._stream()))
+        return ids, count
+
+    def reset_finished(self):
+        """sf_reset_finished: reset on the device every arena ``list_finished`` would list, as auto-reset would
+        have at the end of the step that ended its episode.  With ``auto_reset=False`` and this call after every
+        step, a run is the same as with auto-reset, but the terminal states can be observed in between (the
+        "final observation" of a truncated episode).  No host synchronisation."""
+        self._chk(lib().sf_reset_finished(self._h, self._stream()))
 
     def _get(self, field, shape, dtype):
         out = torch.empty(shape, dtype=dtype, device=self.device)
