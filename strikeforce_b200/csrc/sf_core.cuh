@@ -14,6 +14,8 @@
 #ifndef SF_CORE_CUH
 #define SF_CORE_CUH
 
+#include <string.h>
+
 #include "sf_state.h"
 #include "sf_synth.h"
 
@@ -437,46 +439,89 @@ SF_FN int sf_alloc_bullet(const SfConst &k, SfEnv &e)
  * every half-tick), and on this layout a cell update is a scattered 2-byte write into a 2.6 GB
  * overlay; deriving the flag instead removes those writes and the look-ahead read of update_bull.
  *
- * "Is there a bullet flag on this cell?" is answered by a per-arena TABLE in shared memory: an
- * open-addressing hash set (linear probing) of the flagged cells, SF_BT_SLOTS 16-bit entries
- * (cell + 1, 0 = empty) plus a count.  One lane's rare event is its whole warp's wait -- and, with
- * the phase barriers, its whole CTA's -- so nothing on this path may be slow, not even the
- * overflow: an arena with more than SF_BT_FULL flagged cells (1% of the arenas of the benchmark
- * at any time) SPILLS the next flags into the overlay word of their cell (C_S2, the bit the
- * reference keeps there), marks their bullets BF_SPILL and raises SF_BT_SPILL in its count; while
- * that is up a look-up that misses the table also reads the cell.  sf_resolve_bullets, which
- * consumes every flag, clears the spilled bits through their bullets and wipes the table.  The
- * table is rebuilt from the bullet rows when a kernel picks an arena up. */
+ * "Is there a bullet flag on this cell?" is answered by a per-arena TABLE in shared memory: a
+ * hash set of the flagged cells with two choices of 4-way buckets.  A bucket is one 8-byte word of
+ * four 16-bit keys (cell + 1, 0 = empty, filled from the low end); a cell may live in either of its
+ * two buckets, and an insert takes the emptier one.  A look-up reads both words and compares all
+ * eight keys at once: the same few instructions for every lane, with no loop and no branch on
+ * what the table holds.  One lane's slow event is its whole warp's wait -- and, with the phase
+ * barriers, its whole CTA's -- so nothing on this path may be slow, not even the overflow: a flag
+ * whose two buckets are full, or that would make more than SF_BT_FULL flags in the table, SPILLS
+ * into the overlay word of its cell (C_S2, the bit the reference keeps there), its bullet is
+ * marked BF_SPILL and SF_BT_SPILL is raised in the table's count; while that is up a look-up that
+ * misses the table also reads the cell.  sf_resolve_bullets, which consumes every flag, clears the
+ * spilled bits through their bullets and wipes the table.  The table is rebuilt from the bullet
+ * rows when a kernel picks an arena up.  Which flags spill depends on the order of the inserts;
+ * the answers do not. */
 #ifndef SF_BT_SLOTS
 #define SF_BT_SLOTS 47
 #define SF_BT_FULL 40
 #endif
-#define SF_BT_ENTRIES (SF_BT_SLOTS + 1) /* 48 x uint16 = 24 words per arena */
+#define SF_BT_BUCKETS (SF_BT_SLOTS / 4)               /* 11 */
+#define SF_BT_ENTRIES (4 * SF_BT_BUCKETS + 4)         /* uint16 per arena: the buckets, then the count word (48) */
 #define SF_BT_SPILL 0x8000u
-SF_FN uint16_t &sf_bt_at(const SfTabs &t, int i) { return t.bt[i * t.bt_stride]; }
+#define SF_BT_TOPS 0x80008000u
+#if SF_BT_BUCKETS < 1
+#error "the bullet-flag table needs SF_BT_SLOTS >= 4 (one bucket)"
+#endif
+
+/* word w of the arena's table, w = SF_BT_BUCKETS being the count: entry 4 w .. 4 w + 3 of a
+ * contiguous table (bt_stride = 1), 8-byte words laid out [word][thread] in shared memory */
+SF_FN uint64_t sf_bt_word(const SfTabs &t, int w)
+{
+#ifdef __CUDA_ARCH__
+    return *reinterpret_cast<const uint64_t *>(t.bt + 4 * w * t.bt_stride);
+#else
+    uint64_t v;
+    memcpy(&v, t.bt + 4 * w * t.bt_stride, sizeof v);
+    return v;
+#endif
+}
+SF_FN void sf_bt_set_word(const SfTabs &t, int w, uint64_t v)
+{
+#ifdef __CUDA_ARCH__
+    *reinterpret_cast<uint64_t *>(t.bt + 4 * w * t.bt_stride) = v;
+#else
+    memcpy(t.bt + 4 * w * t.bt_stride, &v, sizeof v);
+#endif
+}
+/* the number of flags in the table | SF_BT_SPILL */
+SF_FN uint16_t &sf_bt_count(const SfTabs &t) { return t.bt[4 * SF_BT_BUCKETS * t.bt_stride]; }
 SF_FN void sf_bt_wipe(const SfTabs &t)
 {
     SF_UNROLL
-    for (int i = 0; i < SF_BT_ENTRIES; ++i) sf_bt_at(t, i) = 0;
+    for (int w = 0; w <= SF_BT_BUCKETS; ++w) sf_bt_set_word(t, w, 0ull);
 }
-/* the slot that holds `cell`, or -1 - (the empty slot where it would go) */
-SF_FN int sf_bt_find(const SfTabs &t, int cell)
+/* keys in a bucket word (they fill it from the low end) */
+SF_FN int sf_bt_fill(uint64_t w) { return (sf_fls64(w) + 16) >> 4; }
+/* the two buckets of `cell` (distinct unless the table has only one) and their words */
+struct SfBtProbe {
+    int b0, b1;
+    uint64_t w0, w1;
+    bool hit; /* `cell` is in one of them */
+};
+SF_FN SfBtProbe sf_bt_probe(const SfTabs &t, int cell)
 {
-    const uint32_t key = (uint32_t)cell + 1u;
-    int i = (int)(((((uint32_t)cell * 40503u) >> 3) & 0xFFFFu) * SF_BT_SLOTS >> 16);
-    SF_NO_UNROLL
-    for (;;) {
-        const uint32_t v = sf_bt_at(t, i);
-        if (v == key) return i;
-        if (v == 0u) return -1 - i;
-        i = i + 1 == SF_BT_SLOTS ? 0 : i + 1;
-    }
+    SfBtProbe p;
+    const uint32_t c = (uint32_t)cell;
+    p.b0 = (int)((((c * 0x9E3779B1u) >> 16) * SF_BT_BUCKETS) >> 16);
+    const int b1 = p.b0 + 1 + (int)((((c * 0x85EBCA6Bu) >> 16) * (SF_BT_BUCKETS - 1)) >> 16);
+    p.b1 = b1 >= SF_BT_BUCKETS ? b1 - SF_BT_BUCKETS : b1;
+    p.w0 = sf_bt_word(t, p.b0), p.w1 = sf_bt_word(t, p.b1);
+    /* a halfword of (word ^ key) is 0 where the key is.  Keys are below 0x8000 (cell ids have 14
+     * bits, sf_state.h), so adding 0x7FFF sets bit 15 of a halfword exactly when it is not 0, and
+     * no carry crosses into the next one */
+    const uint32_t k = (c + 1u) * 0x10001u;
+    const uint32_t nz = (((uint32_t)p.w0 ^ k) + 0x7FFF7FFFu) & (((uint32_t)(p.w0 >> 32) ^ k) + 0x7FFF7FFFu) &
+                        (((uint32_t)p.w1 ^ k) + 0x7FFF7FFFu) & (((uint32_t)(p.w1 >> 32) ^ k) + 0x7FFF7FFFu);
+    p.hit = (nz & SF_BT_TOPS) != SF_BT_TOPS;
+    return p;
 }
 /* node::s[2] of `cell` */
 SF_FN bool sf_flagged(const SfDev &d, const SfTabs &t, int env, int cell)
 {
-    if (sf_bt_find(t, cell) >= 0) return true;
-    return (sf_bt_at(t, SF_BT_SLOTS) & SF_BT_SPILL) && (SF_G(cell) & C_S2);
+    if (sf_bt_probe(t, cell).hit) return true;
+    return (sf_bt_count(t) & SF_BT_SPILL) && (SF_G(cell) & C_S2);
 }
 /* raise the flag of `cell`: 0 = it was up already (in the table), SF_FLAG_NEW = raised in the
  * table, and with BF_SPILL or'ed in: ... in the overlay (the bullet that owns the flag carries
@@ -484,23 +529,27 @@ SF_FN bool sf_flagged(const SfDev &d, const SfTabs &t, int env, int cell)
 #define SF_FLAG_NEW 1u
 SF_FN uint32_t sf_flag_cell(const SfDev &d, const SfTabs &t, int env, int cell)
 {
-    const int i = sf_bt_find(t, cell);
-    if (i >= 0) return 0u;
-    const uint32_t n = sf_bt_at(t, SF_BT_SLOTS);
+    const SfBtProbe p = sf_bt_probe(t, cell);
+    if (p.hit) return 0u;
+    const uint32_t n = sf_bt_count(t);
+    const int f0 = sf_bt_fill(p.w0), f1 = sf_bt_fill(p.w1);
+    const bool room = (n & ~SF_BT_SPILL) < SF_BT_FULL && (f0 < 4 || f1 < 4);
     if (n & SF_BT_SPILL) { /* some flags of this arena live in the overlay: this one? */
         const uint32_t g = SF_G(cell);
         if (g & C_S2) return BF_SPILL;
-        if ((n & ~SF_BT_SPILL) >= SF_BT_FULL) {
+        if (!room) {
             SF_G(cell) = (uint16_t)(g | C_S2);
             return SF_FLAG_NEW | BF_SPILL;
         }
-    } else if (n >= SF_BT_FULL) {
+    } else if (!room) {
         SF_G(cell) = (uint16_t)(SF_G(cell) | C_S2);
-        sf_bt_at(t, SF_BT_SLOTS) = (uint16_t)(n | SF_BT_SPILL);
+        sf_bt_count(t) = (uint16_t)(n | SF_BT_SPILL);
         return SF_FLAG_NEW | BF_SPILL;
     }
-    sf_bt_at(t, -1 - i) = (uint16_t)(cell + 1);
-    sf_bt_at(t, SF_BT_SLOTS) = (uint16_t)(n + 1u);
+    const bool second = f1 < f0;
+    const uint64_t key = (uint64_t)(cell + 1) << (16 * (second ? f1 : f0));
+    sf_bt_set_word(t, second ? p.b1 : p.b0, (second ? p.w1 : p.w0) | key);
+    sf_bt_count(t) = (uint16_t)(n + 1u);
     return SF_FLAG_NEW;
 }
 
@@ -538,7 +587,9 @@ SF_FN int sf_owner_scan(const SfDev &d, int env, const SfEnv &e, int cell, int s
 }
 
 /* rebuild the table from the bullet rows (the owning bullets of a resting arena are exact; the
- * spilled flags are in the overlay already) */
+ * spilled flags are in the overlay already).  The flags go in in slot order, not in the order they
+ * were raised, so a set that fitted may not fit now: a flag with no room spills here like anywhere
+ * else, and its bullet is marked */
 SF_FN void sf_bt_rebuild(const SfDev &d, const SfTabs &t, int env, const SfEnv &e)
 {
     sf_bt_wipe(t);
@@ -557,10 +608,10 @@ SF_FN void sf_bt_rebuild(const SfDev &d, const SfTabs &t, int env, const SfEnv &
         for (int j = 0; j < 4; ++j) {
             const uint32_t mj = j == 0 ? meta[0] : j == 1 ? meta[1] : j == 2 ? meta[2] : meta[3];
             const uint32_t pj = j == 0 ? pw[0] : j == 1 ? pw[1] : j == 2 ? pw[2] : pw[3];
-            if (mj & BF_SPILL) sf_bt_at(t, SF_BT_SLOTS) = (uint16_t)(sf_bt_at(t, SF_BT_SLOTS) | SF_BT_SPILL);
+            if (mj & BF_SPILL) sf_bt_count(t) = (uint16_t)(sf_bt_count(t) | SF_BT_SPILL);
             else if (mj & BF_OWNS) {
                 const uint32_t fl = sf_flag_cell(d, t, env, (int)(pj & POS_CELL));
-                if (fl & BF_SPILL) SF_AT(d.b_meta, b0 + j) = mj | BF_SPILL; /* never: the table held them before */
+                if (fl & BF_SPILL) SF_AT(d.b_meta, b0 + j) = mj | BF_SPILL;
             }
         }
         SF_SYNCWARP();
@@ -978,7 +1029,7 @@ SF_FN void sf_zombie_damage(const SfDev &d, const SfConst &k, int env, SfEnv &e,
 SF_FN void sf_resolve_bullets(const SfDev &d, const SfConst &k, const SfTabs &t, int env, SfEnv &e)
 {
 #ifdef SF_DEBUG_HIST
-    if (e.on) sf_dbg_hist[sf_bt_at(t, SF_BT_SLOTS) < 255 ? sf_bt_at(t, SF_BT_SLOTS) : 255] += 1;
+    if (e.on) sf_dbg_hist[sf_bt_count(t) < 255 ? sf_bt_count(t) : 255] += 1;
 #endif
     const uint64_t quitters = e.on ? (e.quit & e.mh) : 0ull; /* Hp <= 0 by '_': removed, never hit (:640-645) */
     e.quit = 0;

@@ -32,7 +32,7 @@
 #define SF_SMEM_EXP 65536 /* the first half of the exp table (sf_exp_m1) */
 #endif
 #define SF_SMEM_MAP SF_TCELLS /* 9,984, a multiple of 16 */
-#define SF_SMEM_BT (SF_CTA * SF_BT_ENTRIES * 2) /* the bullet-flag tables of the CTA's arenas, [entry][thread] */
+#define SF_SMEM_BT (SF_CTA * SF_BT_ENTRIES * 2) /* the bullet-flag tables of the CTA's arenas, [8-byte word][thread] */
 #define SF_SMEM_BYTES (SF_SMEM_EXP + SF_SMEM_MAP + SF_SMEM_BT) /* 161,536 B: the 164 KB carve-out, 92 KB of L1 */
 #define SF_POW_LUT_LEN (1 << 21)
 #define SF_EXPORT_CAP (1 << 18)
@@ -53,8 +53,9 @@ __device__ __forceinline__ void sf_stage_tables(const SfDev &d, SfTabs &t)
     t.smap = sf_smem + SF_SMEM_EXP;
     t.log_tab = d.log_tab;
     t.rng_cst = d.rng_cst, t.E = d.E;
-    /* entry i of this thread's table at [i][thread]: two neighbouring lanes share a bank, no more */
-    t.bt = reinterpret_cast<uint16_t *>(sf_smem + SF_SMEM_EXP + SF_SMEM_MAP) + threadIdx.x;
+    /* 8-byte word w of this thread's table at [w][thread]: a warp's reads of any words are free of
+     * bank conflicts (SF_CTA is a multiple of 16) */
+    t.bt = reinterpret_cast<uint16_t *>(sf_smem + SF_SMEM_EXP + SF_SMEM_MAP) + 4 * threadIdx.x;
     t.bt_stride = SF_CTA;
 }
 
