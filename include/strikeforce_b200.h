@@ -150,7 +150,16 @@ enum { SF_OBS_P1 = 1 /* loop top, get_my_action gameplay.hpp:956 */,
           (what a convolution library calls NHWC / channels-last; the reference's tensor, Custom.hpp:139, is
           [32][31][31]).  The policy's first convolution then reads the buffer as it is instead of
           transposing 123,008 bytes per observation first. */
-       SF_OBS_NHWC = 0x100 };
+       SF_OBS_NHWC = 0x100,
+       /* OR-ed into the phase, at most one of the two, with or without SF_OBS_NHWC: obs holds 2-byte
+          values, IEEE fp16 or bfloat16, in the same layout and for the same rows.  Element i is the
+          round-to-nearest-even conversion of element i of the fp32 buffer the same call without the flag
+          writes (61,504 B per observation instead of 123,008; SF_STAT_RESERVED0 counts as for fp32).  Every
+          observation value is 0 or in [0.15, 12), so fp16 holds them without overflow or subnormals and keeps more
+          of them distinct; bfloat16 is what a bf16 network reads without a cast.  Both flags set is
+          SF_ERR_ARG, as is either flag for a library that predates them: a caller can probe for them. */
+       SF_OBS_F16 = 0x200,
+       SF_OBS_BF16 = 0x400 };
 
 /* Replaces: the process-wide `gameplay g` and its globals (gameplay.hpp:47-55, 1739). */
 int sf_create(const sf_config *cfg, sf_handle **out);
@@ -195,11 +204,12 @@ int sf_synth_actions(sf_handle *h, uint8_t *actions, uint64_t t, const char *tab
 
 /* Replaces gameplay::bot() up to the Agent::predict call (bots/bot-0.5/Custom.hpp:137-158):
    writes the fp32 [n_envs][n_obs_agents][32][31][31] observation of the driven humans into the
-   DEVICE buffer obs ([..][31][31][32] with phase | SF_OBS_NHWC).  agent_mask bit a selects human slot a
+   DEVICE buffer obs ([..][31][31][32] with phase | SF_OBS_NHWC; fp16 or bfloat16 values with phase |
+   SF_OBS_F16 or phase | SF_OBS_BF16).  obs must be 16-byte aligned.  agent_mask bit a selects human slot a
    (bit 0 = the player).  phase names the
    observation point the caller is at and must match the handle: SF_OBS_P2 between sf_step_a and
    sf_step_b, SF_OBS_P1 otherwise (SF_ERR_ARG if it does not). */
-int sf_observe(sf_handle *h, float *obs, int32_t phase, uint32_t agent_mask, void *stream);
+int sf_observe(sf_handle *h, void *obs, int32_t phase, uint32_t agent_mask, void *stream);
 
 /* Final observations and partial resets without the host (DESIGN.md section 7b).  With auto_reset = 0 an arena
    whose episode ends keeps its terminal state until it is reset, so it can be observed; these three calls find,
@@ -229,8 +239,8 @@ int sf_reset_finished(sf_handle *h, void *stream);
    with SF_OBS_NHWC or-ed into phase) is the observation of arena env_ids[i] (DEVICE int32 [n_max]), for
    i < min(*count, n_max) (count: DEVICE int32, NULL = n_max rows).  Rows from that bound up to n_max are not
    written.  Duplicate ids are allowed; an id outside [0, n_envs) gives an all-zero row.  1 <= n_max <= n_envs;
-   the phase rule and the 16-byte alignment of obs are those of sf_observe. */
-int sf_observe_list(sf_handle *h, float *obs, int32_t phase, uint32_t agent_mask, const int32_t *env_ids,
+   the phase rule, the output formats and the 16-byte alignment of obs are those of sf_observe. */
+int sf_observe_list(sf_handle *h, void *obs, int32_t phase, uint32_t agent_mask, const int32_t *env_ids,
                     const int32_t *count, int32_t n_max, void *stream);
 
 /* Copy a per-arena field into a DEVICE buffer (sizes above). */

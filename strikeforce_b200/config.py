@@ -32,6 +32,7 @@ STATUS_NAMES = ["running", "win", "dead", "timeout", "truncated", "overflow", "u
 
 OBS_P1, OBS_P2 = 1, 2
 OBS_NHWC = 0x100  # OR-ed into the phase: channel innermost
+OBS_F16, OBS_BF16 = 0x200, 0x400  # OR-ed into the phase (at most one): fp16 / bfloat16 values, rounded to nearest even
 
 FIELD_STEP_OUT, FIELD_STATE_HASH, FIELD_COUNTERS, FIELD_POPULATION, FIELD_STATS = 1, 2, 3, 4, 5
 STAT_NAMES = ["steps", "episodes", "wins", "deaths", "timeouts", "truncated", "overflows", "ub_guards",

@@ -8,6 +8,8 @@
  * is no tensor-core work on this path (no dense contraction) and no CPU fallback: every entry
  * point fails with SF_ERR_NO_DEVICE when no CUDA device is usable.
  */
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
 #include <cstdio>
@@ -15,6 +17,7 @@
 #include <cstring>
 #include <new>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "sf_canon_dev.cuh"
@@ -243,6 +246,53 @@ __global__ void sf_population_kernel(const SfDev d, const __grid_constant__ SfCo
 static_assert(SF_OBS_CELLS % 4 == 1 && SF_OBS_CH % 4 == 0, "the copy-out relies on 4 channels = 961 whole chunks");
 static_assert(SF_OBS_ROWS % 4 == 0, "the arrays behind the table stay 16-byte aligned");
 
+/* Half-precision output (SF_OBS_F16 / SF_OBS_BF16, DESIGN.md section 7c): the table rows hold the converted
+   values, so the copy-out moves 2-byte elements and a 16-byte chunk holds eight of them.  Row pitch in elements:
+   - NHWC: 32 halves = 64 B, so a cell's row is four 16-byte chunks read with 16-byte loads.  A quarter-warp
+     phase of those loads covers two window cells; their rows use different halves of the banks whenever the
+     row numbers differ in parity, which consecutive dynamic cells (consecutive rows) always do;
+   - [32][31][31]: 34 halves = 17 words, odd, so that 2-byte reads of different rows fall into different banks
+     as the odd fp32 pitch does. */
+template <typename T, bool NHWC>
+__host__ __device__ constexpr int sf_obs_pitch() { return std::is_same<T, float>::value ? SF_OBS_PITCH : NHWC ? SF_OBS_CH : SF_OBS_CH + 2; }
+template <typename T, bool NHWC>
+__host__ __device__ constexpr int sf_obs_smem() { return SF_OBS_ROWS * sf_obs_pitch<T, NHWC>() * (int)sizeof(T) + 4 * SF_OBS_LIST * 2 + 16; }
+static_assert(sf_obs_smem<float, false>() == SF_OBS_SMEM && sf_obs_smem<float, true>() == SF_OBS_SMEM, "fp32 table");
+static_assert(SF_OBS_CELLS % 8 == 1 && SF_OBS_CH % 8 == 0, "the half copy-out relies on 8 channels = 961 whole chunks");
+static_assert(sf_obs_smem<__half, false>() % 16 == 0 && sf_obs_smem<__half, true>() % 16 == 0, "16-byte aligned arrays");
+
+/* two features as one word of two halves, round to nearest even, the first in the low half */
+template <typename T> __device__ __forceinline__ uint32_t sf_obs_pack2(float a, float b);
+template <> __device__ __forceinline__ uint32_t sf_obs_pack2<__half>(float a, float b)
+{
+    const __half2 v = __floats2half2_rn(a, b);
+    return *reinterpret_cast<const uint32_t *>(&v);
+}
+template <> __device__ __forceinline__ uint32_t sf_obs_pack2<__nv_bfloat16>(float a, float b)
+{
+    const __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
+    return *reinterpret_cast<const uint32_t *>(&v);
+}
+
+/* the 32 transformed features f[] of a cell as the table row `row` of a half type */
+template <typename T, bool NHWC>
+__device__ __forceinline__ void sf_obs_put_half_row(const SfDev &d, T *row, const int32_t f[32], uint32_t *fb)
+{
+    uint32_t wv[SF_OBS_CH / 2];
+#pragma unroll
+    for (int c = 0; c < SF_OBS_CH / 2; ++c)
+        wv[c] = sf_obs_pack2<T>(f[2 * c] ? sf_obs_transform(d, f[2 * c], fb) : 0.f,
+                                f[2 * c + 1] ? sf_obs_transform(d, f[2 * c + 1], fb) : 0.f);
+    if constexpr (NHWC) { /* 64-byte rows: four 16-byte stores */
+#pragma unroll
+        for (int c = 0; c < SF_OBS_CH / 8; ++c)
+            reinterpret_cast<uint4 *>(row)[c] = make_uint4(wv[4 * c], wv[4 * c + 1], wv[4 * c + 2], wv[4 * c + 3]);
+    } else { /* 68-byte rows, 4-byte aligned */
+#pragma unroll
+        for (int c = 0; c < SF_OBS_CH / 2; ++c) reinterpret_cast<uint32_t *>(row)[c] = wv[c];
+    }
+}
+
 /* (arena, observed human slot) of work item `item` */
 __device__ __forceinline__ void sf_obs_item(int item, int nsel, uint32_t agent_mask, int *env, int *slot)
 {
@@ -251,17 +301,115 @@ __device__ __forceinline__ void sf_obs_item(int item, int nsel, uint32_t agent_m
     *env = item / nsel, *slot = __ffs(m) - 1;
 }
 
+/* The copy-out of one window in a half type T from the converted table `feat` (see sf_observe_kernel for the
+   fp32 loops, which these follow); a chunk is eight 2-byte values. */
+template <bool NHWC, typename T>
+__device__ __forceinline__ void sf_obs_copy_out_half(const SfDev &d, const SfConst &k, const SfTabs &t, int env, const SfEnv &e,
+                                                     int vcell, uint32_t team, const int16_t *bmap, const int16_t *tmap,
+                                                     const uint16_t *code, const T *feat, uint4 *dst, uint32_t *fb)
+{
+    constexpr int PITCH = sf_obs_pitch<T, NHWC>();
+    if constexpr (NHWC) {
+        /* the 32 features of a cell are one 64-byte table row = four chunks; chunk idx covers features
+           8p..8p+7 of window cell idx / 4 */
+#pragma unroll 4
+        for (int idx = threadIdx.x; idx < SF_OBS_CELLS * (SF_OBS_CH / 8); idx += SF_OBS_CTA) {
+            const int w = idx / (SF_OBS_CH / 8), p = idx % (SF_OBS_CH / 8);
+            const uint32_t cd = code[w];
+            uint4 v = make_uint4(0u, 0u, 0u, 0u);
+            if (cd == SF_OBS_BEYOND) { /* more dynamic cells than table rows (rare) */
+                const int cell = sf_obs_cell(vcell, w / SF_OBS_WIN, w % SF_OBS_WIN);
+                int32_t f[32];
+                sf_describe_cell(d, k, env, e, cell, t.smap[cell], SF_G(cell), team, bmap[w], tmap[w], f);
+                int32_t g[8];
+#pragma unroll
+                for (int i = 0; i < 8; ++i) g[i] = 0;
+#pragma unroll
+                for (int c = 0; c < SF_OBS_CH / 8; ++c)
+                    if (c == p) {
+#pragma unroll
+                        for (int i = 0; i < 8; ++i) g[i] = f[8 * c + i];
+                    }
+                uint32_t wv[4];
+#pragma unroll
+                for (int i = 0; i < 4; ++i)
+                    wv[i] = sf_obs_pack2<T>(g[2 * i] ? sf_obs_transform(d, g[2 * i], fb) : 0.f,
+                                            g[2 * i + 1] ? sf_obs_transform(d, g[2 * i + 1], fb) : 0.f);
+                v = make_uint4(wv[0], wv[1], wv[2], wv[3]);
+            } else if (cd) {
+                v = *reinterpret_cast<const uint4 *>(feat + cd * PITCH + 8 * p);
+            }
+            __stcs(dst + idx, v);
+        }
+    } else {
+        /* [32][31][31]: 961 = 1 (mod 8), so every eight channels are exactly 961 chunks and chunk q covers the
+           same (channel offset, cell) octuple in each of the four 8-channel groups: a thread reads the eight
+           codes of its chunk once and writes the chunk of every group, eight predicated 2-byte table reads and
+           one 16-byte store each.  The warp stores of group g start 16 g bytes off a 512-byte boundary, as in
+           the fp32 loop. */
+        const uint16_t *hf = reinterpret_cast<const uint16_t *>(feat);
+        for (int q = threadIdx.x; q < SF_OBS_CELLS; q += SF_OBS_CTA) {
+            int cc = (8 * q) / SF_OBS_CELLS, w = 8 * q - cc * SF_OBS_CELLS; /* channel offset in the group, window cell */
+            int row[8]; /* table offset of element j of the chunk: row * pitch + channel offset, -1 = zero */
+            bool beyond = false;
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+                const uint32_t cd = code[w];
+                row[j] = cd ? (int)cd * PITCH + cc : -1;
+                if (cd == SF_OBS_BEYOND) beyond = true, row[j] = -2 - w;
+                if (++w == SF_OBS_CELLS) w = 0, ++cc;
+            }
+            if (!beyond) {
+#pragma unroll
+                for (int g = 0; g < SF_OBS_CH / 8; ++g) {
+                    uint32_t wv[4];
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) {
+                        const uint32_t lo = row[2 * j] >= 0 ? hf[row[2 * j] + 8 * g] : 0u;
+                        const uint32_t hi = row[2 * j + 1] >= 0 ? hf[row[2 * j + 1] + 8 * g] : 0u;
+                        wv[j] = lo | hi << 16;
+                    }
+                    __stcs(dst + g * SF_OBS_CELLS + q, make_uint4(wv[0], wv[1], wv[2], wv[3]));
+                }
+            } else { /* more dynamic cells than table rows (rare): those are described here, once per chunk */
+                uint32_t val[8][SF_OBS_CH / 8];
+                int cj = (8 * q) / SF_OBS_CELLS, wj = 8 * q - cj * SF_OBS_CELLS;
+#pragma unroll 1
+                for (int j = 0; j < 8; ++j) {
+                    if (row[j] <= -2) {
+                        const int cell = sf_obs_cell(vcell, wj / SF_OBS_WIN, wj % SF_OBS_WIN);
+                        int32_t f[32];
+                        sf_describe_cell(d, k, env, e, cell, t.smap[cell], SF_G(cell), team, bmap[wj], tmap[wj], f);
+                        for (int g = 0; g < SF_OBS_CH / 8; ++g)
+                            val[j][g] = f[8 * g + cj] ? sf_obs_pack2<T>(sf_obs_transform(d, f[8 * g + cj], fb), 0.f) & 0xFFFFu : 0u;
+                    } else {
+                        for (int g = 0; g < SF_OBS_CH / 8; ++g) val[j][g] = row[j] >= 0 ? hf[row[j] + 8 * g] : 0u;
+                    }
+                    if (++wj == SF_OBS_CELLS) wj = 0, ++cj;
+                }
+                for (int g = 0; g < SF_OBS_CH / 8; ++g)
+                    __stcs(dst + g * SF_OBS_CELLS + q, make_uint4(val[0][g] | val[1][g] << 16, val[2][g] | val[3][g] << 16,
+                                                                  val[4][g] | val[5][g] << 16, val[6][g] | val[7][g] << 16));
+            }
+        }
+    }
+}
+
 /* NHWC: the same values with the channel innermost, SF_OBS_NHWC of the header.  LIST (sf_observe_list): the
    arena of row r is env_ids[r / nsel] instead of r / nsel, an id outside [0, n_envs) gives a zero row, and the
-   rows written are min(*list_n, n_items / nsel) (list_n == NULL: all); the launch shape is chosen for n_items. */
-template <bool NHWC, bool LIST>
+   rows written are min(*list_n, n_items / nsel) (list_n == NULL: all); the launch shape is chosen for n_items.
+   T: the output element type, float, or __half / __nv_bfloat16 (SF_OBS_F16 / SF_OBS_BF16): the fp32 values
+   converted to nearest even. */
+template <bool NHWC, bool LIST, typename T>
 __global__ void __launch_bounds__(SF_OBS_CTA, SF_OBS_CTAS_PER_SM)
-sf_observe_kernel(const SfDev d, const __grid_constant__ SfConst k, float *__restrict__ obs, uint32_t agent_mask,
+sf_observe_kernel(const SfDev d, const __grid_constant__ SfConst k, T *__restrict__ obs, uint32_t agent_mask,
                   int nsel, int n_items, int rows, int run_len, const int32_t *__restrict__ env_ids,
                   const int32_t *__restrict__ list_n)
 {
-    float *feat = reinterpret_cast<float *>(sf_smem);                         /* [row][SF_OBS_PITCH] */
-    uint16_t *code = reinterpret_cast<uint16_t *>(feat + SF_OBS_ROWS * SF_OBS_PITCH); /* per window cell */
+    constexpr bool F32 = std::is_same<T, float>::value;
+    constexpr int PITCH = sf_obs_pitch<T, NHWC>();
+    T *feat = reinterpret_cast<T *>(sf_smem);                                  /* [row][PITCH] */
+    uint16_t *code = reinterpret_cast<uint16_t *>(feat + SF_OBS_ROWS * PITCH); /* per window cell */
     uint16_t *dlist = code + SF_OBS_LIST;                                     /* window index of dynamic cell i */
     int16_t *bmap = reinterpret_cast<int16_t *>(dlist + SF_OBS_LIST);
     int16_t *tmap = bmap + SF_OBS_LIST;
@@ -274,8 +422,12 @@ sf_observe_kernel(const SfDev d, const __grid_constant__ SfConst k, float *__res
         e0.mb[0] = e0.mb[1] = 0, e0.ntemp = 0, e0.level = 1, e0.hw_h = 0, e0.env = 0;
         int32_t f[32];
         sf_describe_cell(d, k, 0, e0, 0, threadIdx.x, 0u, 0u, -1, -1, f);
+        if constexpr (F32) {
 #pragma unroll
-        for (int c = 0; c < SF_OBS_CH; ++c) feat[threadIdx.x * SF_OBS_PITCH + c] = f[c] ? sf_obs_transform(d, f[c], &fb) : 0.f;
+            for (int c = 0; c < SF_OBS_CH; ++c) feat[threadIdx.x * SF_OBS_PITCH + c] = f[c] ? sf_obs_transform(d, f[c], &fb) : 0.f;
+        } else {
+            sf_obs_put_half_row<T, NHWC>(d, feat + threadIdx.x * PITCH, f, &fb);
+        }
     }
     constexpr int PER = (SF_OBS_CELLS + SF_OBS_CTA - 1) / SF_OBS_CTA;
     if constexpr (LIST) {
@@ -291,7 +443,7 @@ sf_observe_kernel(const SfDev d, const __grid_constant__ SfConst k, float *__res
             listed = id >= 0 && id < d.n_envs;
             env = listed ? id : 0;
         }
-        float *out = obs + (size_t)item * SF_OBS_LEN;
+        T *out = obs + (size_t)item * SF_OBS_LEN;
         /* the few header words the features need */
         SfEnv e;
         const uint32_t misc = d.misc[env];
@@ -364,8 +516,12 @@ sf_observe_kernel(const SfDev d, const __grid_constant__ SfConst k, float *__res
             const int w = dlist[i], cell = sf_obs_cell(vcell, w / SF_OBS_WIN, w % SF_OBS_WIN);
             int32_t f[32];
             sf_describe_cell(d, k, env, e, cell, t.smap[cell], SF_G(cell), team, bmap[w], tmap[w], f);
+            if constexpr (F32) {
 #pragma unroll
-            for (int c = 0; c < SF_OBS_CH; ++c) feat[(16 + i) * SF_OBS_PITCH + c] = f[c] ? sf_obs_transform(d, f[c], &fb) : 0.f;
+                for (int c = 0; c < SF_OBS_CH; ++c) feat[(16 + i) * SF_OBS_PITCH + c] = f[c] ? sf_obs_transform(d, f[c], &fb) : 0.f;
+            } else {
+                sf_obs_put_half_row<T, NHWC>(d, feat + (16 + i) * PITCH, f, &fb);
+            }
         }
         __syncthreads();
         /* the copy-out: no barrier, no shared-memory buffer between the table and HBM; every store instruction
@@ -376,7 +532,9 @@ sf_observe_kernel(const SfDev d, const __grid_constant__ SfConst k, float *__res
            chunks first and the others in a second pass, lane-dense (41% slower: partial-warp stores); a warp
            vote that sends 128 empty cells in a row down a store-only path (7% slower) */
         float4 *dst = reinterpret_cast<float4 *>(out);
-        if constexpr (NHWC) {
+        if constexpr (!F32) {
+            sf_obs_copy_out_half<NHWC, T>(d, k, t, env, e, vcell, team, bmap, tmap, code, feat, reinterpret_cast<uint4 *>(dst), &fb);
+        } else if constexpr (NHWC) {
             /* channel-innermost: the 32 features of a cell are one table row = eight chunks; chunk idx
                covers features 4p..4p+3 of window cell idx / 8 */
 #pragma unroll 4
@@ -956,10 +1114,15 @@ int sf_create(const sf_config *cfg, sf_handle **out)
     SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_B>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
     SF_CREATE_CUDA(cudaFuncSetAttribute(sf_reset_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
     SF_CREATE_CUDA(cudaFuncSetAttribute(sf_rng_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
-    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_observe_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_OBS_SMEM));
-    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_observe_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_OBS_SMEM));
-    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_observe_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_OBS_SMEM));
-    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_observe_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_OBS_SMEM));
+#define SF_OBS_SMEM_ATTR(NHWC, LIST, T) \
+    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_observe_kernel<NHWC, LIST, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, sf_obs_smem<T, NHWC>()))
+#define SF_OBS_SMEM_ATTRS(T) \
+    SF_OBS_SMEM_ATTR(false, false, T); SF_OBS_SMEM_ATTR(true, false, T); SF_OBS_SMEM_ATTR(false, true, T); SF_OBS_SMEM_ATTR(true, true, T)
+    SF_OBS_SMEM_ATTRS(float);
+    SF_OBS_SMEM_ATTRS(__half);
+    SF_OBS_SMEM_ATTRS(__nv_bfloat16);
+#undef SF_OBS_SMEM_ATTRS
+#undef SF_OBS_SMEM_ATTR
     rc = sf_launch_reset(h, nullptr, h->d.n_envs, nullptr, nullptr, 0);
     if (rc == SF_OK) {
         cudaError_t e_ = cudaDeviceSynchronize();
@@ -1106,11 +1269,13 @@ int sf_synth_actions(sf_handle *h, uint8_t *actions, uint64_t t, const char *tab
 
 /* the checks and the launch sf_observe and sf_observe_list share: n_rows rows of observations (arenas 0..n_rows-1,
    or env_ids[0..n_rows) with *count of them written) */
-static int sf_launch_observe(sf_handle *h, const char *fn, float *obs, int32_t phase, uint32_t agent_mask, int n_rows,
+static int sf_launch_observe(sf_handle *h, const char *fn, void *obs, int32_t phase, uint32_t agent_mask, int n_rows,
                              const int32_t *env_ids, const int32_t *count, cudaStream_t s)
 {
     const bool nhwc = (phase & SF_OBS_NHWC) != 0;
-    phase &= ~SF_OBS_NHWC;
+    const int32_t fmt = phase & (SF_OBS_F16 | SF_OBS_BF16);
+    if (fmt == (SF_OBS_F16 | SF_OBS_BF16)) return sf_fail(h, SF_ERR_ARG, std::string(fn) + ": SF_OBS_F16 and SF_OBS_BF16 exclude each other");
+    phase &= ~(SF_OBS_NHWC | SF_OBS_F16 | SF_OBS_BF16);
     if (phase != SF_OBS_P1 && phase != SF_OBS_P2) return sf_fail(h, SF_ERR_ARG, std::string(fn) + ": phase must be SF_OBS_P1 or SF_OBS_P2");
     /* the kernel describes the arena as it stands; the phase says WHERE in the step the caller claims
        to be, and a claim that does not match the handle is an error: P2 is the point between
@@ -1132,9 +1297,15 @@ static int sf_launch_observe(sf_handle *h, const char *fn, float *obs, int32_t p
         for (run_len = 16; run_len > 1 && n_items / run_len < 4 * ctas; run_len >>= 1) {}
     int runs = (n_items + run_len - 1) / run_len;
     int grid = runs < ctas ? runs : ctas;
-#define SF_OBS_LAUNCH(NHWC, LIST)                                                                                          \
-    sf_observe_kernel<NHWC, LIST><<<grid, SF_OBS_CTA, SF_OBS_SMEM, s>>>(h->d, h->k, obs, agent_mask, nsel, n_items, h->obs_rows, \
-                                                                        run_len, env_ids, count)
+#define SF_OBS_LAUNCH_T(NHWC, LIST, T)                                                                                     \
+    sf_observe_kernel<NHWC, LIST, T><<<grid, SF_OBS_CTA, sf_obs_smem<T, NHWC>(), s>>>(h->d, h->k, static_cast<T *>(obs), agent_mask, \
+                                                                                     nsel, n_items, h->obs_rows, run_len, env_ids, count)
+#define SF_OBS_LAUNCH(NHWC, LIST)                                                    \
+    do {                                                                             \
+        if (fmt == SF_OBS_F16) SF_OBS_LAUNCH_T(NHWC, LIST, __half);                  \
+        else if (fmt == SF_OBS_BF16) SF_OBS_LAUNCH_T(NHWC, LIST, __nv_bfloat16);     \
+        else SF_OBS_LAUNCH_T(NHWC, LIST, float);                                     \
+    } while (0)
     if (env_ids) {
         if (nhwc) SF_OBS_LAUNCH(true, true);
         else SF_OBS_LAUNCH(false, true);
@@ -1143,18 +1314,19 @@ static int sf_launch_observe(sf_handle *h, const char *fn, float *obs, int32_t p
         else SF_OBS_LAUNCH(false, false);
     }
 #undef SF_OBS_LAUNCH
+#undef SF_OBS_LAUNCH_T
     h->launches += 1;
     SF_CUDA(h, cudaGetLastError());
     return SF_OK;
 }
 
-int sf_observe(sf_handle *h, float *obs, int32_t phase, uint32_t agent_mask, void *stream)
+int sf_observe(sf_handle *h, void *obs, int32_t phase, uint32_t agent_mask, void *stream)
 {
     if (!h || !obs) return h ? sf_fail(h, SF_ERR_ARG, "sf_observe: null buffer") : SF_ERR_ARG;
     return sf_launch_observe(h, "sf_observe", obs, phase, agent_mask, h->d.n_envs, nullptr, nullptr, static_cast<cudaStream_t>(stream));
 }
 
-int sf_observe_list(sf_handle *h, float *obs, int32_t phase, uint32_t agent_mask, const int32_t *env_ids, const int32_t *count,
+int sf_observe_list(sf_handle *h, void *obs, int32_t phase, uint32_t agent_mask, const int32_t *env_ids, const int32_t *count,
                     int32_t n_max, void *stream)
 {
     if (!h || !obs || !env_ids) return h ? sf_fail(h, SF_ERR_ARG, "sf_observe_list: null buffer") : SF_ERR_ARG;

@@ -19,6 +19,9 @@ from . import data as sfdata
 from .lib import check, lib
 
 
+_OBS_FORMAT = {torch.float32: 0, torch.float16: sfcfg.OBS_F16, torch.bfloat16: sfcfg.OBS_BF16}
+
+
 class BatchedArena:
     def __init__(self, n_envs, mode="Solo", level=1, level_max=None, squad_agents=False, auto_reset=True,
                  max_steps=0, env_id_base=0, player="account1", caps=None, arena=None, device=None, teams=None, sheets=None,
@@ -104,9 +107,14 @@ class BatchedArena:
         return out
 
     # ------------------------------------------------------------------ observation / readback
-    def observe(self, agent_mask=1, phase=sfcfg.OBS_P1, out=None, channels_last=False, env_ids=None, count=None):
+    def observe(self, agent_mask=1, phase=sfcfg.OBS_P1, out=None, channels_last=False, env_ids=None, count=None,
+                dtype=torch.float32):
         """gameplay::bot() up to Agent::predict (bots/bot-0.5/Custom.hpp:137-158): fp32 device
         tensor [n_envs, n_selected, 32, 31, 31].
+
+        ``dtype=torch.float16`` or ``torch.bfloat16`` (SF_OBS_F16 / SF_OBS_BF16) writes half the bytes: every
+        element equals ``.to(dtype)`` of the fp32 observation (round to nearest even), written by the
+        observation kernel itself.  ``out`` must then have that dtype.
 
         ``channels_last=True`` returns a tensor of the same shape and values whose MEMORY is
         [n_envs, n_selected, 31, 31, 32] (SF_OBS_NHWC): ``.flatten(0, 1)`` of it is a channels-last batch that
@@ -118,6 +126,7 @@ class BatchedArena:
         With ``count`` (an int32 CUDA tensor [1], e.g. from ``list_finished``) only the first min(count, n_max)
         rows are written, with no host synchronisation; rows at and beyond ``count`` are whatever ``out`` held
         (uninitialised memory when ``out`` is None)."""
+        assert dtype in _OBS_FORMAT, "observations are float32, float16 or bfloat16"
         nsel = bin(agent_mask).count("1")
         W, CH = sfcfg.OBS_WIN, sfcfg.OBS_CH
         rows = self.n_envs
@@ -130,10 +139,10 @@ class BatchedArena:
             assert count is None, "count goes with env_ids"
         if out is None:
             out = torch.empty((rows, nsel, W, W, CH) if channels_last else (rows, nsel, CH, W, W),
-                              dtype=torch.float32, device=self.device)
-        assert out.is_cuda and out.dtype == torch.float32 and out.is_contiguous()
+                              dtype=dtype, device=self.device)
+        assert out.is_cuda and out.dtype == dtype and out.is_contiguous()
         assert out.numel() == rows * nsel * sfcfg.OBS_LEN
-        ph = phase | (sfcfg.OBS_NHWC if channels_last else 0)
+        ph = phase | (sfcfg.OBS_NHWC if channels_last else 0) | _OBS_FORMAT[dtype]
         if env_ids is None:
             self._chk(lib().sf_observe(self._h, C.c_void_p(out.data_ptr()), ph, agent_mask, self._stream()))
         else:
