@@ -243,6 +243,24 @@ int sf_reset_finished(sf_handle *h, void *stream);
 int sf_observe_list(sf_handle *h, void *obs, int32_t phase, uint32_t agent_mask, const int32_t *env_ids,
                     const int32_t *count, int32_t n_max, void *stream);
 
+/* sf_step for a DEVICE list of arenas (DESIGN.md section 7d): advance some arenas and hold the rest, e.g. the K
+   children of a clone in a search, or the arenas an asynchronous actor has actions for.  The list rules are those
+   of sf_observe_list: entries i < min(*count, n_max) of env_ids (DEVICE int32 [n_max]; count: DEVICE int32, NULL =
+   n_max; both 4-byte aligned) are live, 1 <= n_max <= n_envs, and row i of actions (DEVICE uint8
+   [n_max][agents_per_env], the symbols of sf_step) is the command row of arena env_ids[i].
+   - A listed arena ends the call byte for byte as sf_step with that row would leave it: its state, auto-reset at
+     the end of the step and the pending random stream included, its sf_step_out row and its sf_save record.
+   - Every word of an unlisted arena is untouched, its sf_step_out row too (it still describes the last step that
+     arena took).  The SF_STAT_* statistics add up over the stepped arenas only.
+   - An id outside [0, n_envs) is skipped.  An id listed more than once is stepped once, with the row of its lowest
+     list index; its later entries are ignored.  A skipped or ignored entry writes nothing and counts nothing.
+   - SF_ERR_ARG between sf_step_a and sf_step_b, for a NULL actions or env_ids, a misaligned env_ids or count, and
+     n_max out of range.  The call neither opens nor closes a split step.
+   Stream order, no host synchronisation: the call can be captured in a CUDA graph.  A caller probes for it by
+   looking the symbol up (SF_ABI_VERSION stays 3). */
+int sf_step_list(sf_handle *h, const uint8_t *actions, const int32_t *env_ids, const int32_t *count, int32_t n_max,
+                 void *stream);
+
 /* Copy a per-arena field into a DEVICE buffer (sizes above). */
 int sf_get(sf_handle *h, int32_t field, void *dev_out, void *stream);
 

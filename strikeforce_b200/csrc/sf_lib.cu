@@ -99,33 +99,73 @@ __device__ __forceinline__ void sf_flush_stats(const SfDev &d, const SfStatDelta
  * are (the tick is a serial chain, and the 32 arenas of a warp execute the union of their
  * branches), so a batch that would leave warp slots empty is spread over more warps with fewer
  * arenas each (sf_launch_step picks lpw): the extra lanes idle, the chain of every warp gets
- * shorter because fewer arenas diverge in it. */
-template <int HALF>
+ * shorter because fewer arenas diverge in it.
+ *
+ * LIST (sf_step_list, DESIGN.md section 7d): the work items are the entries i < min(*list_n, n_max) of the device
+ * list env_ids instead of the arenas; entry i steps arena env_ids[i] with action row i, if the id is in range and
+ * the entry owns it (claim[id] == i, set by sf_claim_kernel).  lpw <= 0 picks the arenas per warp here, from the
+ * count, by sf_launch_step's rule, so that ids in order with count = n_envs are chunked exactly as sf_step does. */
+template <int HALF, bool LIST>
 __global__ void __launch_bounds__(SF_CTA, 1)
-sf_step_kernel(const SfDev d, const __grid_constant__ SfConst k, const uint8_t *__restrict__ actions, int lpw)
+sf_step_kernel(const SfDev d, const __grid_constant__ SfConst k, const uint8_t *__restrict__ actions, int lpw,
+               const int32_t *__restrict__ env_ids, const int32_t *__restrict__ list_n, int n_max,
+               const int32_t *__restrict__ claim)
 {
     SfTabs t;
     sf_stage_tables(d, t);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int nchunks = (d.n_envs + lpw - 1) / lpw;
+    int n_list = 0; /* LIST: the live entries; every thread reads the count, so that every warp makes the same number of passes */
+    if constexpr (LIST) {
+        n_list = list_n ? min(max(*list_n, 0), n_max) : n_max;
+        if (lpw <= 0)
+            for (lpw = 1; lpw < 32 && (n_list + lpw - 1) / lpw > (int)gridDim.x * (SF_CTA / 32);) lpw *= 2;
+    }
+/* work items: d.n_envs is read where it is used, as it was before LIST existed (a local copy of it changes the
+   register allocation of the <HALF, false> kernels, whose SASS is held to that of sf_step) */
+#define SF_STEP_ITEMS (LIST ? n_list : d.n_envs)
+    const int nchunks = (SF_STEP_ITEMS + lpw - 1) / lpw;
 #ifndef SF_NO_PHASE_BARRIERS
     /* every warp of the CTA makes the same number of passes (a pass without a chunk walks through
        with all lanes off), so that the phase barriers of sf_step_halves line up */
     const int per_pass = gridDim.x * (SF_CTA / 32);
     for (int base = 0; base < nchunks; base += per_pass) {
         const int chunk = base + blockIdx.x + gridDim.x * warp;
-        bool valid = chunk < nchunks && lane < lpw && chunk * lpw + lane < d.n_envs;
+        bool valid = chunk < nchunks && lane < lpw && chunk * lpw + lane < SF_STEP_ITEMS;
         int env = valid ? chunk * lpw + lane : lane; /* an idle lane reads some arena's header and writes nothing */
 #else
     for (int chunk = blockIdx.x + gridDim.x * warp; chunk < nchunks; chunk += gridDim.x * (SF_CTA / 32)) {
-        bool valid = lane < lpw && chunk * lpw + lane < d.n_envs;
+        bool valid = lane < lpw && chunk * lpw + lane < SF_STEP_ITEMS;
         int env = valid ? chunk * lpw + lane : lane;
 #endif
         SfStatDelta sd;
         memset(&sd, 0, sizeof sd);
-        sf_step_body(d, k, t, env, valid, (actions && valid) ? actions + (size_t)env * k.n_agents : nullptr, HALF, sd);
+        if constexpr (LIST) { /* env is the list entry so far; a skipped or ignored entry idles like a padding lane */
+            const int id = valid ? env_ids[env] : -1;
+            const uint8_t *row = actions + (size_t)env * k.n_agents;
+            valid = id >= 0 && id < d.n_envs && claim[id] == env;
+            sf_step_body(d, k, t, valid ? id : lane, valid, valid ? row : nullptr, HALF, sd);
+        } else {
+            sf_step_body(d, k, t, env, valid, (actions && valid) ? actions + (size_t)env * k.n_agents : nullptr, HALF, sd);
+        }
         __syncwarp();
         sf_flush_stats(d, sd);
+    }
+}
+#undef SF_STEP_ITEMS
+
+/* sf_step_list: entry i < min(*list_n, n_max) with an id in range claims arena env_ids[i] (RELEASE = false:
+   the lowest such entry wins) or gives the claim back (RELEASE = true: the word returns to INT32_MAX, its value
+   between calls) */
+template <bool RELEASE>
+__global__ void sf_claim_kernel(const int32_t *__restrict__ env_ids, const int32_t *__restrict__ list_n, int n_max,
+                                int n_envs, int32_t *claim)
+{
+    const int n = list_n ? min(max(*list_n, 0), n_max) : n_max;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const int id = env_ids[i];
+        if (id < 0 || id >= n_envs) continue;
+        if (RELEASE) claim[id] = INT32_MAX;
+        else atomicMin(&claim[id], i);
     }
 }
 
@@ -914,6 +954,7 @@ struct sf_handle {
     int32_t *d_fin_ids = nullptr; /* sf_reset_finished: the finished arenas, ascending ... */
     int32_t *d_fin_n = nullptr;   /* ... and their number */
     int32_t *d_tile_n = nullptr;  /* sf_list_finished / sf_reset_finished: finished arenas per tile of SF_LIST_TILE */
+    int32_t *d_claim = nullptr;   /* sf_step_list: the list entry that steps each arena; INT32_MAX between calls */
     SfSnapLayout snap;           /* the record layout of sf_save / sf_load (sf_snapshot.cuh) */
     int device = 0, n_sm = 0;
     bool between_halves = false; /* sf_step_a has run, sf_step_b has not: the P2 observation point */
@@ -1016,6 +1057,7 @@ void carve(Carver &c, sf_handle &h)
     c.take(h.d_ids, E), c.take(h.d_tb, E), c.take(h.d_serial, E);
     c.take(h.d_rows, E), c.take(h.d_refused, (size_t)1);
     c.take(h.d_fin_ids, E), c.take(h.d_fin_n, (size_t)1), c.take(h.d_tile_n, (E + SF_LIST_TILE - 1) / SF_LIST_TILE);
+    c.take(h.d_claim, E);
 }
 } // namespace
 
@@ -1109,9 +1151,14 @@ int sf_create(const sf_config *cfg, sf_handle **out)
     SF_CREATE_CUDA(cudaMemcpy(const_cast<uint16_t *>(h->d.log_tab), h->tabs.log_tab.data(), 65536 * 2, cudaMemcpyHostToDevice));
     SF_CREATE_CUDA(cudaMemcpy(const_cast<float *>(h->d.pow_lut), h->tabs.pow_lut.data(), (size_t)SF_POW_LUT_LEN * 4,
                               cudaMemcpyHostToDevice));
-    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_BOTH>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
-    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_A>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
-    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_B>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
+    {
+        const std::vector<int32_t> unclaimed((size_t)h->d.E, INT32_MAX);
+        SF_CREATE_CUDA(cudaMemcpy(h->d_claim, unclaimed.data(), unclaimed.size() * 4, cudaMemcpyHostToDevice));
+    }
+    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_BOTH, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
+    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_A, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
+    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_B, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
+    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_BOTH, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
     SF_CREATE_CUDA(cudaFuncSetAttribute(sf_reset_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
     SF_CREATE_CUDA(cudaFuncSetAttribute(sf_rng_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
 #define SF_OBS_SMEM_ATTR(NHWC, LIST, T) \
@@ -1194,10 +1241,38 @@ static int sf_launch_step(sf_handle *h, int half, const uint8_t *d_actions, cuda
     }
     const int nchunks = (h->d.n_envs + lpw - 1) / lpw;
     int grid = nchunks < h->n_sm ? nchunks : h->n_sm; /* one persistent CTA per SM; warps take chunks round-robin over the CTAs */
-    if (half == SF_HALF_BOTH) sf_step_kernel<SF_HALF_BOTH><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, d_actions, lpw);
-    else if (half == SF_HALF_A) sf_step_kernel<SF_HALF_A><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, nullptr, lpw);
-    else sf_step_kernel<SF_HALF_B><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, d_actions, lpw);
+    if (half == SF_HALF_BOTH)
+        sf_step_kernel<SF_HALF_BOTH, false><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, d_actions, lpw, nullptr, nullptr, 0, nullptr);
+    else if (half == SF_HALF_A)
+        sf_step_kernel<SF_HALF_A, false><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, nullptr, lpw, nullptr, nullptr, 0, nullptr);
+    else sf_step_kernel<SF_HALF_B, false><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, d_actions, lpw, nullptr, nullptr, 0, nullptr);
     h->launches += 1;
+    SF_CUDA(h, cudaGetLastError());
+    return SF_OK;
+}
+
+int sf_step_list(sf_handle *h, const uint8_t *actions, const int32_t *env_ids, const int32_t *count, int32_t n_max, void *stream)
+{
+    if (!h) return SF_ERR_ARG;
+    if (!actions || !env_ids) return sf_fail(h, SF_ERR_ARG, "sf_step_list: null buffer");
+    if (h->between_halves) return sf_fail(h, SF_ERR_ARG, "sf_step_list: the step opened by sf_step_a is still waiting for sf_step_b");
+    if (n_max < 1 || n_max > h->d.n_envs) return sf_fail(h, SF_ERR_ARG, "sf_step_list: n_max must be in [1, n_envs]");
+    if ((reinterpret_cast<uintptr_t>(env_ids) | reinterpret_cast<uintptr_t>(count)) & 3u)
+        return sf_fail(h, SF_ERR_ARG, "sf_step_list: env_ids and count must be 4-byte aligned");
+    SfDeviceGuard guard(h);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    /* claim, step the owners, release (DESIGN.md section 7d).  The step kernel picks the arenas per warp from the
+       device count; its grid is that of sf_launch_step for n_max entries at one arena per warp, which gives
+       sf_step's lpw rule (one persistent CTA per SM, so per_pass = the machine's warp slots) whenever the list
+       is long enough to need more than one arena per warp */
+    const int lpw = h->lanes_per_warp, chunks = lpw > 0 ? (n_max + lpw - 1) / lpw : n_max;
+    const int grid = chunks < h->n_sm ? chunks : h->n_sm;
+    int cgrid = (n_max + 255) / 256;
+    if (cgrid > 4 * h->n_sm) cgrid = 4 * h->n_sm;
+    sf_claim_kernel<false><<<cgrid, 256, 0, s>>>(env_ids, count, n_max, h->d.n_envs, h->d_claim);
+    sf_step_kernel<SF_HALF_BOTH, true><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, actions, lpw, env_ids, count, n_max, h->d_claim);
+    sf_claim_kernel<true><<<cgrid, 256, 0, s>>>(env_ids, count, n_max, h->d.n_envs, h->d_claim);
+    h->launches += 3;
     SF_CUDA(h, cudaGetLastError());
     return SF_OK;
 }

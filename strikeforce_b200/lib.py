@@ -17,7 +17,7 @@ BUILD_SCRIPT = os.path.join(_HERE, "csrc", "build.sh")
 
 EXPORTS = [
     "sf_abi_version", "sf_last_error", "sf_create", "sf_destroy", "sf_reset", "sf_step", "sf_step_a", "sf_step_b",
-    "sf_step_host", "sf_synth_actions", "sf_observe", "sf_list_finished", "sf_reset_finished", "sf_observe_list",
+    "sf_step_host", "sf_step_list", "sf_synth_actions", "sf_observe", "sf_list_finished", "sf_reset_finished", "sf_observe_list",
     "sf_get", "sf_export_env", "sf_snapshot_bytes", "sf_save", "sf_load", "sf_rng_stream", "sf_agents_per_env",
     "sf_num_envs", "sf_launch_count", "sf_device_bytes",
 ]
@@ -60,6 +60,7 @@ def lib():
         L.sf_step_a.argtypes = [vp, vp]
         L.sf_step_b.argtypes = [vp, vp, vp]
         L.sf_step_host.argtypes = [vp, vp, vp, vp]
+        L.sf_step_list.argtypes = [vp, vp, vp, vp, i32, vp]
         L.sf_synth_actions.argtypes = [vp, vp, u64, C.c_char_p, i32, vp]
         L.sf_observe.argtypes = [vp, vp, i32, C.c_uint32, vp]
         L.sf_list_finished.argtypes = [vp, vp, vp, vp]

@@ -84,6 +84,23 @@ class BatchedArena:
         self._chk(lib().sf_step(self._h, self._act_ptr(actions), self._stream()))
         self.step_count += 1
 
+    def step_list(self, actions, env_ids, count=None):
+        """sf_step_list: step the arenas of a device list and leave every other arena untouched.
+        ``env_ids`` is an int32 CUDA tensor [n_max] and ``actions`` a uint8 CUDA tensor [n_max, n_agents] whose row i
+        holds the commands of arena env_ids[i] (the row order of ``observe(env_ids=)``).  With ``count`` (an int32
+        CUDA tensor [1], e.g. from ``list_finished``) only the first min(count, n_max) entries are live.  An id
+        outside [0, n_envs) is skipped; a repeated id is stepped once, with the row of its first entry.  A listed
+        arena ends as ``step`` with its row would leave it; the statistics count the stepped arenas only.  No host
+        synchronisation; ``step_count`` is not advanced (the arenas no longer share one step number)."""
+        assert env_ids.is_cuda and env_ids.dtype == torch.int32 and env_ids.is_contiguous() and env_ids.dim() == 1
+        n_max = env_ids.numel()
+        assert actions.is_cuda and actions.dtype == torch.uint8 and actions.is_contiguous()
+        assert actions.numel() == n_max * self.n_agents
+        if count is not None:
+            assert count.is_cuda and count.dtype == torch.int32 and count.numel() == 1
+        self._chk(lib().sf_step_list(self._h, C.c_void_p(actions.data_ptr()), C.c_void_p(env_ids.data_ptr()),
+                                     None if count is None else C.c_void_p(count.data_ptr()), n_max, self._stream()))
+
     def step_a(self):
         self._chk(lib().sf_step_a(self._h, self._stream()))
 
