@@ -308,6 +308,36 @@ int sf_save(sf_handle *h, const int32_t *env_ids, int32_t n, void *records, void
 int sf_load(sf_handle *h, const int32_t *env_ids, int32_t n, const void *records, int32_t n_records,
             const int32_t *rows, void *stream);
 
+/* sf_save / sf_load for a DEVICE list of arenas (DESIGN.md section 7e): the record calls of a search loop that
+   runs on the device, e.g. clone a root into the K slots a policy picked and restore them afterwards, or a
+   checkpoint of the arenas sf_list_finished just listed.  The list rules are those of sf_observe_list: entries
+   i < min(*count, n_max) of env_ids (DEVICE int32 [n_max]; count: DEVICE int32, NULL = n_max; rows and status
+   DEVICE int32 too; all 4-byte aligned) are live, 1 <= n_max <= n_envs; records is a DEVICE buffer
+   [..][sf_snapshot_bytes], 16-byte aligned.  Stream order, no host synchronisation, no host-side state that
+   changes between calls: both calls can be captured in a CUDA graph.  SF_ERR_ARG between sf_step_a and
+   sf_step_b, for a NULL records or env_ids, misalignment and n_max out of range.  A caller probes for them by
+   looking the symbols up (SF_ABI_VERSION stays 3).
+
+   sf_save_list: row i of records becomes the record of arena env_ids[i] for every live i, byte for byte what
+   sf_save writes for that id.  Duplicate ids are allowed; an id outside [0, n_envs) gives an all-zero row (magic
+   0: no load accepts it).  Rows from min(*count, n_max) to n_max are not written.  One kernel launch.
+
+   sf_load_list: arena env_ids[i] is overwritten with record row rows[i] (rows NULL: row i), as sf_load of that
+   record would leave it (a record of another global id re-seeds the pending stream).  An id outside [0, n_envs)
+   is skipped; an id listed more than once is loaded once, from its lowest live index; skipped and ignored
+   entries are not checked and change nothing.  All or nothing, decided on the device: an owning entry is refused
+   when its row is outside [0, n_records) or its record is not one of this configuration (magic, version, size,
+   fingerprint), and if any is, no arena changes.  *status (DEVICE int32 [1]) is written by every call, the count
+   of 0 included: the number of refused owning entries, so 0 means the listed arenas were loaded.  Every word of
+   an unlisted arena is untouched; the SF_STAT_* statistics are not touched.  Also SF_ERR_ARG for a NULL status,
+   n_records < 1 and rows == NULL with n_records < n_max.  A memset of *status and five kernel launches (claim,
+   check, copy, re-seed, release), which share the claim words of sf_step_list: calls of one handle that use
+   them (sf_step_list, sf_load_list) go to one stream. */
+int sf_save_list(sf_handle *h, void *records, const int32_t *env_ids, const int32_t *count, int32_t n_max,
+                 void *stream);
+int sf_load_list(sf_handle *h, const void *records, int32_t n_records, const int32_t *rows,
+                 const int32_t *env_ids, const int32_t *count, int32_t n_max, int32_t *status, void *stream);
+
 /* Replaces Random::_srand + Random::_rand (random.hpp:54-76) for a batch of independent
    streams: seeds stream i with (tb[i], serial[i]) and writes n_draws outputs per stream into
    the HOST buffer out_host[draw * n_streams + i].  Known-answer tests use it. */

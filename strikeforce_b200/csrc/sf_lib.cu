@@ -751,28 +751,73 @@ __device__ __forceinline__ void sf_snap_block(const SfSnapSeg &g, uint32_t lo, u
 }
 
 /* SAVE: records[i] = arena ids[i] (ids NULL: arena i).  LOAD: arena ids[i] = records[rows[i]] (rows NULL:
-   row i), unless sf_snap_check_kernel refused a referenced record. */
-template <bool SAVE>
-__global__ void __launch_bounds__(SF_SNAP_CTA)
+   row i), unless sf_snap_check_kernel refused a referenced record.
+ *
+ * LIST (sf_save_list / sf_load_list, DESIGN.md section 7e): n is n_max and the entries are i < min(*list_n, n_max);
+ * turns whose tile lies beyond that exit.  Each turn compacts its tile's valid entries into s_env / s_rec (nv of
+ * them), so the copy below is the same code: for a save an entry with an id in [0, n_envs), for a load an entry
+ * that owns its id (claim[id] == i, sf_claim_kernel).  A save writes zeros over the item's bytes of the record of
+ * every other live entry of the tile (the header with item 0), so an out-of-range id gives an all-zero row.
+ * The LIST instantiations ask for 6 CTAs per SM, the occupancy the 40 registers of the others give: left to itself
+ * ptxas aims at 8 for the load and spills inside the SoA copy loop.  (0, for the others: no minimum, as before.) */
+template <bool SAVE, bool LIST>
+__global__ void __launch_bounds__(SF_SNAP_CTA, LIST ? 6 : 0)
 sf_snap_kernel(const __grid_constant__ SfSnapLayout L, int64_t env_id_base, const int32_t *__restrict__ ids, int n,
-               uint8_t *records, const int32_t *__restrict__ rows, const int *refused)
+               uint8_t *records, const int32_t *__restrict__ rows, const int *refused,
+               const int32_t *__restrict__ list_n, int n_envs, const int32_t *__restrict__ claim)
 {
     __shared__ __align__(16) uint8_t stage[SF_SNAP_STAGE];
     __shared__ int s_env[SF_SNAP_TILE];
     __shared__ size_t s_rec[SF_SNAP_TILE]; /* byte offset of the entry's record */
+    __shared__ uint32_t s_nv, s_zero;       /* LIST: valid entries of the turn's tile; live entries a save zeroes */
     if (!SAVE && *reinterpret_cast<const volatile int *>(refused)) return;
+    if constexpr (LIST) n = list_n ? min(max(*list_n, 0), n) : n;
     const long n_work = (long)((n + SF_SNAP_TILE - 1) / SF_SNAP_TILE) * L.n_item;
     for (long w = blockIdx.x; w < n_work; w += gridDim.x) {
         const int tile = (int)(w / L.n_item), item = (int)(w % L.n_item);
         const SfSnapItem it = L.item[item];
-        const int nv = min(SF_SNAP_TILE, n - tile * SF_SNAP_TILE);
+        int nv = min(SF_SNAP_TILE, n - tile * SF_SNAP_TILE);
         __syncthreads(); /* the last turn is done with the stage and the entry table */
-        if (threadIdx.x < nv) {
-            const int i = tile * SF_SNAP_TILE + threadIdx.x;
-            s_env[threadIdx.x] = ids ? ids[i] : i;
-            s_rec[threadIdx.x] = (size_t)(SAVE || !rows ? i : rows[i]) * L.bytes;
+        if constexpr (LIST) {
+            if (threadIdx.x < SF_SNAP_TILE) {
+                const int i = tile * SF_SNAP_TILE + threadIdx.x;
+                const int id = threadIdx.x < nv ? ids[i] : -1;
+                const bool ok = id >= 0 && id < n_envs && (SAVE || claim[id] == i);
+                const uint32_t m = __ballot_sync(0xffffffffu, ok);
+                if (ok) {
+                    const int j = __popc(m & ((1u << threadIdx.x) - 1u));
+                    s_env[j] = id;
+                    s_rec[j] = (size_t)(SAVE || !rows ? i : rows[i]) * L.bytes;
+                }
+                if (threadIdx.x == 0) s_nv = __popc(m), s_zero = SAVE ? ~m & (0xffffffffu >> (SF_SNAP_TILE - nv)) : 0u;
+            }
+            __syncthreads();
+            nv = (int)s_nv;
+            if (SAVE && s_zero) { /* the item's bytes of the record rows of out-of-range ids */
+                uint32_t zlo, zhi;
+                if (it.first >= L.n_soa) {
+                    const SfSnapSeg &g = L.seg[it.first];
+                    zlo = g.off + it.lo, zhi = it.hi == g.elem ? sf_snap_end(L, it.first) : g.off + it.hi;
+                } else {
+                    zlo = item == 0 ? 0u : L.seg[it.first].off, zhi = sf_snap_end(L, it.last - 1);
+                }
+                const int zc = (int)((zhi - zlo) / 16);
+                for (int q = threadIdx.x; q < SF_SNAP_TILE * zc; q += SF_SNAP_CTA) {
+                    const int j = q / zc;
+                    if ((s_zero >> j) & 1u)
+                        __stcs(reinterpret_cast<uint4 *>(records + (size_t)(tile * SF_SNAP_TILE + j) * L.bytes + zlo) + (q - j * zc),
+                               make_uint4(0u, 0u, 0u, 0u));
+                }
+            }
+            if (nv == 0) continue;
+        } else {
+            if (threadIdx.x < nv) {
+                const int i = tile * SF_SNAP_TILE + threadIdx.x;
+                s_env[threadIdx.x] = ids ? ids[i] : i;
+                s_rec[threadIdx.x] = (size_t)(SAVE || !rows ? i : rows[i]) * L.bytes;
+            }
+            __syncthreads();
         }
-        __syncthreads();
         if (it.first >= L.n_soa) {
             const SfSnapSeg &g = L.seg[it.first];
             const uint32_t hi = it.hi == g.elem ? sf_snap_end(L, it.first) - g.off : it.hi; /* the last piece covers the padding */
@@ -819,22 +864,44 @@ sf_snap_kernel(const __grid_constant__ SfSnapLayout L, int64_t env_id_base, cons
     }
 }
 
-/* magic, version, size and fingerprint of every record a load references */
+/* magic, version, size and fingerprint of every record a load references.  LIST (sf_load_list): only the entries
+   i < min(*list_n, n) that own their id are checked, and *refused (the caller's status, zeroed before the launch)
+   counts the refused ones: a row outside [0, n_records) or an incompatible record */
+template <bool LIST>
 __global__ void sf_snap_check_kernel(const __grid_constant__ SfSnapLayout L, const uint8_t *records, const int32_t *rows,
-                                     int n, int *refused)
+                                     int n, int *refused, const int32_t *ids, const int32_t *list_n, int n_envs,
+                                     int n_records, const int32_t *claim)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if constexpr (LIST) {
+        if (i >= (list_n ? min(max(*list_n, 0), n) : n)) return;
+        const int id = ids[i];
+        if (id < 0 || id >= n_envs || claim[id] != i) return;
+        const int row = rows ? rows[i] : i;
+        if (row < 0 || row >= n_records ||
+            !sf_snap_compatible(reinterpret_cast<const uint32_t *>(records + (size_t)row * L.bytes), L))
+            atomicAdd(refused, 1);
+        return;
+    }
     if (i >= n) return;
     const uint32_t *w = reinterpret_cast<const uint32_t *>(records + (size_t)(rows ? rows[i] : i) * L.bytes);
     if (!sf_snap_compatible(w, L)) atomicOr(refused, 1);
 }
 
-/* after the copy: the pending stream of every arena that took a record of another global id */
+/* after the copy: the pending stream of every arena that took a record of another global id.  LIST: the entries
+   i < min(*list_n, n) that own their id */
+template <bool LIST>
 __global__ void sf_snap_reseed_kernel(const SfDev d, const __grid_constant__ SfConst k, const uint8_t *records, uint32_t bytes,
-                                      const int32_t *ids, const int32_t *rows, int n, const int *refused)
+                                      const int32_t *ids, const int32_t *rows, int n, const int *refused,
+                                      const int32_t *list_n, const int32_t *claim)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n || *refused) return;
+    if constexpr (LIST) {
+        if (list_n && i >= *list_n) return;
+        const int id = ids[i];
+        if (id < 0 || id >= d.n_envs || claim[id] != i) return;
+    }
     SfTabs t;
     sf_global_tabs(d, t);
     const uint32_t *w = reinterpret_cast<const uint32_t *>(records + (size_t)(rows ? rows[i] : i) * bytes);
@@ -1559,8 +1626,9 @@ int sf_save(sf_handle *h, const int32_t *env_ids, int32_t n, void *records, void
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     int rc = sf_snap_args(h, "sf_save", env_ids, n, records, false, s);
     if (rc) return rc;
-    sf_snap_kernel<true><<<sf_snap_grid(h, n), SF_SNAP_CTA, 0, s>>>(h->snap, h->k.env_id_base, env_ids ? h->d_ids : nullptr, n,
-                                                                   static_cast<uint8_t *>(records), nullptr, nullptr);
+    sf_snap_kernel<true, false><<<sf_snap_grid(h, n), SF_SNAP_CTA, 0, s>>>(h->snap, h->k.env_id_base, env_ids ? h->d_ids : nullptr, n,
+                                                                          static_cast<uint8_t *>(records), nullptr, nullptr,
+                                                                          nullptr, 0, nullptr);
     h->launches += 1;
     SF_CUDA(h, cudaGetLastError());
     SF_CUDA(h, cudaStreamSynchronize(s)); /* the staging buffers are reused by the next call */
@@ -1585,16 +1653,79 @@ int sf_load(sf_handle *h, const int32_t *env_ids, int32_t n, const void *records
     const uint8_t *rec = static_cast<const uint8_t *>(records);
     const int32_t *d_ids = env_ids ? h->d_ids : nullptr, *d_rows = rows ? h->d_rows : nullptr;
     SF_CUDA(h, cudaMemsetAsync(h->d_refused, 0, sizeof(int), s));
-    sf_snap_check_kernel<<<(n + 255) / 256, 256, 0, s>>>(h->snap, rec, d_rows, n, h->d_refused);
-    sf_snap_kernel<false><<<sf_snap_grid(h, n), SF_SNAP_CTA, 0, s>>>(h->snap, h->k.env_id_base, d_ids, n, const_cast<uint8_t *>(rec),
-                                                                    d_rows, h->d_refused);
-    sf_snap_reseed_kernel<<<(n + 255) / 256, 256, 0, s>>>(h->d, h->k, rec, h->snap.bytes, d_ids, d_rows, n, h->d_refused);
+    sf_snap_check_kernel<false><<<(n + 255) / 256, 256, 0, s>>>(h->snap, rec, d_rows, n, h->d_refused, nullptr, nullptr, 0, 0, nullptr);
+    sf_snap_kernel<false, false><<<sf_snap_grid(h, n), SF_SNAP_CTA, 0, s>>>(h->snap, h->k.env_id_base, d_ids, n, const_cast<uint8_t *>(rec),
+                                                                           d_rows, h->d_refused, nullptr, 0, nullptr);
+    sf_snap_reseed_kernel<false><<<(n + 255) / 256, 256, 0, s>>>(h->d, h->k, rec, h->snap.bytes, d_ids, d_rows, n, h->d_refused,
+                                                                nullptr, nullptr);
     h->launches += 3;
     SF_CUDA(h, cudaGetLastError());
     int refused = 0;
     SF_CUDA(h, cudaMemcpyAsync(&refused, h->d_refused, sizeof refused, cudaMemcpyDeviceToHost, s));
     SF_CUDA(h, cudaStreamSynchronize(s));
     if (refused) return sf_fail(h, SF_ERR_ARG, "sf_load: a record is not one of this configuration (magic, version, size or fingerprint)");
+    return SF_OK;
+}
+
+/* the argument checks sf_save_list and sf_load_list share: nothing here reads a device buffer */
+static int sf_snap_list_args(sf_handle *h, const char *fn, const void *records, const int32_t *env_ids,
+                             const int32_t *count, int32_t n_max)
+{
+    if (!records || !env_ids) return sf_fail(h, SF_ERR_ARG, std::string(fn) + ": null buffer");
+    if (h->between_halves) return sf_fail(h, SF_ERR_ARG, std::string(fn) + ": the step opened by sf_step_a is still waiting for sf_step_b");
+    if (n_max < 1 || n_max > h->d.n_envs) return sf_fail(h, SF_ERR_ARG, std::string(fn) + ": n_max must be in [1, n_envs]");
+    if (reinterpret_cast<uintptr_t>(records) & 15u) return sf_fail(h, SF_ERR_ARG, std::string(fn) + ": records must be 16-byte aligned");
+    if ((reinterpret_cast<uintptr_t>(env_ids) | reinterpret_cast<uintptr_t>(count)) & 3u)
+        return sf_fail(h, SF_ERR_ARG, std::string(fn) + ": env_ids and count must be 4-byte aligned");
+    return SF_OK;
+}
+
+int sf_save_list(sf_handle *h, void *records, const int32_t *env_ids, const int32_t *count, int32_t n_max, void *stream)
+{
+    if (!h) return SF_ERR_ARG;
+    int rc = sf_snap_list_args(h, "sf_save_list", records, env_ids, count, n_max);
+    if (rc) return rc;
+    SfDeviceGuard guard(h);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    sf_snap_kernel<true, true><<<sf_snap_grid(h, n_max), SF_SNAP_CTA, 0, s>>>(h->snap, h->k.env_id_base, env_ids, n_max,
+                                                                            static_cast<uint8_t *>(records), nullptr, nullptr,
+                                                                            count, h->d.n_envs, nullptr);
+    h->launches += 1;
+    SF_CUDA(h, cudaGetLastError());
+    return SF_OK;
+}
+
+int sf_load_list(sf_handle *h, const void *records, int32_t n_records, const int32_t *rows, const int32_t *env_ids,
+                 const int32_t *count, int32_t n_max, int32_t *status, void *stream)
+{
+    if (!h) return SF_ERR_ARG;
+    int rc = sf_snap_list_args(h, "sf_load_list", records, env_ids, count, n_max);
+    if (rc) return rc;
+    if (!status) return sf_fail(h, SF_ERR_ARG, "sf_load_list: null status");
+    if ((reinterpret_cast<uintptr_t>(rows) | reinterpret_cast<uintptr_t>(status)) & 3u)
+        return sf_fail(h, SF_ERR_ARG, "sf_load_list: rows and status must be 4-byte aligned");
+    if (n_records < 1) return sf_fail(h, SF_ERR_ARG, "sf_load_list: n_records must be at least 1");
+    if (!rows && n_records < n_max) return sf_fail(h, SF_ERR_ARG, "sf_load_list: fewer records than entries");
+    SfDeviceGuard guard(h);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const uint8_t *rec = static_cast<const uint8_t *>(records);
+    int *st = reinterpret_cast<int *>(status);
+    /* claim, check (counts the refused owners into *status), copy, re-seed, release (DESIGN.md section 7e).  The
+       copy and the re-seed read *status on the device and do nothing unless it is 0; the release runs either way */
+    int cgrid = (n_max + 255) / 256;
+    if (cgrid > 4 * h->n_sm) cgrid = 4 * h->n_sm;
+    SF_CUDA(h, cudaMemsetAsync(status, 0, sizeof(int32_t), s));
+    sf_claim_kernel<false><<<cgrid, 256, 0, s>>>(env_ids, count, n_max, h->d.n_envs, h->d_claim);
+    sf_snap_check_kernel<true><<<(n_max + 255) / 256, 256, 0, s>>>(h->snap, rec, rows, n_max, st, env_ids, count, h->d.n_envs,
+                                                                  n_records, h->d_claim);
+    sf_snap_kernel<false, true><<<sf_snap_grid(h, n_max), SF_SNAP_CTA, 0, s>>>(h->snap, h->k.env_id_base, env_ids, n_max,
+                                                                             const_cast<uint8_t *>(rec), rows, st, count,
+                                                                             h->d.n_envs, h->d_claim);
+    sf_snap_reseed_kernel<true><<<(n_max + 255) / 256, 256, 0, s>>>(h->d, h->k, rec, h->snap.bytes, env_ids, rows, n_max, st,
+                                                                   count, h->d_claim);
+    sf_claim_kernel<true><<<cgrid, 256, 0, s>>>(env_ids, count, n_max, h->d.n_envs, h->d_claim);
+    h->launches += 5;
+    SF_CUDA(h, cudaGetLastError());
     return SF_OK;
 }
 

@@ -237,23 +237,80 @@ class BatchedArena:
     def _ids(ids):
         return None if ids is None else np.ascontiguousarray(ids, dtype=np.int32).reshape(-1)
 
-    def save(self, env_ids=None, out=None):
-        """Records of arenas ``env_ids`` (default: all, in order) as a uint8 device tensor
-        [n, snapshot_bytes].  A checkpoint on disk is ``save().cpu().numpy()``."""
-        ids = self._ids(env_ids)
-        n = self.n_envs if ids is None else len(ids)
+    @staticmethod
+    def _device_list(t, what):
+        assert t.is_cuda and t.dtype == torch.int32 and t.is_contiguous() and t.dim() == 1, \
+            "%s: an int32 CUDA tensor [n_max]" % what
+        return C.c_void_p(t.data_ptr())
+
+    @staticmethod
+    def _device_count(count):
+        if count is None:
+            return None
+        assert count.is_cuda and count.dtype == torch.int32 and count.numel() == 1
+        return C.c_void_p(count.data_ptr())
+
+    def _record_buffer(self, out, n):
         if out is None:
             out = torch.empty((n, self.snapshot_bytes), dtype=torch.uint8, device=self.device)
         assert out.is_cuda and out.dtype == torch.uint8 and out.is_contiguous()
         assert out.numel() == n * self.snapshot_bytes
+        return out
+
+    def save(self, env_ids=None, out=None, count=None):
+        """Records of arenas ``env_ids`` (default: all, in order) as a uint8 device tensor
+        [n, snapshot_bytes].  A checkpoint on disk is ``save().cpu().numpy()``.
+
+        ``env_ids`` as an int32 CUDA tensor [n_max] (sf_save_list) saves a device list with no host
+        synchronisation: row i is the record of arena env_ids[i] (duplicates allowed, an id outside [0, n_envs)
+        gives an all-zero row that no load accepts).  With ``count`` (an int32 CUDA tensor [1]) only the first
+        min(count, n_max) rows are written; the others are whatever ``out`` held."""
+        if isinstance(env_ids, torch.Tensor) and env_ids.is_cuda:
+            ids = self._device_list(env_ids, "env_ids")
+            out = self._record_buffer(out, env_ids.numel())
+            self._chk(lib().sf_save_list(self._h, C.c_void_p(out.data_ptr()), ids, self._device_count(count),
+                                         env_ids.numel(), self._stream()))
+            return out
+        assert count is None, "count goes with a device env_ids"
+        ids = self._ids(env_ids)
+        n = self.n_envs if ids is None else len(ids)
+        out = self._record_buffer(out, n)
         self._chk(lib().sf_save(self._h, None if ids is None else ids.ctypes.data, n, C.c_void_p(out.data_ptr()),
                                 self._stream()))
         return out
 
-    def load(self, records, env_ids=None, rows=None):
+    def load(self, records, env_ids=None, rows=None, count=None, status=None):
         """Overwrite arenas ``env_ids`` (default: all, in order; distinct) with the records ``records[rows[i]]``
         (default: row i).  ``records`` is a uint8 tensor [n_records, snapshot_bytes] (a host array or tensor is
-        copied to the device first).  Raises (and changes no arena) when a record is not of this configuration."""
+        copied to the device first).  Raises (and changes no arena) when a record is not of this configuration.
+
+        ``env_ids`` as an int32 CUDA tensor [n_max] (sf_load_list) loads a device list with no host
+        synchronisation; ``records`` must then be a CUDA tensor and ``rows`` None or an int32 CUDA tensor [n_max].
+        Only the first min(count, n_max) entries are live (``count``: an int32 CUDA tensor [1], None = all).  An id
+        outside [0, n_envs) is skipped; a repeated id is loaded once, from its first entry.  All or nothing, decided
+        on the device: the int32 CUDA tensor [1] returned (``status``, when given) holds the number of refused
+        entries (a row outside the records, or a record of another configuration), and no arena changed unless it
+        is 0.  It is not read back.
+
+        Broadcast (one root into many slots): ``root = save(root_id)`` once, then ``load(root, slots,
+        rows=zeros)``, with ``zeros`` an int32 CUDA tensor of zeros: every slot reads the same record, which stays
+        in L2, instead of K copies of it."""
+        if isinstance(env_ids, torch.Tensor) and env_ids.is_cuda:
+            ids = self._device_list(env_ids, "env_ids")
+            n_max = env_ids.numel()
+            assert isinstance(records, torch.Tensor) and records.is_cuda and records.dtype == torch.uint8
+            assert records.is_contiguous() and records.numel() % self.snapshot_bytes == 0
+            rws = None if rows is None else self._device_list(rows, "rows")
+            if rows is not None:
+                assert rows.numel() == n_max
+            if status is None:
+                status = torch.empty(1, dtype=torch.int32, device=self.device)
+            assert status.is_cuda and status.dtype == torch.int32 and status.numel() == 1
+            self._chk(lib().sf_load_list(self._h, C.c_void_p(records.data_ptr()), records.numel() // self.snapshot_bytes,
+                                         rws, ids, self._device_count(count), n_max, C.c_void_p(status.data_ptr()),
+                                         self._stream()))
+            return status
+        assert count is None and status is None, "count and status go with a device env_ids"
         records = torch.as_tensor(records)
         if not records.is_cuda:
             records = records.to(self.device)
@@ -266,9 +323,20 @@ class BatchedArena:
         self._chk(lib().sf_load(self._h, None if ids is None else ids.ctypes.data, n, C.c_void_p(records.data_ptr()),
                                 records.shape[0], None if rws is None else rws.ctypes.data, self._stream()))
 
-    def clone(self, src_ids, dst_ids):
+    def clone(self, src_ids, dst_ids, count=None, scratch=None, status=None):
         """Arena dst_ids[i] becomes a copy of arena src_ids[i]: one save of the distinct sources, one load.
-        A copy under another global id goes on with the source's episode and then follows its own seeds."""
+        A copy under another global id goes on with the source's episode and then follows its own seeds.
+
+        With int32 CUDA tensors [n_max] for both lists: ``save(src_ids, out=scratch, count=count)`` and then
+        ``load(scratch, dst_ids, count=count, status=status)``, with no host synchronisation (a CUDA graph can
+        capture it).  ``scratch`` is a uint8 CUDA tensor [n_max, snapshot_bytes] (allocated when None).  Returns
+        the status tensor of the load: 0 when every listed destination was loaded; an out-of-range source gives a
+        zero record, which refuses the whole clone if a destination in range takes it."""
+        if isinstance(src_ids, torch.Tensor) and src_ids.is_cuda:
+            assert isinstance(dst_ids, torch.Tensor) and dst_ids.is_cuda and dst_ids.numel() == src_ids.numel()
+            scratch = self.save(src_ids, out=scratch, count=count)
+            return self.load(scratch, dst_ids, count=count, status=status)
+        assert count is None and scratch is None and status is None, "count, scratch and status go with device lists"
         src = self._ids(src_ids)
         uniq, rows = np.unique(src, return_inverse=True)
         self.load(self.save(uniq), dst_ids, rows=rows)
