@@ -261,6 +261,42 @@ int sf_observe_list(sf_handle *h, void *obs, int32_t phase, uint32_t agent_mask,
 int sf_step_list(sf_handle *h, const uint8_t *actions, const int32_t *env_ids, const int32_t *count, int32_t n_max,
                  void *stream);
 
+/* Action masks (DESIGN.md section 7f): which commands would change the arena if a driven human obeyed them
+   now, so that a search can skip children that equal the idle one and a policy can leave out commands that do
+   nothing.  The alphabet, in bit order, is valid_commands (gameplay.hpp:45) in the reference's order, then '_':
+   bit j of a mask word stands for SF_COMMANDS[j].
+
+   For an arena and an agent slot a (a column of the action row; slot a drives human slot a):
+   - Controllable: the slot's symbol reaches obey.  The arena's status is SF_RUNNING, human a is live, and a is
+     ind, or a Battle Royale player slot that is not a random NPC, or a squad agent (a < agents_per_env) that is
+     not a random NPC (the branches of human_action).  A slot that is not controllable gets mask 0.
+   - Delivered symbol d(s): what human_action hands to obey.  s itself for ind and Battle Royale players; for
+     squad agents s if s is one of "+xzqeawsd", '+' otherwise.
+   - The bit of '+' is set for every controllable slot, so such a mask is never empty.
+   - The bit of '_' is set iff the slot is controllable and d('_') = '_'.
+   - Every other bit s is set iff the slot is controllable and the arena after obey(a, d(s)) differs from the
+     arena after obey(a, '+'), both from the arena as stored now.  "Differs" means the canonical record
+     (sf_canon.h) or the status differs; the teleport and the chest claim at the end of obey are part of both
+     sides, and an SF_OVERFLOW that the command would cause is a difference.  '3' is never set.
+   The mask describes the state at the time of the call and enforces nothing: sf_step obeys every symbol as
+   before.  Between sf_step_a and sf_step_b (P2) the state is exactly what obey starts from, except for the
+   humans that act before slot a in the same human_action.  At P1 (the loop top) half A of the next step
+   (spawns, zombies, bullets) still runs before obey.  The call is allowed at both points. */
+#define SF_COMMANDS "+qe3uzxawsdfghjkl;'cvbnm,./[]_"
+#define SF_N_COMMANDS 30
+
+/* The masks of every arena (env_ids NULL: rows = n_envs, count must be NULL and n_max = n_envs) or of a DEVICE
+   list of arenas with the list rules of sf_observe_list: entries i < min(*count, n_max) of env_ids (DEVICE int32
+   [n_max]; count: DEVICE int32, NULL = n_max) are live, row i belongs to arena env_ids[i], duplicates are
+   allowed, an id outside [0, n_envs) gives an all-zero row, rows from the count up to n_max are not written,
+   1 <= n_max <= n_envs.  mask: DEVICE uint32 [rows][agents_per_env]; mask, env_ids and count 4-byte aligned.
+   One kernel launch in stream order, no host synchronisation, no device memory of its own; it writes nothing
+   in the handle (state, sf_step_out, statistics and records stay as they are).  SF_ERR_ARG for a NULL mask,
+   misalignment, n_max out of range and a count without env_ids.  A caller probes for it by looking the symbol
+   up (SF_ABI_VERSION stays 3). */
+int sf_action_mask(sf_handle *h, uint32_t *mask, const int32_t *env_ids, const int32_t *count, int32_t n_max,
+                   void *stream);
+
 /* Copy a per-arena field into a DEVICE buffer (sizes above). */
 int sf_get(sf_handle *h, int32_t field, void *dev_out, void *stream);
 

@@ -41,6 +41,9 @@ STAT_NAMES = ["steps", "episodes", "wins", "deaths", "timeouts", "truncated", "o
 # valid_commands (gameplay.hpp:45) and the 9 symbols the shipped bots expose (Custom.hpp:162)
 ACTIONS9 = b"+xzqeawsd"
 ACTIONS28 = b"+qeuzxawsdfghjkl;'cvbnm,./[]"
+# SF_COMMANDS: the alphabet of sf_action_mask in bit order (valid_commands, then '_'); bit j stands for COMMANDS[j]
+COMMANDS = b"+qe3uzxawsdfghjkl;'cvbnm,./[]_"
+N_COMMANDS = 30
 
 ERRORS = {0: "ok", -1: "bad argument", -2: "no CUDA device (there is no CPU path)", -3: "CUDA error",
           -4: "unsupported", -5: "out of memory"}

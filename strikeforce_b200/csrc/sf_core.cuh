@@ -527,6 +527,7 @@ SF_FN bool sf_flagged(const SfDev &d, const SfTabs &t, int env, int cell)
  * table, and with BF_SPILL or'ed in: ... in the overlay (the bullet that owns the flag carries
  * that bit: it is the one that takes the flag down again) */
 #define SF_FLAG_NEW 1u
+template <bool kMark = true> /* false: a flag with no room spills in the table's count only (sf_action_mask_slot) */
 SF_FN uint32_t sf_flag_cell(const SfDev &d, const SfTabs &t, int env, int cell)
 {
     const SfBtProbe p = sf_bt_probe(t, cell);
@@ -538,11 +539,11 @@ SF_FN uint32_t sf_flag_cell(const SfDev &d, const SfTabs &t, int env, int cell)
         const uint32_t g = SF_G(cell);
         if (g & C_S2) return BF_SPILL;
         if (!room) {
-            SF_G(cell) = (uint16_t)(g | C_S2);
+            if (kMark) SF_G(cell) = (uint16_t)(g | C_S2);
             return SF_FLAG_NEW | BF_SPILL;
         }
     } else if (!room) {
-        SF_G(cell) = (uint16_t)(SF_G(cell) | C_S2);
+        if (kMark) SF_G(cell) = (uint16_t)(SF_G(cell) | C_S2);
         sf_bt_count(t) = (uint16_t)(n | SF_BT_SPILL);
         return SF_FLAG_NEW | BF_SPILL;
     }
@@ -589,7 +590,9 @@ SF_FN int sf_owner_scan(const SfDev &d, int env, const SfEnv &e, int cell, int s
 /* rebuild the table from the bullet rows (the owning bullets of a resting arena are exact; the
  * spilled flags are in the overlay already).  The flags go in in slot order, not in the order they
  * were raised, so a set that fitted may not fit now: a flag with no room spills here like anywhere
- * else, and its bullet is marked */
+ * else, and its bullet is marked.  kMark = false writes nothing outside the table: such a new spill
+ * raises SF_BT_SPILL but is neither marked nor put into the overlay (see sf_mask_flagged). */
+template <bool kMark = true>
 SF_FN void sf_bt_rebuild(const SfDev &d, const SfTabs &t, int env, const SfEnv &e)
 {
     sf_bt_wipe(t);
@@ -610,8 +613,8 @@ SF_FN void sf_bt_rebuild(const SfDev &d, const SfTabs &t, int env, const SfEnv &
             const uint32_t pj = j == 0 ? pw[0] : j == 1 ? pw[1] : j == 2 ? pw[2] : pw[3];
             if (mj & BF_SPILL) sf_bt_count(t) = (uint16_t)(sf_bt_count(t) | SF_BT_SPILL);
             else if (mj & BF_OWNS) {
-                const uint32_t fl = sf_flag_cell(d, t, env, (int)(pj & POS_CELL));
-                if (fl & BF_SPILL) SF_AT(d.b_meta, b0 + j) = mj | BF_SPILL;
+                const uint32_t fl = sf_flag_cell<kMark>(d, t, env, (int)(pj & POS_CELL));
+                if (kMark && (fl & BF_SPILL)) SF_AT(d.b_meta, b0 + j) = mj | BF_SPILL;
             }
         }
         SF_SYNCWARP();
@@ -1265,7 +1268,9 @@ SF_FN int sf_key_index(int c, int group)
  * Everything a command can need -- the human's own cell, the one cell it can act on (ahead
  * for '[' ']' 'z' 'x', in the walking direction for 'a' 's' 'd' 'w'), and its selection, stamina
  * and mindamage when it fires or consumes -- is loaded up front in one round of independent
- * loads; the rules then run on registers. */
+ * loads; the rules then run on registers.
+ * A change to these rules changes what each command does to the state: sf_action_mask_slot (below)
+ * states for every command when it changes the state, and must be changed with them. */
 SF_FN void sf_obey(const SfDev &d, const SfConst &k, const SfTabs &t, int env, SfEnv &e, int h, int c, uint32_t pw,
                    uint32_t sel)
 {
@@ -1503,6 +1508,125 @@ SF_FN void sf_human_action(const SfDev &d, const SfConst &k, const SfTabs &t, in
         if (e.on && ((live >> h) & 1)) sf_obey(d, k, t, env, e, h, c, pw, sel);
         SF_SYNCWARP();
     }
+}
+
+/* ------------------------------------------------------------------ action masks */
+
+/* Which commands of SF_COMMANDS (strikeforce_b200.h: bit j of a mask word is SF_COMMANDS[j]) would change
+ * the arena if the slot's human obeyed them now (sf_action_mask, DESIGN.md section 7f).  Bit s is set when
+ * the state after sf_obey(a, d(s)) differs from the state after sf_obey(a, '+') in the canonical record or
+ * the status; '+' is always set, '_' by rule.  This is a predicate over what sf_obey reads, not a dry run of
+ * it: every rule below restates one branch of sf_obey, and a change there is a change here. */
+enum {
+    SF_CB_PLUS = 0, SF_CB_Q = 1, SF_CB_E = 2, SF_CB_U = 4, SF_CB_Z = 5, SF_CB_X = 6,
+    SF_CB_A = 7, SF_CB_W = 8, SF_CB_S = 9, SF_CB_D = 10, /* the walks */
+    SF_CB_CONS = 11, SF_CB_THR = 15, SF_CB_WPN = 19,      /* "fghj", "kl;'", "cvbnm,./" */
+    SF_CB_BLOCK = 27, SF_CB_PORTAL = 28, SF_CB_QUIT = 29
+};
+#define SF_MASK_AGENT 0x7E7u /* "+xzqeawsd": what a squad agent's command can be (sf_human_action) */
+
+/* node::s[2] of `cell` after sf_bt_rebuild<false>: as sf_flagged after the step's rebuild.  A flag the
+ * rebuild could not fit is in the overlay when its bullet was marked before; one that spilled only now was
+ * neither put there nor marked, and is found by its owning bullet (one live owner per flagged cell). */
+SF_FN bool sf_mask_flagged(const SfDev &d, const SfTabs &t, int env, const SfEnv &e, int cell)
+{
+    if (sf_flagged(d, t, env, cell)) return true;
+    return (sf_bt_count(t) & SF_BT_SPILL) && sf_owner_scan(d, env, e, cell, -1) >= 0;
+}
+
+/* where the tail of sf_obey (teleport, claim_chest) leaves human h that ends its command on `cell`, whose
+ * word in memory is g_mem (sf_obey holds it only when have_g); cell `from` holds g_from instead of its
+ * stored word (the cell a walk left).  Returns the final cell, | 1 << 16 when a chest is claimed there:
+ * two commands that leave the human with the same value change the canonical record alike. */
+SF_FN uint32_t sf_mask_tail(const SfDev &d, const SfConst &k, const SfTabs &t, int env, const SfEnv &e, int cell,
+                            uint32_t g_mem, bool have_g, int from, uint32_t g_from)
+{
+    uint32_t g = have_g ? g_mem : 0u;
+    const uint32_t stc = t.smap[cell];
+    int pidx = -1;
+    if (stc & (M_UP | M_DOWN)) pidx = (int)(stc >> M_TARGET_SHIFT);
+    else if (((g >> C_KIND_SHIFT) & 7u) == K_ENTRANCE) pidx = SF_T(d.t_pidx, sf_find_built(d, env, e, cell));
+    if (pidx >= 0) {
+        const int dc = sf_exit_cell(d, k, env, pidx);
+        const uint32_t gd = dc == cell ? g_mem : dc == from ? g_from : (uint32_t)SF_G(dc);
+        if (sf_showit(t.smap[dc], gd, false) == SH_EXIT && !sf_mask_flagged(d, t, env, e, dc)) cell = dc, g = gd;
+    }
+    const uint32_t kind = (g >> C_KIND_SHIFT) & 7u;
+    return (uint32_t)cell | (kind >= K_CHEST0 && kind < K_BLOCK ? 1u << 16 : 0u);
+}
+
+/* the mask word of agent slot a (human slot a) of a loaded arena whose flag table sf_bt_rebuild<false> built */
+SF_FN uint32_t sf_action_mask_slot(const SfDev &d, const SfConst &k, const SfTabs &t, int env, const SfEnv &e, int a)
+{
+    if (!e.on || !((e.mh >> a) & 1)) return 0u;
+    /* controllable: the branches of sf_human_action that hand the slot's symbol to obey */
+    const uint32_t sel = SF_AT(d.h_sel, a);
+    uint32_t allowed = ~0u;
+    if (a != k.ind) {
+        if (sel & HS_RNPC) return 0u;
+        if (!(k.mode == SF_MODE_ROYALE && a < k.n_players)) {
+            if (!((sel & HS_AGENT) && a < k.n_agents)) return 0u;
+            allowed = SF_MASK_AGENT; /* any other symbol reaches obey as '+' */
+        }
+    }
+    const uint32_t pw = SF_AT(d.h_pw, a);
+    const int cell = (int)(pw & POS_CELL), way0 = (int)(pw >> POS_HI_SHIFT);
+    const int vec = (int)((sel >> HS_VEC_SHIFT) & 3u) - 1, ind = (int)((sel >> HS_IND_SHIFT) & 15u) - 1;
+    const SfTemplate &tp = sf_tmpl(k, a);
+    const uint32_t cons = SF_AT(d.h_cons, a), thr = SF_AT(d.h_thr, a), bp = SF_AT(d.h_bp, a);
+    const int st = SF_AT(d.h_stam, a);
+    /* '+'; 'q' / 'e' turn; '_' quits */
+    uint32_t m = 1u << SF_CB_PLUS | 1u << SF_CB_Q | 1u << SF_CB_E | 1u << SF_CB_QUIT;
+    /* a selection key selects an item the human has, unless it is the one selected */
+    SF_UNROLL
+    for (int i = 0; i < 4; ++i) {
+        if (((cons >> (8 * i)) & 0xFFu) && !(vec == 0 && ind == i)) m |= 1u << (SF_CB_CONS + i);
+        if (((thr >> (8 * i)) & 0xFFu) && !(vec == 1 && ind == i)) m |= 1u << (SF_CB_THR + i);
+    }
+    SF_UNROLL
+    for (int i = 0; i < 8; ++i)
+        if (((tp.w_owned >> i) & 1u) && !(vec == 2 && ind == i)) m |= 1u << (SF_CB_WPN + i);
+    /* 'u' consumes the selected consumable */
+    if (vec == 0 && ind >= 0 && ((cons >> (8 * ind)) & 0xFFu) >= 1) m |= 1u << SF_CB_U;
+    /* the cell ahead: 'z' 'x' '[' ']' */
+    int na;
+    if (sf_neighbour(cell, way0, &na)) {
+        const uint32_t sa = t.smap[na], ga = SF_G(na);
+        /* a bullet goes in (or the arena overflows): the cell is no wall, and no staircase nobody stands on */
+        const bool shot = !(sa & M_WALL) && (!(sa & (M_UP | M_DOWN)) || (ga & (C_S0 | C_S1)));
+        if (shot) m |= 1u << SF_CB_Z;
+        if (vec == 1 && ind >= 0) { /* a throw spends an item (or drops an empty selection) */
+            if (st + tp.thr[ind].stamina >= 0) m |= 1u << SF_CB_X;
+        } else if (vec == 2 && ind >= 0) { /* a shot costs stamina, and fires if the cell lets it */
+            const int ws = tp.wpn[ind].stamina;
+            if (st + ws >= 0 && (ws != 0 || shot)) m |= 1u << SF_CB_X;
+        }
+        if (sf_showit(sa, ga, false) == SH_DOT && !sf_mask_flagged(d, t, env, e, na)) {
+            if (bp & 0xFFu) m |= 1u << SF_CB_BLOCK;      /* blocks */
+            if (bp & 0xFFFF00u) m |= 1u << SF_CB_PORTAL; /* portals, or a pending exit */
+        }
+    }
+    /* the walks: where the human ends (teleport and chest included) against where '+' leaves it */
+    const uint32_t g0 = SF_G(cell);
+    const uint32_t stay = sf_mask_tail(d, k, t, env, e, cell, g0, (sel & HS_ON_ENT) != 0, -1, 0u);
+    SF_UNROLL
+    for (int dir = 0; dir < 4; ++dir) {
+        int nc;
+        bool moves = false;
+        uint32_t gn = 0;
+        if (sf_neighbour(cell, dir, &nc)) {
+            gn = SF_G(nc);
+            const int sit = sf_showit(t.smap[nc], gn, false);
+            moves = sit == SH_CHEST || sit == SH_UP || sit == SH_DOWN || sit == SH_DOT ||
+                    (sit == SH_EXIT && sf_mask_flagged(d, t, env, e, nc));
+        }
+        const uint32_t end = moves ? sf_mask_tail(d, k, t, env, e, nc, (gn & ~C_OCC) | C_S0 | (uint32_t)a, true, cell,
+                                                  g0 & ~(C_S0 | C_OCC))
+                                   : sf_mask_tail(d, k, t, env, e, cell, g0, true, -1, 0u);
+        /* way - 1: 0 down 's', 1 right 'd', 2 up 'w', 3 left 'a' */
+        if (end != stay) m |= 1u << (dir == 0 ? SF_CB_S : dir == 1 ? SF_CB_D : dir == 2 ? SF_CB_W : SF_CB_A);
+    }
+    return m & allowed;
 }
 
 /* ------------------------------------------------------------------ reset */

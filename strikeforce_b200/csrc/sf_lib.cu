@@ -1002,6 +1002,38 @@ sf_reset_finished_kernel(const SfDev d, const __grid_constant__ SfConst k, const
     }
 }
 
+/* sf_action_mask (DESIGN.md section 7f): one thread per row, walking the slots of its arena.  The arena is picked
+ * up as the step picks it up -- header, then its bullet-flag table rebuilt in this thread's 96 bytes of shared
+ * memory ([8-byte word][thread], as in the step kernel) -- but with sf_bt_rebuild<false>, which writes nothing
+ * outside the table.  Entry i < min(*list_n, n_max) (LIST) or arena i writes row i; an id outside [0, n_envs)
+ * writes zeros.  Every lane of a warp reaches the rebuild, whose loop is warp-uniform. */
+#define SF_MASK_CTA 128
+#define SF_MASK_SMEM (SF_MASK_CTA * SF_BT_ENTRIES * 2)
+template <bool LIST>
+__global__ void __launch_bounds__(SF_MASK_CTA)
+sf_action_mask_kernel(const SfDev d, const __grid_constant__ SfConst k, uint32_t *__restrict__ mask,
+                      const int32_t *__restrict__ env_ids, const int32_t *__restrict__ list_n, int n_max)
+{
+    const int n = LIST ? (list_n ? min(max(*list_n, 0), n_max) : n_max) : d.n_envs;
+    if ((int)blockIdx.x * SF_MASK_CTA >= n) return; /* the whole CTA is beyond the count */
+    SfTabs t;
+    sf_global_tabs(d, t);
+    t.bt = reinterpret_cast<uint16_t *>(sf_smem) + 4 * threadIdx.x;
+    t.bt_stride = SF_MASK_CTA;
+    const int i = (int)blockIdx.x * SF_MASK_CTA + (int)threadIdx.x;
+    const int id = i < n ? (LIST ? env_ids[i] : i) : -1;
+    const bool valid = id >= 0 && id < d.n_envs;
+    const int env = valid ? id : (int)(threadIdx.x & 31); /* an idle lane reads some arena's header (E >= 32) */
+    SfEnv e;
+    sf_load_env(d, env, e);
+    if (!valid) e.on = false;
+    sf_bt_rebuild<false>(d, t, env, e);
+    if (i < n) {
+        uint32_t *row = mask + (size_t)i * k.n_agents;
+        for (int a = 0; a < k.n_agents; ++a) row[a] = valid ? sf_action_mask_slot(d, k, t, env, e, a) : 0u;
+    }
+}
+
 /* ====================================================================== host side */
 
 struct sf_handle {
@@ -1476,6 +1508,26 @@ int sf_observe_list(sf_handle *h, void *obs, int32_t phase, uint32_t agent_mask,
     if ((reinterpret_cast<uintptr_t>(env_ids) | reinterpret_cast<uintptr_t>(count)) & 3u)
         return sf_fail(h, SF_ERR_ARG, "sf_observe_list: env_ids and count must be 4-byte aligned");
     return sf_launch_observe(h, "sf_observe_list", obs, phase, agent_mask, n_max, env_ids, count, static_cast<cudaStream_t>(stream));
+}
+
+int sf_action_mask(sf_handle *h, uint32_t *mask, const int32_t *env_ids, const int32_t *count, int32_t n_max,
+                   void *stream)
+{
+    if (!h) return SF_ERR_ARG;
+    if (!mask) return sf_fail(h, SF_ERR_ARG, "sf_action_mask: null mask");
+    if (!env_ids && count) return sf_fail(h, SF_ERR_ARG, "sf_action_mask: count goes with env_ids");
+    if (!env_ids && n_max != h->d.n_envs) return sf_fail(h, SF_ERR_ARG, "sf_action_mask: without env_ids n_max must be n_envs");
+    if (n_max < 1 || n_max > h->d.n_envs) return sf_fail(h, SF_ERR_ARG, "sf_action_mask: n_max must be in [1, n_envs]");
+    if ((reinterpret_cast<uintptr_t>(mask) | reinterpret_cast<uintptr_t>(env_ids) | reinterpret_cast<uintptr_t>(count)) & 3u)
+        return sf_fail(h, SF_ERR_ARG, "sf_action_mask: mask, env_ids and count must be 4-byte aligned");
+    SfDeviceGuard guard(h);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const int grid = (n_max + SF_MASK_CTA - 1) / SF_MASK_CTA;
+    if (env_ids) sf_action_mask_kernel<true><<<grid, SF_MASK_CTA, SF_MASK_SMEM, s>>>(h->d, h->k, mask, env_ids, count, n_max);
+    else sf_action_mask_kernel<false><<<grid, SF_MASK_CTA, SF_MASK_SMEM, s>>>(h->d, h->k, mask, nullptr, nullptr, n_max);
+    h->launches += 1;
+    SF_CUDA(h, cudaGetLastError());
+    return SF_OK;
 }
 
 /* the two launches of the compaction (see sf_list_count_kernel) */

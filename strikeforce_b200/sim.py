@@ -41,6 +41,7 @@ class BatchedArena:
         self.n_agents = lib().sf_agents_per_env(self._h)
         self.step_count = 0
         self._synth = torch.empty((n_envs, self.n_agents), dtype=torch.uint8, device=self.device)
+        self._mask_bits = {}  # action_mask(table=): bit index of each symbol of a table, on the device
 
     # ------------------------------------------------------------------ lifetime
     def close(self):
@@ -170,6 +171,37 @@ class BatchedArena:
         if channels_last:
             return out.view(rows, nsel, W, W, CH).permute(0, 1, 4, 2, 3)
         return out
+
+    def action_mask(self, env_ids=None, count=None, out=None, table=None):
+        """sf_action_mask: which commands would change each driven human's arena now (include/strikeforce_b200.h,
+        DESIGN.md section 7f).  An int32 CUDA tensor [rows, n_agents] of mask words: bit j stands for
+        ``config.COMMANDS[j]`` (bit 31 is never set); a slot whose human the caller does not drive, or an arena that
+        has ended, gets 0, and every other slot has the bit of '+'.
+
+        ``env_ids`` / ``count`` follow ``observe(env_ids=, count=)``: row i is arena env_ids[i], an id outside
+        [0, n_envs) gives a zero row, rows at and beyond ``count`` are whatever ``out`` held.  With ``table`` (bytes,
+        e.g. ``config.ACTIONS9``) the result is instead a bool CUDA tensor [rows, n_agents, len(table)] whose
+        [..., j] is the bit of table[j], computed on the device.  No host synchronisation either way."""
+        rows = self.n_envs
+        ids = cnt = None
+        if env_ids is not None:
+            ids = self._device_list(env_ids, "env_ids")
+            rows = env_ids.numel()
+            cnt = self._device_count(count)
+        else:
+            assert count is None, "count goes with env_ids"
+        if out is None:
+            out = torch.empty((rows, self.n_agents), dtype=torch.int32, device=self.device)
+        assert out.is_cuda and out.dtype == torch.int32 and out.is_contiguous() and out.numel() == rows * self.n_agents
+        self._chk(lib().sf_action_mask(self._h, C.c_void_p(out.data_ptr()), ids, cnt, rows, self._stream()))
+        if table is None:
+            return out
+        table = bytes(table)
+        bits = self._mask_bits.get(table)
+        if bits is None:  # one copy per table, so that a captured graph holds no host-to-device copy
+            bits = torch.tensor([sfcfg.COMMANDS.index(c) for c in table], dtype=torch.int32, device=self.device)
+            self._mask_bits[table] = bits
+        return ((out.unsqueeze(-1) >> bits) & 1).bool()
 
     # ------------------------------------------------------------------ finished arenas (final observations)
     def list_finished(self, ids=None, count=None):
