@@ -131,7 +131,8 @@ enum {
     SF_FIELD_STATE_HASH = 2, /* uint64[n_envs]: sf_canon.h hash of each arena (parity checks)    */
     SF_FIELD_COUNTERS   = 3, /* int32[n_envs][8]: frame kills teams_kills loot chest steps status hp */
     SF_FIELD_POPULATION = 4, /* int32[n_envs][6]: humans zombies bullets chests built portals    */
-    SF_FIELD_STATS      = 5  /* int64[16] device-reduced episode statistics (see SF_STAT_*)      */
+    SF_FIELD_STATS      = 5, /* int64[16] device-reduced episode statistics (see SF_STAT_*)      */
+    SF_FIELD_AGENT_OUT  = 6  /* sf_agent_out[n_envs][agents_per_env], after sf_enable_agent_out   */
 };
 
 /* slots of SF_FIELD_STATS: sums over the handle's arenas since sf_create (NCCL all-reduce
@@ -296,6 +297,46 @@ int sf_step_list(sf_handle *h, const uint8_t *actions, const int32_t *env_ids, c
    up (SF_ABI_VERSION stays 3). */
 int sf_action_mask(sf_handle *h, uint32_t *mask, const int32_t *env_ids, const int32_t *count, int32_t n_max,
                    void *stream);
+
+/* Per-agent step outputs (DESIGN.md section 7g): what the last step did to each human the caller drives, for a
+   trainer with one row per driven human (the 16 players of a Battle Royale arena, ind and the squad agents) --
+   sf_step_out describes ind alone.  Row (e, a), for arena e and agent slot a (0 <= a < agents_per_env; column a
+   of the action row drives human slot a), describes the last step arena e took through sf_step, sf_step_a +
+   sf_step_b, sf_step_host or sf_step_list (as a listed arena):
+   - SF_AGENT_DRIVEN: slot a was controllable in the state the step started from -- the arena was SF_RUNNING,
+     human a was live, and a is ind, or a Battle Royale player or a squad agent (a < agents_per_env) that is not a
+     random NPC.  This is the rule of sf_action_mask: DRIVEN is exactly "the sf_action_mask word was not 0" just
+     before the step.
+   - SF_AGENT_DIED: DRIVEN, and human a was not live at the end of the step (every way the tick removes a human,
+     '_' included), read before any auto-reset.
+   - d_hp, d_damage, d_effect, d_kills: Hp, Human::damage, Human::effect and Human::kills of human slot a at the end
+     of the step (before any auto-reset) minus at its start.  damage and effect are what the human dealt; kills
+     counts the other-team humans and the zombies it killed (gameplay.hpp:574-634).
+   - A slot that is not DRIVEN gets an all-zero row, e.g. every slot of an arena that had ended and waits for
+     sf_reset_finished.  When row ind is DRIVEN, its d_hp, d_damage and d_effect equal the step's sf_step_out.
+   - After an SF_OVERFLOW or SF_UB_GUARD step only SF_AGENT_DRIVEN is defined (the state is undefined as well).
+   - Rows are those of the last step: sf_step_list leaves the rows of unlisted arenas alone, and sf_reset,
+     sf_reset_finished, sf_load and sf_load_list do not touch rows.  They are not part of an arena record.
+     Between sf_step_a and sf_step_b the rows are unspecified.
+   The values are taken inside the step kernel: a slot freed by a death can hold a spawned NPC a step later, and
+   auto-reset re-creates an arena before the step returns, so reading the state around a step cannot give them.
+   With agent outputs on, the state, sf_step_out, the statistics and the records are byte for byte what they are
+   without. */
+typedef struct sf_agent_out {
+    int32_t flags;    /* SF_AGENT_DRIVEN | SF_AGENT_DIED                      */
+    int32_t d_hp;     /* Hp of human slot a: end of the step minus start       */
+    int32_t d_damage; /* Human::damage delta (dealt), gameplay.hpp:574-634     */
+    int32_t d_effect; /* Human::effect delta (dealt)                           */
+    int32_t d_kills;  /* Human::kills delta (other-team humans and zombies)    */
+} sf_agent_out;
+enum { SF_AGENT_DRIVEN = 1, SF_AGENT_DIED = 2 };
+
+/* Opt in to agent outputs, once per handle: allocates the handle's rows (n_envs * agents_per_env * 20 bytes of
+   device memory, counted by sf_device_bytes), zeroed, and from then on every step call of the handle writes
+   them.  A handle that never calls it runs the step kernels it always ran.  A second call does nothing;
+   SF_ERR_ARG between sf_step_a and sf_step_b.  sf_get(SF_FIELD_AGENT_OUT) reads the rows (one kernel launch; it
+   is SF_ERR_ARG before this call).  A caller probes for it by looking the symbol up (SF_ABI_VERSION stays 3). */
+int sf_enable_agent_out(sf_handle *h);
 
 /* Copy a per-arena field into a DEVICE buffer (sizes above). */
 int sf_get(sf_handle *h, int32_t field, void *dev_out, void *stream);

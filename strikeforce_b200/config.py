@@ -35,6 +35,10 @@ OBS_NHWC = 0x100  # OR-ed into the phase: channel innermost
 OBS_F16, OBS_BF16 = 0x200, 0x400  # OR-ed into the phase (at most one): fp16 / bfloat16 values, rounded to nearest even
 
 FIELD_STEP_OUT, FIELD_STATE_HASH, FIELD_COUNTERS, FIELD_POPULATION, FIELD_STATS = 1, 2, 3, 4, 5
+FIELD_AGENT_OUT = 6  # sf_agent_out [n_envs][n_agents], after sf_enable_agent_out
+# sf_agent_out: the per-agent step outputs (include/strikeforce_b200.h, DESIGN.md section 7g)
+AGENT_DRIVEN, AGENT_DIED = 1, 2  # bits of the flags field
+AGENT_OUT_FIELDS = ("flags", "d_hp", "d_damage", "d_effect", "d_kills")
 STAT_NAMES = ["steps", "episodes", "wins", "deaths", "timeouts", "truncated", "overflows", "ub_guards",
               "kills", "teams_kills", "loot", "rng_draws", "algo_bytes", "reserved0", "reserved1", "reserved2"]
 

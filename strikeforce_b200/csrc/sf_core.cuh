@@ -1555,20 +1555,36 @@ SF_FN uint32_t sf_mask_tail(const SfDev &d, const SfConst &k, const SfTabs &t, i
     return (uint32_t)cell | (kind >= K_CHEST0 && kind < K_BLOCK ? 1u << 16 : 0u);
 }
 
+/* Controllable: the branches of sf_human_action that hand agent slot a's symbol to obey -- a running arena, a live
+ * human a, and a is ind, or a Battle Royale player or a squad agent that is not a random NPC.  The one statement of
+ * the rule, for a function body with `d`, `k`, `env`, `e` and `a` in scope: it returns `no` when slot a is not
+ * controllable, and otherwise leaves the human's word in `sel` and in `allowed` the symbols that reach obey as
+ * themselves (all for ind and the players, SF_MASK_AGENT for a squad agent: any other symbol reaches obey as '+').
+ * sf_action_mask_slot expands it in place and the agent outputs call sf_controllable: a call inside
+ * sf_action_mask_slot gives ptxas another block layout, so that sf_action_mask_kernel would not keep its SASS. */
+#define SF_CONTROLLABLE_RULE(no)                                                                                     \
+    if (!e.on || !((e.mh >> a) & 1)) return no;                                                                     \
+    const uint32_t sel = SF_AT(d.h_sel, a);                                                                         \
+    uint32_t allowed = ~0u;                                                                                         \
+    if (a != k.ind) {                                                                                               \
+        if (sel & HS_RNPC) return no;                                                                               \
+        if (!(k.mode == SF_MODE_ROYALE && a < k.n_players)) {                                                       \
+            if (!((sel & HS_AGENT) && a < k.n_agents)) return no;                                                   \
+            allowed = SF_MASK_AGENT;                                                                                \
+        }                                                                                                           \
+    }
+
+/* slot a is controllable in the arena as loaded (SF_CONTROLLABLE_RULE): DRIVEN of the agent outputs */
+SF_FN bool sf_controllable(const SfDev &d, const SfConst &k, int env, const SfEnv &e, int a)
+{
+    SF_CONTROLLABLE_RULE(false)
+    return allowed != 0u; /* always true here */
+}
+
 /* the mask word of agent slot a (human slot a) of a loaded arena whose flag table sf_bt_rebuild<false> built */
 SF_FN uint32_t sf_action_mask_slot(const SfDev &d, const SfConst &k, const SfTabs &t, int env, const SfEnv &e, int a)
 {
-    if (!e.on || !((e.mh >> a) & 1)) return 0u;
-    /* controllable: the branches of sf_human_action that hand the slot's symbol to obey */
-    const uint32_t sel = SF_AT(d.h_sel, a);
-    uint32_t allowed = ~0u;
-    if (a != k.ind) {
-        if (sel & HS_RNPC) return 0u;
-        if (!(k.mode == SF_MODE_ROYALE && a < k.n_players)) {
-            if (!((sel & HS_AGENT) && a < k.n_agents)) return 0u;
-            allowed = SF_MASK_AGENT; /* any other symbol reaches obey as '+' */
-        }
-    }
+    SF_CONTROLLABLE_RULE(0u)
     const uint32_t pw = SF_AT(d.h_pw, a);
     const int cell = (int)(pw & POS_CELL), way0 = (int)(pw >> POS_HI_SHIFT);
     const int vec = (int)((sel >> HS_VEC_SHIFT) & 3u) - 1, ind = (int)((sel >> HS_IND_SHIFT) & 15u) - 1;
@@ -1890,9 +1906,16 @@ SF_FN void sf_reset_finished_body(const SfDev &d, const SfConst &k, const SfTabs
  *
  * Nothing but `e` stays in registers across the tick: the step output starts as "minus the
  * values at entry" in d.out and gets the values at exit added, and the statistics read the
- * entry values back from the header arrays, which are only overwritten by sf_store_env. */
+ * entry values back from the header arrays, which are only overwritten by sf_store_env.
+ *
+ * AGENTS (sf_enable_agent_out, DESIGN.md section 7g): `ao` is the handle's agent-output buffer,
+ * [field][agent slot][n_envs] int32 with the fields of sf_agent_out, and the rows of the arena are
+ * kept the same way: half A (or the whole step) writes DRIVEN and minus the entry values of each
+ * driven slot, half B (or the whole step) adds the values at exit and DIED, before any auto-reset. */
+#define SF_AO(field, a) ao[((size_t)(field) * (size_t)k.n_agents + (size_t)(a)) * (size_t)d.n_envs + (size_t)env]
+template <bool AGENTS = false>
 SF_FN void sf_step_body(const SfDev &d, const SfConst &k, const SfTabs &t, int env, bool valid,
-                        const uint8_t *actions, int half, SfStatDelta &sd)
+                        const uint8_t *actions, int half, SfStatDelta &sd, int32_t *ao = nullptr)
 {
     if (half != SF_HALF_B) {
         sf_advance_pending(d, t, env, valid, SF_WARM_PER_STEP);
@@ -1909,6 +1932,19 @@ SF_FN void sf_step_body(const SfDev &d, const SfConst &k, const SfTabs &t, int e
         o.d_kills -= e.kills, o.d_teams_kills -= e.tkills, o.d_loot -= e.loot;
         o.d_hp -= SF_AT(d.h_hp, k.ind), o.d_damage -= SF_AT(d.h_dmg, k.ind), o.d_effect -= SF_AT(d.h_eff, k.ind);
         d.out[env] = o;
+        if constexpr (AGENTS) {
+            if (half != SF_HALF_B) {
+#pragma unroll 1
+                for (int a = 0; a < k.n_agents; ++a) {
+                    const bool driven = sf_controllable(d, k, env, e, a);
+                    SF_AO(0, a) = driven ? (int32_t)SF_AGENT_DRIVEN : 0;
+                    SF_AO(1, a) = driven ? -SF_AT(d.h_hp, a) : 0;
+                    SF_AO(2, a) = driven ? -SF_AT(d.h_dmg, a) : 0;
+                    SF_AO(3, a) = driven ? -SF_AT(d.h_eff, a) : 0;
+                    SF_AO(4, a) = driven ? -SF_AT(d.h_kills, a) : 0;
+                }
+            }
+        }
     }
     if (half != SF_HALF_B && e.on) sd.algo_bytes += sf_algo_bytes(k, e);
     sf_bt_rebuild(d, t, env, e);
@@ -1922,6 +1958,20 @@ SF_FN void sf_step_body(const SfDev &d, const SfConst &k, const SfTabs &t, int e
         o.episode_steps = (int32_t)e.steps;
         d.out[env] = o;
         if (d.out_mirror) d.out_mirror[env] = o; /* straight into the caller's host buffer, no copy afterwards */
+        if constexpr (AGENTS) {
+            /* the end of the step as played: read before the auto-reset below re-creates the arena */
+            if (half != SF_HALF_A) {
+#pragma unroll 1
+                for (int a = 0; a < k.n_agents; ++a) {
+                    if (!(SF_AO(0, a) & SF_AGENT_DRIVEN)) continue;
+                    if (!((e.mh >> a) & 1)) SF_AO(0, a) = SF_AGENT_DRIVEN | SF_AGENT_DIED;
+                    SF_AO(1, a) += SF_AT(d.h_hp, a);
+                    SF_AO(2, a) += SF_AT(d.h_dmg, a);
+                    SF_AO(3, a) += SF_AT(d.h_eff, a);
+                    SF_AO(4, a) += SF_AT(d.h_kills, a);
+                }
+            }
+        }
     }
     /* Auto-reset happens at the end of the whole step: an episode that ends in half A (an overflow or
        guard abort) is stored as it ended, half B runs on it with nothing to do, keeps its terminal status
@@ -1952,5 +2002,6 @@ SF_FN void sf_step_body(const SfDev &d, const SfConst &k, const SfTabs &t, int e
     }
     SF_SYNCWARP();
 }
+#undef SF_AO
 
 #endif /* SF_CORE_CUH */

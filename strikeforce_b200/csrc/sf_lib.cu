@@ -104,12 +104,16 @@ __device__ __forceinline__ void sf_flush_stats(const SfDev &d, const SfStatDelta
  * LIST (sf_step_list, DESIGN.md section 7d): the work items are the entries i < min(*list_n, n_max) of the device
  * list env_ids instead of the arenas; entry i steps arena env_ids[i] with action row i, if the id is in range and
  * the entry owns it (claim[id] == i, set by sf_claim_kernel).  lpw <= 0 picks the arenas per warp here, from the
- * count, by sf_launch_step's rule, so that ids in order with count = n_envs are chunked exactly as sf_step does. */
-template <int HALF, bool LIST>
+ * count, by sf_launch_step's rule, so that ids in order with count = n_envs are chunked exactly as sf_step does.
+ *
+ * AGENTS (sf_enable_agent_out, DESIGN.md section 7g): the stepped arenas also write their rows of the handle's
+ * agent-output buffer agent_out ([field][slot][n_envs]: the lanes of a warp store neighbouring words).  The
+ * buffer is the last parameter, so that the parameters the other instantiations read keep their offsets. */
+template <int HALF, bool LIST, bool AGENTS>
 __global__ void __launch_bounds__(SF_CTA, 1)
 sf_step_kernel(const SfDev d, const __grid_constant__ SfConst k, const uint8_t *__restrict__ actions, int lpw,
                const int32_t *__restrict__ env_ids, const int32_t *__restrict__ list_n, int n_max,
-               const int32_t *__restrict__ claim)
+               const int32_t *__restrict__ claim, int32_t *__restrict__ agent_out)
 {
     SfTabs t;
     sf_stage_tables(d, t);
@@ -143,9 +147,10 @@ sf_step_kernel(const SfDev d, const __grid_constant__ SfConst k, const uint8_t *
             const int id = valid ? env_ids[env] : -1;
             const uint8_t *row = actions + (size_t)env * k.n_agents;
             valid = id >= 0 && id < d.n_envs && claim[id] == env;
-            sf_step_body(d, k, t, valid ? id : lane, valid, valid ? row : nullptr, HALF, sd);
+            sf_step_body<AGENTS>(d, k, t, valid ? id : lane, valid, valid ? row : nullptr, HALF, sd, agent_out);
         } else {
-            sf_step_body(d, k, t, env, valid, (actions && valid) ? actions + (size_t)env * k.n_agents : nullptr, HALF, sd);
+            sf_step_body<AGENTS>(d, k, t, env, valid, (actions && valid) ? actions + (size_t)env * k.n_agents : nullptr, HALF,
+                                 sd, agent_out);
         }
         __syncwarp();
         sf_flush_stats(d, sd);
@@ -1034,6 +1039,19 @@ sf_action_mask_kernel(const SfDev d, const __grid_constant__ SfConst k, uint32_t
     }
 }
 
+/* sf_get(SF_FIELD_AGENT_OUT): the handle's rows, [field][slot][n_envs], as sf_agent_out [n_envs][slot].  One
+ * thread per output word, so that the stores are coalesced; the loads gather from L2. */
+__global__ void sf_agent_out_kernel(const int32_t *__restrict__ ao, int n_envs, int n_agents, int32_t *__restrict__ out)
+{
+    const long n = (long)n_envs * n_agents * 5;
+    for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) {
+        const int f = (int)(i % 5);
+        const long row = i / 5; /* env * n_agents + a */
+        const int a = (int)(row % n_agents), env = (int)(row / n_agents);
+        out[i] = ao[((long)f * n_agents + a) * n_envs + env];
+    }
+}
+
 /* ====================================================================== host side */
 
 struct sf_handle {
@@ -1054,6 +1072,7 @@ struct sf_handle {
     int32_t *d_fin_n = nullptr;   /* ... and their number */
     int32_t *d_tile_n = nullptr;  /* sf_list_finished / sf_reset_finished: finished arenas per tile of SF_LIST_TILE */
     int32_t *d_claim = nullptr;   /* sf_step_list: the list entry that steps each arena; INT32_MAX between calls */
+    int32_t *d_agent_out = nullptr; /* sf_enable_agent_out: [field][slot][n_envs] (its own allocation), or NULL */
     SfSnapLayout snap;           /* the record layout of sf_save / sf_load (sf_snapshot.cuh) */
     int device = 0, n_sm = 0;
     bool between_halves = false; /* sf_step_a has run, sf_step_b has not: the P2 observation point */
@@ -1254,10 +1273,14 @@ int sf_create(const sf_config *cfg, sf_handle **out)
         const std::vector<int32_t> unclaimed((size_t)h->d.E, INT32_MAX);
         SF_CREATE_CUDA(cudaMemcpy(h->d_claim, unclaimed.data(), unclaimed.size() * 4, cudaMemcpyHostToDevice));
     }
-    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_BOTH, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
-    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_A, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
-    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_B, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
-    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_BOTH, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
+#define SF_STEP_SMEM_ATTRS(AGENTS)                                                                                              \
+    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_BOTH, false, AGENTS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES)); \
+    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_A, false, AGENTS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));    \
+    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_B, false, AGENTS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));    \
+    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_BOTH, true, AGENTS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES))
+    SF_STEP_SMEM_ATTRS(false);
+    SF_STEP_SMEM_ATTRS(true);
+#undef SF_STEP_SMEM_ATTRS
     SF_CREATE_CUDA(cudaFuncSetAttribute(sf_reset_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
     SF_CREATE_CUDA(cudaFuncSetAttribute(sf_rng_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
 #define SF_OBS_SMEM_ATTR(NHWC, LIST, T) \
@@ -1292,6 +1315,7 @@ int sf_destroy(sf_handle *h)
         SfDeviceGuard guard(h);
         cudaDeviceSynchronize();
         cudaFree(h->arena);
+        if (h->d_agent_out) cudaFree(h->d_agent_out);
     }
     delete h;
     return SF_OK;
@@ -1340,11 +1364,18 @@ static int sf_launch_step(sf_handle *h, int half, const uint8_t *d_actions, cuda
     }
     const int nchunks = (h->d.n_envs + lpw - 1) / lpw;
     int grid = nchunks < h->n_sm ? nchunks : h->n_sm; /* one persistent CTA per SM; warps take chunks round-robin over the CTAs */
-    if (half == SF_HALF_BOTH)
-        sf_step_kernel<SF_HALF_BOTH, false><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, d_actions, lpw, nullptr, nullptr, 0, nullptr);
-    else if (half == SF_HALF_A)
-        sf_step_kernel<SF_HALF_A, false><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, nullptr, lpw, nullptr, nullptr, 0, nullptr);
-    else sf_step_kernel<SF_HALF_B, false><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, d_actions, lpw, nullptr, nullptr, 0, nullptr);
+    int32_t *ao = h->d_agent_out;
+#define SF_STEP_LAUNCH(AGENTS)                                                                                                  \
+    do {                                                                                                                        \
+        if (half == SF_HALF_BOTH)                                                                                               \
+            sf_step_kernel<SF_HALF_BOTH, false, AGENTS><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, d_actions, lpw, nullptr, nullptr, 0, nullptr, ao); \
+        else if (half == SF_HALF_A)                                                                                             \
+            sf_step_kernel<SF_HALF_A, false, AGENTS><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, nullptr, lpw, nullptr, nullptr, 0, nullptr, ao); \
+        else sf_step_kernel<SF_HALF_B, false, AGENTS><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, d_actions, lpw, nullptr, nullptr, 0, nullptr, ao); \
+    } while (0)
+    if (ao) SF_STEP_LAUNCH(true);
+    else SF_STEP_LAUNCH(false);
+#undef SF_STEP_LAUNCH
     h->launches += 1;
     SF_CUDA(h, cudaGetLastError());
     return SF_OK;
@@ -1369,7 +1400,12 @@ int sf_step_list(sf_handle *h, const uint8_t *actions, const int32_t *env_ids, c
     int cgrid = (n_max + 255) / 256;
     if (cgrid > 4 * h->n_sm) cgrid = 4 * h->n_sm;
     sf_claim_kernel<false><<<cgrid, 256, 0, s>>>(env_ids, count, n_max, h->d.n_envs, h->d_claim);
-    sf_step_kernel<SF_HALF_BOTH, true><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, actions, lpw, env_ids, count, n_max, h->d_claim);
+    if (h->d_agent_out)
+        sf_step_kernel<SF_HALF_BOTH, true, true><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, actions, lpw, env_ids, count, n_max,
+                                                                                   h->d_claim, h->d_agent_out);
+    else
+        sf_step_kernel<SF_HALF_BOTH, true, false><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, actions, lpw, env_ids, count, n_max,
+                                                                                    h->d_claim, nullptr);
     sf_claim_kernel<true><<<cgrid, 256, 0, s>>>(env_ids, count, n_max, h->d.n_envs, h->d_claim);
     h->launches += 3;
     SF_CUDA(h, cudaGetLastError());
@@ -1567,6 +1603,27 @@ int sf_reset_finished(sf_handle *h, void *stream)
     return SF_OK;
 }
 
+int sf_enable_agent_out(sf_handle *h)
+{
+    if (!h) return SF_ERR_ARG;
+    if (h->between_halves) return sf_fail(h, SF_ERR_ARG, "sf_enable_agent_out: the step opened by sf_step_a is still waiting for sf_step_b");
+    if (h->d_agent_out) return SF_OK;
+    SfDeviceGuard guard(h);
+    const size_t bytes = (size_t)h->d.n_envs * (size_t)h->k.n_agents * sizeof(sf_agent_out);
+    int32_t *p = nullptr;
+    SF_CUDA(h, cudaMalloc(&p, bytes));
+    /* zeroed before any stream of the caller can step with it */
+    cudaError_t e = cudaMemset(p, 0, bytes);
+    if (e == cudaSuccess) e = cudaDeviceSynchronize();
+    if (e != cudaSuccess) {
+        cudaFree(p);
+        return sf_fail(h, SF_ERR_CUDA, std::string("sf_enable_agent_out: ") + cudaGetErrorString(e));
+    }
+    h->d_agent_out = p;
+    h->arena_bytes += bytes;
+    return SF_OK;
+}
+
 int sf_get(sf_handle *h, int32_t field, void *dev_out, void *stream)
 {
     if (!h || !dev_out) return h ? sf_fail(h, SF_ERR_ARG, "sf_get: null buffer") : SF_ERR_ARG;
@@ -1589,6 +1646,14 @@ int sf_get(sf_handle *h, int32_t field, void *dev_out, void *stream)
     case SF_FIELD_POPULATION:
         sf_population_kernel<<<grid, 128, 0, s>>>(h->d, h->k, static_cast<int32_t *>(dev_out));
         break;
+    case SF_FIELD_AGENT_OUT: {
+        if (!h->d_agent_out) return sf_fail(h, SF_ERR_ARG, "sf_get: SF_FIELD_AGENT_OUT needs sf_enable_agent_out first");
+        const long words = (long)n * h->k.n_agents * 5;
+        long ag = (words + 255) / 256;
+        if (ag > 8L * h->n_sm) ag = 8L * h->n_sm;
+        sf_agent_out_kernel<<<(int)ag, 256, 0, s>>>(h->d_agent_out, n, h->k.n_agents, static_cast<int32_t *>(dev_out));
+        break;
+    }
     default:
         return sf_fail(h, SF_ERR_ARG, "sf_get: unknown field");
     }

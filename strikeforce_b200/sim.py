@@ -25,7 +25,9 @@ _OBS_FORMAT = {torch.float32: 0, torch.float16: sfcfg.OBS_F16, torch.bfloat16: s
 class BatchedArena:
     def __init__(self, n_envs, mode="Solo", level=1, level_max=None, squad_agents=False, auto_reset=True,
                  max_steps=0, env_id_base=0, player="account1", caps=None, arena=None, device=None, teams=None, sheets=None,
-                 ind=0):
+                 ind=0, agent_out=False):
+        """``agent_out=True`` turns on the per-agent step outputs (sf_enable_agent_out, read with ``agent_out()``)
+        from the first step on."""
         if not torch.cuda.is_available():
             # fail loudly: there is no CPU path (sf_create would report SF_ERR_NO_DEVICE as well)
             raise RuntimeError("strikeforce_b200 needs a CUDA device; it has no CPU fallback")
@@ -42,6 +44,8 @@ class BatchedArena:
         self.step_count = 0
         self._synth = torch.empty((n_envs, self.n_agents), dtype=torch.uint8, device=self.device)
         self._mask_bits = {}  # action_mask(table=): bit index of each symbol of a table, on the device
+        if agent_out:
+            self._chk(lib().sf_enable_agent_out(self._h))
 
     # ------------------------------------------------------------------ lifetime
     def close(self):
@@ -233,6 +237,16 @@ class BatchedArena:
     def step_out(self):
         """int32 [n_envs, 8]: status d_kills d_teams_kills d_loot d_hp d_damage d_effect episode_steps."""
         return self._get(sfcfg.FIELD_STEP_OUT, (self.n_envs, 8), torch.int32)
+
+    def agent_out(self):
+        """Per-agent step outputs (sf_get(SF_FIELD_AGENT_OUT), DESIGN.md section 7g): int32 CUDA tensor
+        [n_envs, n_agents, 5], the fields ``config.AGENT_OUT_FIELDS`` (flags d_hp d_damage d_effect d_kills) of what
+        the last step of each arena did to the human each column of the action row drives.  flags has
+        ``config.AGENT_DRIVEN`` for a slot that was controllable when the step started (``action_mask() != 0``
+        then) and ``config.AGENT_DIED`` when that human was gone at its end, before any auto-reset; a slot that was
+        not driven is all zeros.  After ``step_list``, index it with the list's ids: unlisted arenas keep the rows
+        of their own last step.  Needs ``agent_out=True`` at construction; no host synchronisation."""
+        return self._get(sfcfg.FIELD_AGENT_OUT, (self.n_envs, self.n_agents, len(sfcfg.AGENT_OUT_FIELDS)), torch.int32)
 
     def state_hash(self):
         return self._get(sfcfg.FIELD_STATE_HASH, (self.n_envs,), torch.int64)
