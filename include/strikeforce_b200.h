@@ -338,6 +338,63 @@ enum { SF_AGENT_DRIVEN = 1, SF_AGENT_DIED = 2 };
    is SF_ERR_ARG before this call).  A caller probes for it by looking the symbol up (SF_ABI_VERSION stays 3). */
 int sf_enable_agent_out(sf_handle *h);
 
+/* Match logs (DESIGN.md section 7h): an opt-in per-arena tape of the command symbols the reference's logger writes
+   to a .sf_sample file (gameplay.hpp:966-991), so that an episode played here can be written as a match log and
+   replayed by the reference's client.  The tape of arena e holds the symbols of the episode e's last step played,
+   in file order; each step of a running arena appends
+   1. the symbol ind was given, actions[ind] as obey receives it, then
+   2. in ascending slot order the symbol of every other human that is live when human_action gathers commands (the
+      state after half-tick A) and is a Battle Royale player or a squad agent that is not a random NPC -- the rule
+      of sf_action_mask on that state.  A squad agent's symbol is the delivered one: a symbol outside "+xzqeawsd"
+      is logged as '+'.
+   A tape restarts when a step begins with the arena's step count at 0; it then takes the episode's seeds (tb,
+   serial: rebuilt from the term constants of the arena's stream; they seed the same stream, and equal the seeds
+   of sf_reset below 10^18), level, episode counter and global id.  So sf_reset, auto-reset and sf_reset_finished
+   do not touch tapes: after an auto-reset the tape still describes the finished episode until the arena's next
+   step, and with auto_reset = 1 the arenas whose sf_step_out status is terminal are exported before the next step.
+   sf_step_list appends for listed arenas only; the split step restarts in sf_step_a and appends in sf_step_b.
+   sf_load and an accepted sf_load_list clear SF_LOG_COMPLETE on the arenas they overwrite.  Tapes are not part of
+   arena records.  With logs on, the state, sf_step_out, agent outputs, statistics and records are byte for byte
+   what they are without.
+   An exported row is an sf_log_head followed by cap_symbols bytes of tape (the first n_symbols count), padded to
+   a multiple of 16 bytes: sf_log_row_bytes. */
+typedef struct sf_log_head {
+    int32_t flags;     /* SF_LOG_*                                                              */
+    int32_t status;    /* SF_RUNNING while the episode runs, then how it ended                  */
+    int32_t level;     /* the episode's level (the offline format does not carry it)            */
+    uint32_t episode;  /* the arena's episode counter                                           */
+    int32_t steps;     /* steps since the restart, those past a full tape included              */
+    int32_t n_symbols; /* symbols on the tape, at most cap_symbols                              */
+    int64_t tb;        /* seeds of the episode's stream (Random::_srand), the log header        */
+    int64_t serial;
+    int64_t global_id; /* env_id_base + arena                                                   */
+} sf_log_head;
+enum {
+    SF_LOG_COMPLETE = 1,     /* the tape holds every step since its restart, taken by this handle        */
+    SF_LOG_TRUNCATED = 2,    /* the tape was full: later symbols were dropped (COMPLETE is cleared)      */
+    SF_LOG_ABORTED = 4,      /* the episode ended in SF_OVERFLOW or SF_UB_GUARD                           */
+    SF_LOG_UNREPLAYABLE = 8  /* a symbol the reference's reader (file >> char) skips: NUL or white space  */
+};
+#define SF_LOG_CAP_MAX (1 << 24) /* symbols per tape */
+
+/* Opt in to match logs, once per handle: allocates n_envs rows of sf_log_row_bytes (counted by sf_device_bytes),
+   zeroed (no tape is COMPLETE before its first restart), and from then on every step call of the handle records.
+   SF_ERR_ARG between sf_step_a and sf_step_b, for cap_symbols outside [1, SF_LOG_CAP_MAX], and for a second call
+   with another capacity; a second call with the same capacity does nothing.  A caller probes for it by looking the
+   symbol up (SF_ABI_VERSION stays 3). */
+int sf_enable_log(sf_handle *h, int32_t cap_symbols);
+
+/* bytes of one exported row: sizeof(sf_log_head) + cap_symbols rounded up to 16; 0 before sf_enable_log */
+int32_t sf_log_row_bytes(const sf_handle *h);
+
+/* Export tapes into the DEVICE buffer rows (16-byte aligned), one launch, no host synchronisation.  env_ids ==
+   NULL: row i is the tape of arena i, for every arena (n_max must be n_envs, count NULL).  Otherwise the list
+   rules of sf_action_mask: row i < min(*count, n_max) (count read on the device; NULL = n_max) is the tape of
+   arena env_ids[i], duplicates allowed, an id outside [0, n_envs) gives an all-zero row, rows beyond the count
+   are not written.  Allowed at P1 and between sf_step_a and sf_step_b (the tape as it stands).  SF_ERR_ARG
+   before sf_enable_log, for NULL rows, misalignment, n_max out of range and a count without env_ids. */
+int sf_log_list(sf_handle *h, void *rows, const int32_t *env_ids, const int32_t *count, int32_t n_max, void *stream);
+
 /* Copy a per-arena field into a DEVICE buffer (sizes above). */
 int sf_get(sf_handle *h, int32_t field, void *dev_out, void *stream);
 

@@ -39,6 +39,19 @@ FIELD_AGENT_OUT = 6  # sf_agent_out [n_envs][n_agents], after sf_enable_agent_ou
 # sf_agent_out: the per-agent step outputs (include/strikeforce_b200.h, DESIGN.md section 7g)
 AGENT_DRIVEN, AGENT_DIED = 1, 2  # bits of the flags field
 AGENT_OUT_FIELDS = ("flags", "d_hp", "d_damage", "d_effect", "d_kills")
+# match logs (sf_enable_log / sf_log_list, include/strikeforce_b200.h, DESIGN.md section 7h)
+LOG_COMPLETE, LOG_TRUNCATED, LOG_ABORTED, LOG_UNREPLAYABLE = 1, 2, 4, 8  # bits of the flags field
+LOG_CAP_MAX = 1 << 24
+# sf_log_head, the start of an exported row; cap_symbols bytes of tape follow, the row padded to 16 bytes
+LOG_HEAD = np.dtype([("flags", "<i4"), ("status", "<i4"), ("level", "<i4"), ("episode", "<u4"), ("steps", "<i4"),
+                     ("n_symbols", "<i4"), ("tb", "<i8"), ("serial", "<i8"), ("global_id", "<i8")])
+
+
+def log_row_bytes(cap_symbols):
+    """bytes of one exported row (sf_log_row_bytes)"""
+    return LOG_HEAD.itemsize + (cap_symbols + 15) // 16 * 16
+
+
 STAT_NAMES = ["steps", "episodes", "wins", "deaths", "timeouts", "truncated", "overflows", "ub_guards",
               "kills", "teams_kills", "loot", "rng_draws", "algo_bytes", "reserved0", "reserved1", "reserved2"]
 

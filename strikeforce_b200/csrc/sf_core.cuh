@@ -1454,18 +1454,83 @@ SF_FN void sf_obey(const SfDev &d, const SfConst &k, const SfTabs &t, int env, S
     }
 }
 
+/* ------------------------------------------------------------------ match logs */
+
+/* The handle's tapes (sf_enable_log, DESIGN.md section 7h): rows of row_bytes, [arena], each an sf_log_head and
+ * cap symbols -- the layout sf_log_list exports.  rows == NULL: logs off. */
+struct SfLog {
+    uint8_t *rows;
+    int32_t row_bytes, cap;
+};
+
+SF_FN sf_log_head *sf_log_at(const SfLog &lg, int env)
+{
+    return reinterpret_cast<sf_log_head *>(lg.rows + (size_t)env * (size_t)lg.row_bytes);
+}
+
+/* a step began at step count 0: restart the tape for the episode the arena plays.  The seeds come back from the
+ * term constants of the arena's stream (sf_seed_pending): digit i of tb is (constant & 0xFF) / 2 - 1, digit i of
+ * serial is 3^(log us) - 1 with 2 log us = constant >> 8.  Only 18 digits are kept there, so the seeds written are
+ * those of sf_reset modulo 10^18 -- equal below 10^18 (sf_reset refuses negative seeds), and splitting them gives
+ * the same 36 constants in any case. */
+SF_FN void sf_log_restart(const SfDev &d, const SfConst &k, const SfTabs &t, const SfLog &lg, int env, const SfEnv &e)
+{
+    int64_t tb = 0, serial = 0;
+#pragma unroll 1
+    for (int i = 17; i >= 0; --i) {
+        const uint32_t c = d.rng_cst[sf_cst_index(d, e.bank ? 1 : 0, i, env)];
+        tb = tb * 10 + (int64_t)((c & 0xFFu) >> 1) - 1;
+        serial = serial * 10 + (int64_t)sf_exp_m1(t, c >> 8);
+    }
+    sf_log_head *hd = sf_log_at(lg, env);
+    hd->flags = SF_LOG_COMPLETE, hd->status = SF_RUNNING, hd->level = e.level, hd->episode = e.episode;
+    hd->steps = 0, hd->n_symbols = 0;
+    hd->tb = tb, hd->serial = serial, hd->global_id = k.env_id_base + env;
+}
+
+/* append symbol c to the tape of arena env */
+SF_FN void sf_log_put(const SfLog &lg, int env, int c)
+{
+    sf_log_head *hd = sf_log_at(lg, env);
+    const int n = hd->n_symbols;
+    if (n < lg.cap) {
+        reinterpret_cast<uint8_t *>(hd + 1)[n] = (uint8_t)c;
+        hd->n_symbols = n + 1;
+        /* `file >> char` skips white space (the C locale's isspace) and a NUL does not survive as itself */
+        if (c == 0 || c == ' ' || (c >= '\t' && c <= '\r')) hd->flags |= SF_LOG_UNREPLAYABLE;
+    } else {
+        hd->flags = (hd->flags & ~SF_LOG_COMPLETE) | SF_LOG_TRUNCATED;
+    }
+}
+
+/* the end of a step (or half) the arena began running: how far the episode got */
+SF_FN void sf_log_exit(const SfLog &lg, int env, const SfEnv &e)
+{
+    sf_log_head *hd = sf_log_at(lg, env);
+    hd->status = e.status, hd->steps = (int32_t)e.steps;
+    if (e.status == SF_OVERFLOW || e.status == SF_UB_GUARD) hd->flags |= SF_LOG_ABORTED;
+}
+
 /* human_action, gameplay.hpp:965-1012.  actions = this arena's row of the action buffer:
  * [ind] the player's command (get_my_action, :939-963; ind = 0 outside Battle Royale), the other
  * entries what bot() returns for the agent-driven squad humans (bots/bot-0.5/Custom.hpp:137-158, one
- * of "+xzqeawsd") or, in Battle Royale, what the other players sent. */
+ * of "+xzqeawsd") or, in Battle Royale, what the other players sent.
+ *
+ * LOG (sf_enable_log, DESIGN.md section 7h): with lg.rows set, the symbols the reference's logger writes go to the
+ * arena's tape -- ind's first, then in the gather loop every live Battle Royale player and squad agent (the
+ * humans of SF_CONTROLLABLE_RULE other than ind) with the symbol it is delivered. */
+template <bool LOG = false>
 SF_FN void sf_human_action(const SfDev &d, const SfConst &k, const SfTabs &t, int env, SfEnv &e,
-                           const uint8_t *actions)
+                           const uint8_t *actions, SfLog lg = SfLog{})
 {
     /* commands wait in h_cmd between the two loops (command[], gameplay.hpp:43) */
     const uint64_t live = e.on ? e.mh : 0ull;
     const int hi = SF_WARP_MAX(live ? sf_fls64(live) : -1);
     const int ind = k.ind;
     const int cmd0 = (actions && e.on) ? actions[ind] : '+';
+    if constexpr (LOG) {
+        if (lg.rows && e.on) sf_log_put(lg, env, cmd0);
+    }
     for (int h = 0; h <= hi; ++h) {
         if (h == ind) continue; /* command[ind] is the player's own, set before human_action (:956-961) */
         bool is_live = (live >> h) & 1;
@@ -1480,6 +1545,10 @@ SF_FN void sf_human_action(const SfDev &d, const SfConst &k, const SfTabs &t, in
                 bool ok = c == '+' || c == 'x' || c == 'z' || c == 'q' || c == 'e' || c == 'a' || c == 'w' ||
                           c == 's' || c == 'd';
                 if (!ok) c = '+';
+            }
+            if constexpr (LOG) {
+                if (lg.rows && ((k.mode == SF_MODE_ROYALE && h < k.n_players) || ((sel & HS_AGENT) && h < k.n_agents)))
+                    sf_log_put(lg, env, c);
             }
         }
         if (is_live) SF_AT(d.h_cmd, h) = (uint8_t)c;
@@ -1774,8 +1843,9 @@ SF_FN void sf_eval_end(const SfDev &d, const SfConst &k, int env, SfEnv &e)
  * half-ticks end with the same three calls (update_tmp, hit_human / hit_zombie, ++frame,
  * update_bull), so they run as two rounds of one loop: round 0 = spawns + zombie_action +
  * portal_damage (:1444-1456), round 1 = human_action (:1464). */
+template <bool LOG = false>
 SF_FN void sf_step_halves(const SfDev &d, const SfConst &k, const SfTabs &t, int env, SfEnv &e,
-                          const uint8_t *actions, int first, int last)
+                          const uint8_t *actions, int first, int last, SfLog lg = SfLog{})
 {
 #pragma unroll 1
     for (int ph = first; ph <= last; ++ph) {
@@ -1787,7 +1857,7 @@ SF_FN void sf_step_halves(const SfDev &d, const SfConst &k, const SfTabs &t, int
             SF_PHASE_SYNC(2);
             sf_portal_damage(d, k, t, env, e);
         } else {
-            sf_human_action(d, k, t, env, e, actions);
+            sf_human_action<LOG>(d, k, t, env, e, actions, lg);
         }
         SF_PHASE_SYNC(3);
         sf_resolve_bullets(d, k, t, env, e);
@@ -1908,14 +1978,18 @@ SF_FN void sf_reset_finished_body(const SfDev &d, const SfConst &k, const SfTabs
  * values at entry" in d.out and gets the values at exit added, and the statistics read the
  * entry values back from the header arrays, which are only overwritten by sf_store_env.
  *
- * AGENTS (sf_enable_agent_out, DESIGN.md section 7g): `ao` is the handle's agent-output buffer,
- * [field][agent slot][n_envs] int32 with the fields of sf_agent_out, and the rows of the arena are
- * kept the same way: half A (or the whole step) writes DRIVEN and minus the entry values of each
- * driven slot, half B (or the whole step) adds the values at exit and DIED, before any auto-reset. */
+ * EXTRAS: the opt-in outputs of the step, each present when its buffer is set.
+ * - Agent outputs (sf_enable_agent_out, DESIGN.md section 7g): `ao` is the handle's agent-output buffer,
+ *   [field][agent slot][n_envs] int32 with the fields of sf_agent_out, and the rows of the arena are
+ *   kept the same way: half A (or the whole step) writes DRIVEN and minus the entry values of each
+ *   driven slot, half B (or the whole step) adds the values at exit and DIED, before any auto-reset.
+ * - Match logs (sf_enable_log, DESIGN.md section 7h): `lg` holds the handle's tapes.  Half A (or the
+ *   whole step) restarts the tape of an arena at step count 0, sf_human_action appends, and the half
+ *   that ran writes the status and step count, before any auto-reset. */
 #define SF_AO(field, a) ao[((size_t)(field) * (size_t)k.n_agents + (size_t)(a)) * (size_t)d.n_envs + (size_t)env]
-template <bool AGENTS = false>
+template <bool EXTRAS = false>
 SF_FN void sf_step_body(const SfDev &d, const SfConst &k, const SfTabs &t, int env, bool valid,
-                        const uint8_t *actions, int half, SfStatDelta &sd, int32_t *ao = nullptr)
+                        const uint8_t *actions, int half, SfStatDelta &sd, int32_t *ao = nullptr, SfLog lg = SfLog{})
 {
     if (half != SF_HALF_B) {
         sf_advance_pending(d, t, env, valid, SF_WARM_PER_STEP);
@@ -1932,8 +2006,8 @@ SF_FN void sf_step_body(const SfDev &d, const SfConst &k, const SfTabs &t, int e
         o.d_kills -= e.kills, o.d_teams_kills -= e.tkills, o.d_loot -= e.loot;
         o.d_hp -= SF_AT(d.h_hp, k.ind), o.d_damage -= SF_AT(d.h_dmg, k.ind), o.d_effect -= SF_AT(d.h_eff, k.ind);
         d.out[env] = o;
-        if constexpr (AGENTS) {
-            if (half != SF_HALF_B) {
+        if constexpr (EXTRAS) {
+            if (ao && half != SF_HALF_B) {
 #pragma unroll 1
                 for (int a = 0; a < k.n_agents; ++a) {
                     const bool driven = sf_controllable(d, k, env, e, a);
@@ -1944,11 +2018,12 @@ SF_FN void sf_step_body(const SfDev &d, const SfConst &k, const SfTabs &t, int e
                     SF_AO(4, a) = driven ? -SF_AT(d.h_kills, a) : 0;
                 }
             }
+            if (lg.rows && half != SF_HALF_B && e.on && e.steps == 0) sf_log_restart(d, k, t, lg, env, e);
         }
     }
     if (half != SF_HALF_B && e.on) sd.algo_bytes += sf_algo_bytes(k, e);
     sf_bt_rebuild(d, t, env, e);
-    sf_step_halves(d, k, t, env, e, actions, half == SF_HALF_B ? 1 : 0, half == SF_HALF_A ? 0 : 1);
+    sf_step_halves<EXTRAS>(d, k, t, env, e, actions, half == SF_HALF_B ? 1 : 0, half == SF_HALF_A ? 0 : 1, lg);
     if (valid) {
         /* a terminal arena that is not auto-reset waits for sf_reset: report, change nothing */
         sf_step_out o = d.out[env];
@@ -1958,9 +2033,9 @@ SF_FN void sf_step_body(const SfDev &d, const SfConst &k, const SfTabs &t, int e
         o.episode_steps = (int32_t)e.steps;
         d.out[env] = o;
         if (d.out_mirror) d.out_mirror[env] = o; /* straight into the caller's host buffer, no copy afterwards */
-        if constexpr (AGENTS) {
+        if constexpr (EXTRAS) {
             /* the end of the step as played: read before the auto-reset below re-creates the arena */
-            if (half != SF_HALF_A) {
+            if (ao && half != SF_HALF_A) {
 #pragma unroll 1
                 for (int a = 0; a < k.n_agents; ++a) {
                     if (!(SF_AO(0, a) & SF_AGENT_DRIVEN)) continue;
@@ -1971,6 +2046,7 @@ SF_FN void sf_step_body(const SfDev &d, const SfConst &k, const SfTabs &t, int e
                     SF_AO(4, a) += SF_AT(d.h_kills, a);
                 }
             }
+            if (lg.rows && was_on) sf_log_exit(lg, env, e);
         }
     }
     /* Auto-reset happens at the end of the whole step: an episode that ends in half A (an overflow or

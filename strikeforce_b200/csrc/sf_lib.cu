@@ -106,14 +106,16 @@ __device__ __forceinline__ void sf_flush_stats(const SfDev &d, const SfStatDelta
  * the entry owns it (claim[id] == i, set by sf_claim_kernel).  lpw <= 0 picks the arenas per warp here, from the
  * count, by sf_launch_step's rule, so that ids in order with count = n_envs are chunked exactly as sf_step does.
  *
- * AGENTS (sf_enable_agent_out, DESIGN.md section 7g): the stepped arenas also write their rows of the handle's
- * agent-output buffer agent_out ([field][slot][n_envs]: the lanes of a warp store neighbouring words).  The
- * buffer is the last parameter, so that the parameters the other instantiations read keep their offsets. */
-template <int HALF, bool LIST, bool AGENTS>
+ * EXTRAS: the opt-in outputs, each written when its buffer is set -- agent outputs (sf_enable_agent_out, DESIGN.md
+ * section 7g): the stepped arenas write their rows of the handle's agent-output buffer agent_out ([field][slot][n_envs]:
+ * the lanes of a warp store neighbouring words); match logs (sf_enable_log, section 7h): they restart and append to
+ * their tapes in log.  The buffers are the last parameters, so that the parameters the other instantiations read keep
+ * their offsets. */
+template <int HALF, bool LIST, bool EXTRAS>
 __global__ void __launch_bounds__(SF_CTA, 1)
 sf_step_kernel(const SfDev d, const __grid_constant__ SfConst k, const uint8_t *__restrict__ actions, int lpw,
                const int32_t *__restrict__ env_ids, const int32_t *__restrict__ list_n, int n_max,
-               const int32_t *__restrict__ claim, int32_t *__restrict__ agent_out)
+               const int32_t *__restrict__ claim, int32_t *__restrict__ agent_out, const SfLog log)
 {
     SfTabs t;
     sf_stage_tables(d, t);
@@ -147,10 +149,10 @@ sf_step_kernel(const SfDev d, const __grid_constant__ SfConst k, const uint8_t *
             const int id = valid ? env_ids[env] : -1;
             const uint8_t *row = actions + (size_t)env * k.n_agents;
             valid = id >= 0 && id < d.n_envs && claim[id] == env;
-            sf_step_body<AGENTS>(d, k, t, valid ? id : lane, valid, valid ? row : nullptr, HALF, sd, agent_out);
+            sf_step_body<EXTRAS>(d, k, t, valid ? id : lane, valid, valid ? row : nullptr, HALF, sd, agent_out, log);
         } else {
-            sf_step_body<AGENTS>(d, k, t, env, valid, (actions && valid) ? actions + (size_t)env * k.n_agents : nullptr, HALF,
-                                 sd, agent_out);
+            sf_step_body<EXTRAS>(d, k, t, env, valid, (actions && valid) ? actions + (size_t)env * k.n_agents : nullptr, HALF,
+                                 sd, agent_out, log);
         }
         __syncwarp();
         sf_flush_stats(d, sd);
@@ -1052,6 +1054,36 @@ __global__ void sf_agent_out_kernel(const int32_t *__restrict__ ao, int n_envs, 
     }
 }
 
+/* sf_log_list (DESIGN.md section 7h): copy tapes into export rows, one 16-byte word per thread and step of the
+ * loop, so that a warp reads and writes 512 contiguous bytes of a row.  Row i < min(*list_n, n_max) (LIST) or
+ * arena i is the row of arena env_ids[i] (LIST) or i; an id outside [0, n_envs) gives an all-zero row. */
+template <bool LIST>
+__global__ void sf_log_export_kernel(const uint4 *__restrict__ tapes, int n_envs, int row_words, uint4 *__restrict__ out,
+                                     const int32_t *__restrict__ env_ids, const int32_t *__restrict__ list_n, int n_max)
+{
+    const int n = LIST ? (list_n ? min(max(*list_n, 0), n_max) : n_max) : n_envs;
+    const long words = (long)n * row_words;
+    for (long w = (long)blockIdx.x * blockDim.x + threadIdx.x; w < words; w += (long)gridDim.x * blockDim.x) {
+        const long i = w / row_words;
+        const int id = LIST ? env_ids[i] : (int)i;
+        out[w] = id >= 0 && id < n_envs ? tapes[(long)id * row_words + (w - i * row_words)] : make_uint4(0u, 0u, 0u, 0u);
+    }
+}
+
+/* sf_load / sf_load_list: an arena a load overwrote does not have its history on its tape any more -- clear
+ * SF_LOG_COMPLETE of entry i < min(*list_n, n) (list_n NULL: n) with an id in range (ids NULL: arena i), if the load
+ * was accepted (*refused == 0, read here on the device).  A repeated id is cleared twice, to the same value. */
+__global__ void sf_log_unload_kernel(uint8_t *__restrict__ tapes, int row_bytes, int n_envs, const int32_t *__restrict__ ids,
+                                     const int32_t *__restrict__ list_n, int n, const int32_t *__restrict__ refused)
+{
+    if (*refused != 0) return;
+    const int m = list_n ? min(max(*list_n, 0), n) : n;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < m; i += gridDim.x * blockDim.x) {
+        const int id = ids ? ids[i] : i;
+        if (id >= 0 && id < n_envs) reinterpret_cast<sf_log_head *>(tapes + (size_t)id * row_bytes)->flags &= ~SF_LOG_COMPLETE;
+    }
+}
+
 /* ====================================================================== host side */
 
 struct sf_handle {
@@ -1073,6 +1105,7 @@ struct sf_handle {
     int32_t *d_tile_n = nullptr;  /* sf_list_finished / sf_reset_finished: finished arenas per tile of SF_LIST_TILE */
     int32_t *d_claim = nullptr;   /* sf_step_list: the list entry that steps each arena; INT32_MAX between calls */
     int32_t *d_agent_out = nullptr; /* sf_enable_agent_out: [field][slot][n_envs] (its own allocation), or NULL */
+    SfLog log = {nullptr, 0, 0};    /* sf_enable_log: the tapes, [n_envs][row_bytes] (their own allocation) */
     SfSnapLayout snap;           /* the record layout of sf_save / sf_load (sf_snapshot.cuh) */
     int device = 0, n_sm = 0;
     bool between_halves = false; /* sf_step_a has run, sf_step_b has not: the P2 observation point */
@@ -1273,11 +1306,11 @@ int sf_create(const sf_config *cfg, sf_handle **out)
         const std::vector<int32_t> unclaimed((size_t)h->d.E, INT32_MAX);
         SF_CREATE_CUDA(cudaMemcpy(h->d_claim, unclaimed.data(), unclaimed.size() * 4, cudaMemcpyHostToDevice));
     }
-#define SF_STEP_SMEM_ATTRS(AGENTS)                                                                                              \
-    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_BOTH, false, AGENTS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES)); \
-    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_A, false, AGENTS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));    \
-    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_B, false, AGENTS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));    \
-    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_BOTH, true, AGENTS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES))
+#define SF_STEP_SMEM_ATTRS(EXTRAS)                                                                                              \
+    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_BOTH, false, EXTRAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES)); \
+    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_A, false, EXTRAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));    \
+    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_B, false, EXTRAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));    \
+    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_step_kernel<SF_HALF_BOTH, true, EXTRAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES))
     SF_STEP_SMEM_ATTRS(false);
     SF_STEP_SMEM_ATTRS(true);
 #undef SF_STEP_SMEM_ATTRS
@@ -1316,6 +1349,7 @@ int sf_destroy(sf_handle *h)
         cudaDeviceSynchronize();
         cudaFree(h->arena);
         if (h->d_agent_out) cudaFree(h->d_agent_out);
+        if (h->log.rows) cudaFree(h->log.rows);
     }
     delete h;
     return SF_OK;
@@ -1365,15 +1399,16 @@ static int sf_launch_step(sf_handle *h, int half, const uint8_t *d_actions, cuda
     const int nchunks = (h->d.n_envs + lpw - 1) / lpw;
     int grid = nchunks < h->n_sm ? nchunks : h->n_sm; /* one persistent CTA per SM; warps take chunks round-robin over the CTAs */
     int32_t *ao = h->d_agent_out;
-#define SF_STEP_LAUNCH(AGENTS)                                                                                                  \
+    const SfLog lg = h->log;
+#define SF_STEP_LAUNCH(EXTRAS)                                                                                                  \
     do {                                                                                                                        \
         if (half == SF_HALF_BOTH)                                                                                               \
-            sf_step_kernel<SF_HALF_BOTH, false, AGENTS><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, d_actions, lpw, nullptr, nullptr, 0, nullptr, ao); \
+            sf_step_kernel<SF_HALF_BOTH, false, EXTRAS><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, d_actions, lpw, nullptr, nullptr, 0, nullptr, ao, lg); \
         else if (half == SF_HALF_A)                                                                                             \
-            sf_step_kernel<SF_HALF_A, false, AGENTS><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, nullptr, lpw, nullptr, nullptr, 0, nullptr, ao); \
-        else sf_step_kernel<SF_HALF_B, false, AGENTS><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, d_actions, lpw, nullptr, nullptr, 0, nullptr, ao); \
+            sf_step_kernel<SF_HALF_A, false, EXTRAS><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, nullptr, lpw, nullptr, nullptr, 0, nullptr, ao, lg); \
+        else sf_step_kernel<SF_HALF_B, false, EXTRAS><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, d_actions, lpw, nullptr, nullptr, 0, nullptr, ao, lg); \
     } while (0)
-    if (ao) SF_STEP_LAUNCH(true);
+    if (ao || lg.rows) SF_STEP_LAUNCH(true);
     else SF_STEP_LAUNCH(false);
 #undef SF_STEP_LAUNCH
     h->launches += 1;
@@ -1400,12 +1435,12 @@ int sf_step_list(sf_handle *h, const uint8_t *actions, const int32_t *env_ids, c
     int cgrid = (n_max + 255) / 256;
     if (cgrid > 4 * h->n_sm) cgrid = 4 * h->n_sm;
     sf_claim_kernel<false><<<cgrid, 256, 0, s>>>(env_ids, count, n_max, h->d.n_envs, h->d_claim);
-    if (h->d_agent_out)
+    if (h->d_agent_out || h->log.rows)
         sf_step_kernel<SF_HALF_BOTH, true, true><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, actions, lpw, env_ids, count, n_max,
-                                                                                   h->d_claim, h->d_agent_out);
+                                                                                   h->d_claim, h->d_agent_out, h->log);
     else
         sf_step_kernel<SF_HALF_BOTH, true, false><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, actions, lpw, env_ids, count, n_max,
-                                                                                    h->d_claim, nullptr);
+                                                                                    h->d_claim, nullptr, h->log);
     sf_claim_kernel<true><<<cgrid, 256, 0, s>>>(env_ids, count, n_max, h->d.n_envs, h->d_claim);
     h->launches += 3;
     SF_CUDA(h, cudaGetLastError());
@@ -1624,6 +1659,58 @@ int sf_enable_agent_out(sf_handle *h)
     return SF_OK;
 }
 
+int sf_enable_log(sf_handle *h, int32_t cap_symbols)
+{
+    if (!h) return SF_ERR_ARG;
+    if (h->between_halves) return sf_fail(h, SF_ERR_ARG, "sf_enable_log: the step opened by sf_step_a is still waiting for sf_step_b");
+    if (cap_symbols < 1 || cap_symbols > SF_LOG_CAP_MAX)
+        return sf_fail(h, SF_ERR_ARG, "sf_enable_log: cap_symbols must be in [1, SF_LOG_CAP_MAX]");
+    if (h->log.rows)
+        return cap_symbols == h->log.cap ? SF_OK : sf_fail(h, SF_ERR_ARG, "sf_enable_log: logs are on with another capacity");
+    SfDeviceGuard guard(h);
+    const int32_t row_bytes = (int32_t)sizeof(sf_log_head) + ((cap_symbols + 15) & ~15);
+    const size_t bytes = (size_t)h->d.n_envs * (size_t)row_bytes;
+    uint8_t *p = nullptr;
+    SF_CUDA(h, cudaMalloc(&p, bytes));
+    /* zeroed before any stream of the caller can step with it */
+    cudaError_t e = cudaMemset(p, 0, bytes);
+    if (e == cudaSuccess) e = cudaDeviceSynchronize();
+    if (e != cudaSuccess) {
+        cudaFree(p);
+        return sf_fail(h, SF_ERR_CUDA, std::string("sf_enable_log: ") + cudaGetErrorString(e));
+    }
+    h->log = SfLog{p, row_bytes, cap_symbols};
+    h->arena_bytes += bytes;
+    return SF_OK;
+}
+
+int32_t sf_log_row_bytes(const sf_handle *h) { return h ? h->log.row_bytes : 0; }
+
+int sf_log_list(sf_handle *h, void *rows, const int32_t *env_ids, const int32_t *count, int32_t n_max, void *stream)
+{
+    if (!h) return SF_ERR_ARG;
+    if (!h->log.rows) return sf_fail(h, SF_ERR_ARG, "sf_log_list: needs sf_enable_log first");
+    if (!rows) return sf_fail(h, SF_ERR_ARG, "sf_log_list: null rows");
+    if (!env_ids && count) return sf_fail(h, SF_ERR_ARG, "sf_log_list: count goes with env_ids");
+    if (!env_ids && n_max != h->d.n_envs) return sf_fail(h, SF_ERR_ARG, "sf_log_list: without env_ids n_max must be n_envs");
+    if (n_max < 1 || n_max > h->d.n_envs) return sf_fail(h, SF_ERR_ARG, "sf_log_list: n_max must be in [1, n_envs]");
+    if (reinterpret_cast<uintptr_t>(rows) & 15u) return sf_fail(h, SF_ERR_ARG, "sf_log_list: rows must be 16-byte aligned");
+    if ((reinterpret_cast<uintptr_t>(env_ids) | reinterpret_cast<uintptr_t>(count)) & 3u)
+        return sf_fail(h, SF_ERR_ARG, "sf_log_list: env_ids and count must be 4-byte aligned");
+    SfDeviceGuard guard(h);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const int row_words = h->log.row_bytes / 16;
+    long grid = ((long)n_max * row_words + 255) / 256;
+    if (grid > 8L * h->n_sm) grid = 8L * h->n_sm;
+    const uint4 *tapes = reinterpret_cast<const uint4 *>(h->log.rows);
+    uint4 *out = static_cast<uint4 *>(rows);
+    if (env_ids) sf_log_export_kernel<true><<<(int)grid, 256, 0, s>>>(tapes, h->d.n_envs, row_words, out, env_ids, count, n_max);
+    else sf_log_export_kernel<false><<<(int)grid, 256, 0, s>>>(tapes, h->d.n_envs, row_words, out, nullptr, nullptr, n_max);
+    h->launches += 1;
+    SF_CUDA(h, cudaGetLastError());
+    return SF_OK;
+}
+
 int sf_get(sf_handle *h, int32_t field, void *dev_out, void *stream)
 {
     if (!h || !dev_out) return h ? sf_fail(h, SF_ERR_ARG, "sf_get: null buffer") : SF_ERR_ARG;
@@ -1776,6 +1863,11 @@ int sf_load(sf_handle *h, const int32_t *env_ids, int32_t n, const void *records
     sf_snap_reseed_kernel<false><<<(n + 255) / 256, 256, 0, s>>>(h->d, h->k, rec, h->snap.bytes, d_ids, d_rows, n, h->d_refused,
                                                                 nullptr, nullptr);
     h->launches += 3;
+    if (h->log.rows) {
+        sf_log_unload_kernel<<<(n + 255) / 256, 256, 0, s>>>(h->log.rows, h->log.row_bytes, h->d.n_envs, d_ids, nullptr, n,
+                                                             h->d_refused);
+        h->launches += 1;
+    }
     SF_CUDA(h, cudaGetLastError());
     int refused = 0;
     SF_CUDA(h, cudaMemcpyAsync(&refused, h->d_refused, sizeof refused, cudaMemcpyDeviceToHost, s));
@@ -1842,6 +1934,10 @@ int sf_load_list(sf_handle *h, const void *records, int32_t n_records, const int
                                                                    count, h->d_claim);
     sf_claim_kernel<true><<<cgrid, 256, 0, s>>>(env_ids, count, n_max, h->d.n_envs, h->d_claim);
     h->launches += 5;
+    if (h->log.rows) {
+        sf_log_unload_kernel<<<cgrid, 256, 0, s>>>(h->log.rows, h->log.row_bytes, h->d.n_envs, env_ids, count, n_max, st);
+        h->launches += 1;
+    }
     SF_CUDA(h, cudaGetLastError());
     return SF_OK;
 }

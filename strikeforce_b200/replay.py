@@ -145,6 +145,36 @@ def read(path):
     return MatchLog(tb, serial, players, ind, team, name, sheet, rest.encode("latin-1"))
 
 
+def write_device_log(path, row, cfg, name="1"):
+    """Write the match-log row ``row`` (one row of ``BatchedArena.match_logs()`` on the host: uint8 numpy array or
+    bytes) of a handle created with configuration ``cfg`` (``config.make_config``, e.g. ``BatchedArena.cfg``) as a
+    ``.sf_sample`` file the reference's replay mode reads.  Offline modes go through ``write`` with the logged
+    player sheet, Battle Royale through ``write_royale`` with the handle's teams, sheets and ``ind``.  Returns the
+    episode's level, which the offline format does not carry (the client's menu asks for it).
+
+    Raises ValueError for a row that is not ``LOG_COMPLETE`` (a tape that restarted before this handle logged, was
+    overwritten by a load, or ran out of capacity) or is ``LOG_UNREPLAYABLE`` (a symbol the reference's reader skips):
+    such a file would replay a different episode."""
+    from . import config as sfcfg
+    row = np.frombuffer(bytes(row), dtype=np.uint8)
+    head = row[:sfcfg.LOG_HEAD.itemsize].view(sfcfg.LOG_HEAD)[0]
+    flags = int(head["flags"])
+    if not flags & sfcfg.LOG_COMPLETE:
+        raise ValueError("match log of arena %d is not complete (flags %#x)" % (int(head["global_id"]), flags))
+    if flags & sfcfg.LOG_UNREPLAYABLE:
+        raise ValueError("match log of arena %d holds a symbol the reference cannot read back" % int(head["global_id"]))
+    start = sfcfg.LOG_HEAD.itemsize
+    commands = row[start:start + int(head["n_symbols"])].tobytes()
+    tb, serial = int(head["tb"]), int(head["serial"])
+    if cfg.mode == sfcfg.MODE_ROYALE:
+        n = cfg.royale_players
+        sheets = np.array([list(cfg.royale_sheets[i]) for i in range(n)], dtype=np.int32)
+        write_royale(path, tb, serial, sheets, [cfg.royale_teams[i] for i in range(n)], commands, ind=cfg.royale_ind)
+    else:
+        write(path, tb, serial, logged_sheet(list(cfg.player_sheet)), commands, name=name)
+    return int(head["level"])
+
+
 def commands_per_step(log: MatchLog, n_agents_alive):
     """Split the command stream into steps: ``n_agents_alive(step)`` = number of logged humans that
     step (1 offline without squad agents)."""

@@ -25,9 +25,10 @@ _OBS_FORMAT = {torch.float32: 0, torch.float16: sfcfg.OBS_F16, torch.bfloat16: s
 class BatchedArena:
     def __init__(self, n_envs, mode="Solo", level=1, level_max=None, squad_agents=False, auto_reset=True,
                  max_steps=0, env_id_base=0, player="account1", caps=None, arena=None, device=None, teams=None, sheets=None,
-                 ind=0, agent_out=False):
+                 ind=0, agent_out=False, match_log=0):
         """``agent_out=True`` turns on the per-agent step outputs (sf_enable_agent_out, read with ``agent_out()``)
-        from the first step on."""
+        from the first step on.  ``match_log`` > 0 turns on match logs (sf_enable_log, read with ``match_logs()``)
+        with tapes of that many command symbols."""
         if not torch.cuda.is_available():
             # fail loudly: there is no CPU path (sf_create would report SF_ERR_NO_DEVICE as well)
             raise RuntimeError("strikeforce_b200 needs a CUDA device; it has no CPU fallback")
@@ -46,6 +47,8 @@ class BatchedArena:
         self._mask_bits = {}  # action_mask(table=): bit index of each symbol of a table, on the device
         if agent_out:
             self._chk(lib().sf_enable_agent_out(self._h))
+        if match_log:
+            self._chk(lib().sf_enable_log(self._h, match_log))
 
     # ------------------------------------------------------------------ lifetime
     def close(self):
@@ -247,6 +250,27 @@ class BatchedArena:
         not driven is all zeros.  After ``step_list``, index it with the list's ids: unlisted arenas keep the rows
         of their own last step.  Needs ``agent_out=True`` at construction; no host synchronisation."""
         return self._get(sfcfg.FIELD_AGENT_OUT, (self.n_envs, self.n_agents, len(sfcfg.AGENT_OUT_FIELDS)), torch.int32)
+
+    def match_logs(self, env_ids=None, count=None, out=None):
+        """Match-log tapes (sf_log_list, DESIGN.md section 7h): a uint8 CUDA tensor [rows, sf_log_row_bytes], each
+        row a ``config.LOG_HEAD`` (flags, status, level, episode, steps, n_symbols, tb, serial, global_id) and the
+        tape's command symbols in the order of the reference's .sf_sample file; ``replay.write_device_log`` turns a
+        row into a file.  ``env_ids`` / ``count`` follow ``action_mask``: row i is arena env_ids[i], an id outside
+        [0, n_envs) gives an all-zero row, rows at and beyond ``count`` are whatever ``out`` held.  Needs
+        ``match_log`` at construction; no host synchronisation."""
+        row_bytes = lib().sf_log_row_bytes(self._h)
+        rows, ids, cnt = self.n_envs, None, None
+        if env_ids is not None:
+            ids = self._device_list(env_ids, "env_ids")
+            rows = env_ids.numel()
+            cnt = self._device_count(count)
+        else:
+            assert count is None, "count goes with env_ids"
+        if out is None:
+            out = torch.empty((rows, row_bytes), dtype=torch.uint8, device=self.device)
+        assert out.is_cuda and out.dtype == torch.uint8 and out.is_contiguous() and out.numel() == rows * row_bytes
+        self._chk(lib().sf_log_list(self._h, C.c_void_p(out.data_ptr()), ids, cnt, rows, self._stream()))
+        return out
 
     def state_hash(self):
         return self._get(sfcfg.FIELD_STATE_HASH, (self.n_envs,), torch.int64)
