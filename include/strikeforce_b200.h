@@ -132,7 +132,9 @@ enum {
     SF_FIELD_COUNTERS   = 3, /* int32[n_envs][8]: frame kills teams_kills loot chest steps status hp */
     SF_FIELD_POPULATION = 4, /* int32[n_envs][6]: humans zombies bullets chests built portals    */
     SF_FIELD_STATS      = 5, /* int64[16] device-reduced episode statistics (see SF_STAT_*)      */
-    SF_FIELD_AGENT_OUT  = 6  /* sf_agent_out[n_envs][agents_per_env], after sf_enable_agent_out   */
+    SF_FIELD_AGENT_OUT  = 6, /* sf_agent_out[n_envs][agents_per_env], after sf_enable_agent_out   */
+    SF_FIELD_REPLAY     = 7, /* sf_replay_state[n_envs], after sf_enable_replay                   */
+    SF_FIELD_REPLAY_DEALT = 8 /* uint8[n_envs][agents_per_env]: symbols dealt by the last step    */
 };
 
 /* slots of SF_FIELD_STATS: sums over the handle's arenas since sf_create (NCCL all-reduce
@@ -394,6 +396,69 @@ int32_t sf_log_row_bytes(const sf_handle *h);
    are not written.  Allowed at P1 and between sf_step_a and sf_step_b (the tape as it stands).  SF_ERR_ARG
    before sf_enable_log, for NULL rows, misalignment, n_max out of range and a count without env_ids. */
 int sf_log_list(sf_handle *h, void *rows, const int32_t *env_ids, const int32_t *count, int32_t n_max, void *stream);
+
+/* Replay (DESIGN.md section 7i): command tapes loaded into arenas and dealt by the step, the reading half of the
+   match logs above.  A handle opts in once with sf_enable_replay(h, cap_symbols); every arena then has a replay
+   tape and a replay state.
+   Loading: sf_replay_load takes rows in the layout sf_log_list exports (an sf_log_head, then the symbols, padded to
+   16 bytes; sf_replay_row_bytes equals sf_log_row_bytes of a handle with the same capacity, so an exported row loads
+   as it is).  It reads tb, serial, level, episode and n_symbols of the head and ignores the other fields.  Loading a
+   row into arena e resets e exactly as sf_reset(e, tb, serial) would, but with the head's level instead of the one
+   the global id gives and the head's episode as the episode counter; then it copies the tape and arms it (cursor 0,
+   SF_REPLAY_ARMED, steps 0, status SF_RUNNING).  A log this handle took, loaded back into the arena it came from,
+   gives the same log again when logs are on.  An entry is refused for n_symbols outside [0, cap_symbols], tb < 0 or
+   serial < 0, and a level outside [1, 64] (SF_MAX_LEVEL) or other than 1 on a Battle Royale handle.
+   Dealing: every step call of a replay handle (sf_step, sf_step_a + sf_step_b, sf_step_host, and sf_step_list for
+   the listed arenas) deals from armed tapes.  In human_action ind's symbol is the next tape symbol; then, in
+   ascending slot order, each human the logger records (the humans of SF_CONTROLLABLE_RULE on the state after
+   half-tick A other than ind: exactly those sf_log_list's tape appends for) takes the next tape symbol instead of
+   its action-row entry.  A symbol dealt to a squad agent is delivered as an action-row symbol is: outside
+   "+xzqeawsd" it becomes '+'.  Random NPCs and humans that are not recorded are not affected.  A step that needs a
+   symbol past the end of the tape takes that symbol and the rest of its symbols from the action row, sets
+   SF_REPLAY_EXHAUSTED and disarms the tape at the end of the step; later steps use the action rows.
+   End: a step that leaves an armed arena in a terminal status sets SF_REPLAY_ENDED, records the status and disarms
+   the tape, before any auto-reset; with symbols left over it also sets SF_REPLAY_SURPLUS (the replay left the
+   recorded episode: another sheet, capacities, max_steps or level, or a tape that is not one episode).  With
+   auto-reset the next episode follows the arena's own seed chain and the action rows.
+   sf_reset, sf_load and an accepted sf_load_list disarm the tapes of the arenas they overwrite; sf_reset_finished
+   does not touch the replay state.  Tapes and replay states are not part of arena records.
+   Outputs: sf_get(SF_FIELD_REPLAY) gives sf_replay_state[n_envs]; sf_get(SF_FIELD_REPLAY_DEALT) gives uint8
+   [n_envs][agents_per_env], entry a the symbol the arena's last step took from its tape for human slot a as it was
+   delivered to obey, 0 for a slot that took none (every step of a replay handle writes the rows of the arenas it
+   steps; unspecified between sf_step_a and sf_step_b).  Both are one launch and SF_ERR_ARG before the opt-in.
+   On a replay handle with no tape armed the state, sf_step_out, agent outputs, logs, statistics and records are
+   byte for byte those of a handle without replay; an armed tape makes the step ignore the action-row entry of
+   every slot it deals to. */
+typedef struct sf_replay_state {
+    int32_t flags;     /* SF_REPLAY_*                                                       */
+    int32_t cursor;    /* symbols dealt                                                     */
+    int32_t n_symbols; /* symbols on the tape                                               */
+    int32_t steps;     /* steps taken since the load                                        */
+    int32_t status;    /* SF_RUNNING, or how the replayed episode ended                     */
+} sf_replay_state;
+enum {
+    SF_REPLAY_ARMED = 1,     /* the next step deals from the tape                                 */
+    SF_REPLAY_EXHAUSTED = 2, /* a step needed a symbol past the end of the tape                   */
+    SF_REPLAY_ENDED = 4,     /* the replayed episode ended (status holds how)                     */
+    SF_REPLAY_SURPLUS = 8    /* it ended with symbols left over                                   */
+};
+
+/* Opt in to replay, once per handle: allocates zeroed tapes and states (counted by sf_device_bytes).  SF_ERR_ARG
+   between sf_step_a and sf_step_b, for cap_symbols outside [1, SF_LOG_CAP_MAX], and for a second call with another
+   capacity; a second call with the same capacity does nothing.  Probed for by symbol (SF_ABI_VERSION stays 3). */
+int sf_enable_replay(sf_handle *h, int32_t cap_symbols);
+
+/* bytes of one load row (equal to sf_log_row_bytes for the same capacity); 0 before sf_enable_replay */
+int32_t sf_replay_row_bytes(const sf_handle *h);
+
+/* Load the DEVICE rows (16-byte aligned, sf_replay_row_bytes each) into arenas, in stream order with no host
+   synchronisation (capturable in a CUDA graph), with the list rules and the all-or-nothing refusal of
+   sf_load_list: row i < min(*count, n_max) (count NULL: n_max) goes to arena env_ids[i]; an id outside [0, n_envs)
+   is skipped; a repeated id is loaded once, from its lowest live index; *status (device int32) becomes the number
+   of refused owning entries, and nothing changes unless it is 0.  SF_ERR_ARG before sf_enable_replay, between
+   sf_step_a and sf_step_b, for NULL or misaligned buffers and for n_max outside [1, n_envs]. */
+int sf_replay_load(sf_handle *h, const void *rows, const int32_t *env_ids, const int32_t *count, int32_t n_max,
+                   int32_t *status, void *stream);
 
 /* Copy a per-arena field into a DEVICE buffer (sizes above). */
 int sf_get(sf_handle *h, int32_t field, void *dev_out, void *stream);

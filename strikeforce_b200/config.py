@@ -52,6 +52,18 @@ def log_row_bytes(cap_symbols):
     return LOG_HEAD.itemsize + (cap_symbols + 15) // 16 * 16
 
 
+# replay (sf_enable_replay / sf_replay_load, include/strikeforce_b200.h, DESIGN.md section 7i)
+FIELD_REPLAY = 7        # sf_replay_state [n_envs], after sf_enable_replay
+FIELD_REPLAY_DEALT = 8  # uint8 [n_envs][n_agents]: the symbols the last step took from the tapes
+REPLAY_ARMED, REPLAY_EXHAUSTED, REPLAY_ENDED, REPLAY_SURPLUS = 1, 2, 4, 8  # bits of the flags field
+REPLAY_STATE = np.dtype([("flags", "<i4"), ("cursor", "<i4"), ("n_symbols", "<i4"), ("steps", "<i4"), ("status", "<i4")])
+
+
+def replay_row_bytes(cap_symbols):
+    """bytes of one load row (sf_replay_row_bytes): the layout of an exported match-log row"""
+    return log_row_bytes(cap_symbols)
+
+
 STAT_NAMES = ["steps", "episodes", "wins", "deaths", "timeouts", "truncated", "overflows", "ub_guards",
               "kills", "teams_kills", "loot", "rng_draws", "algo_bytes", "reserved0", "reserved1", "reserved2"]
 

@@ -1511,6 +1511,56 @@ SF_FN void sf_log_exit(const SfLog &lg, int env, const SfEnv &e)
     if (e.status == SF_OVERFLOW || e.status == SF_UB_GUARD) hd->flags |= SF_LOG_ABORTED;
 }
 
+/* ------------------------------------------------------------------ replay */
+
+/* The handle's replay tapes (sf_enable_replay, DESIGN.md section 7i): rows of row_bytes, [arena], each the load row
+ * as sf_replay_load copied it (an sf_log_head, then the symbols); the arenas' sf_replay_state; and the dealt rows,
+ * [slot][n_envs] bytes, so that the lanes of a warp store neighbouring bytes.  st == NULL: replay off. */
+struct SfReplay {
+    uint8_t *tapes;
+    sf_replay_state *st;
+    uint8_t *dealt;
+    int32_t row_bytes, cap;
+};
+
+SF_FN const uint8_t *sf_replay_tape(const SfReplay &rp, int env)
+{
+    return rp.tapes + (size_t)env * (size_t)rp.row_bytes + sizeof(sf_log_head);
+}
+
+/* the end of a step (or half) of an arena whose tape is armed: a terminal status ends the replay, an exhausted tape
+ * is disarmed (EXHAUSTED is only set in human_action, so only by the half that ends the step) */
+SF_FN void sf_replay_exit(const SfReplay &rp, int env, const SfEnv &e)
+{
+    sf_replay_state &s = rp.st[env];
+    int f = s.flags;
+    if (!(f & SF_REPLAY_ARMED)) return;
+    s.steps = (int32_t)e.steps;
+    if (e.status != SF_RUNNING) {
+        f = (f & ~SF_REPLAY_ARMED) | SF_REPLAY_ENDED | (s.cursor < s.n_symbols ? SF_REPLAY_SURPLUS : 0);
+        s.status = e.status;
+    } else if (f & SF_REPLAY_EXHAUSTED) {
+        f &= ~SF_REPLAY_ARMED;
+    }
+    s.flags = f;
+}
+
+/* sf_replay_load refuses a row whose head is not one this handle can play: a tape longer than its capacity,
+ * negative seeds (sf_reset refuses them too), or a level without tables (Battle Royale plays level 1 only) */
+SF_FN bool sf_replay_refused(const sf_log_head &hd, int32_t cap, int mode)
+{
+    return hd.n_symbols < 0 || hd.n_symbols > cap || hd.tb < 0 || hd.serial < 0 || hd.level < 1 ||
+           hd.level > SF_MAX_LEVEL || (mode == SF_MODE_ROYALE && hd.level != 1);
+}
+
+/* the replay state of an arena that has just taken a tape of n symbols */
+SF_FN void sf_replay_arm(const SfReplay &rp, int env, int32_t n)
+{
+    sf_replay_state s;
+    s.flags = SF_REPLAY_ARMED, s.cursor = 0, s.n_symbols = n, s.steps = 0, s.status = SF_RUNNING;
+    rp.st[env] = s;
+}
+
 /* human_action, gameplay.hpp:965-1012.  actions = this arena's row of the action buffer:
  * [ind] the player's command (get_my_action, :939-963; ind = 0 outside Battle Royale), the other
  * entries what bot() returns for the agent-driven squad humans (bots/bot-0.5/Custom.hpp:137-158, one
@@ -1518,17 +1568,36 @@ SF_FN void sf_log_exit(const SfLog &lg, int env, const SfEnv &e)
  *
  * LOG (sf_enable_log, DESIGN.md section 7h): with lg.rows set, the symbols the reference's logger writes go to the
  * arena's tape -- ind's first, then in the gather loop every live Battle Royale player and squad agent (the
- * humans of SF_CONTROLLABLE_RULE other than ind) with the symbol it is delivered. */
+ * humans of SF_CONTROLLABLE_RULE other than ind) with the symbol it is delivered.  With rp.st set and the arena's
+ * replay tape armed, the same humans in the same order take their symbols from the tape instead of the action row
+ * (DESIGN.md section 7i), a squad agent's through the same delivery rule, and the symbols dealt go to the dealt row;
+ * past the end of the tape the rest come from the action row and the state gets EXHAUSTED. */
 template <bool LOG = false>
 SF_FN void sf_human_action(const SfDev &d, const SfConst &k, const SfTabs &t, int env, SfEnv &e,
-                           const uint8_t *actions, SfLog lg = SfLog{})
+                           const uint8_t *actions, SfLog lg = SfLog{}, SfReplay rp = SfReplay{})
 {
     /* commands wait in h_cmd between the two loops (command[], gameplay.hpp:43) */
     const uint64_t live = e.on ? e.mh : 0ull;
     const int hi = SF_WARP_MAX(live ? sf_fls64(live) : -1);
     const int ind = k.ind;
-    const int cmd0 = (actions && e.on) ? actions[ind] : '+';
+    int cmd0 = (actions && e.on) ? actions[ind] : '+';
+    /* replay: armed at entry, still dealing, cursor, tape length */
+    bool rp_armed = false, rp_on = false;
+    int rp_cur = 0, rp_n = 0;
     if constexpr (LOG) {
+        if (rp.st && e.on) {
+            const sf_replay_state s = rp.st[env];
+            rp_armed = rp_on = (s.flags & SF_REPLAY_ARMED) != 0;
+            rp_cur = s.cursor, rp_n = s.n_symbols;
+        }
+        if (rp_on) {
+            if (rp_cur < rp_n) {
+                cmd0 = sf_replay_tape(rp, env)[rp_cur++];
+                rp.dealt[(size_t)ind * (size_t)d.n_envs + (size_t)env] = (uint8_t)cmd0;
+            } else {
+                rp_on = false;
+            }
+        }
         if (lg.rows && e.on) sf_log_put(lg, env, cmd0);
     }
     for (int h = 0; h <= hi; ++h) {
@@ -1547,12 +1616,30 @@ SF_FN void sf_human_action(const SfDev &d, const SfConst &k, const SfTabs &t, in
                 if (!ok) c = '+';
             }
             if constexpr (LOG) {
-                if (lg.rows && ((k.mode == SF_MODE_ROYALE && h < k.n_players) || ((sel & HS_AGENT) && h < k.n_agents)))
-                    sf_log_put(lg, env, c);
+                const bool player = k.mode == SF_MODE_ROYALE && h < k.n_players;
+                const bool logged = player || ((sel & HS_AGENT) && h < k.n_agents);
+                if (logged && rp_on) {
+                    if (rp_cur < rp_n) {
+                        c = sf_replay_tape(rp, env)[rp_cur++];
+                        bool ok = player || c == '+' || c == 'x' || c == 'z' || c == 'q' || c == 'e' || c == 'a' ||
+                                  c == 'w' || c == 's' || c == 'd';
+                        if (!ok) c = '+';
+                        rp.dealt[(size_t)h * (size_t)d.n_envs + (size_t)env] = (uint8_t)c;
+                    } else {
+                        rp_on = false;
+                    }
+                }
+                if (lg.rows && logged) sf_log_put(lg, env, c);
             }
         }
         if (is_live) SF_AT(d.h_cmd, h) = (uint8_t)c;
         SF_SYNCWARP();
+    }
+    if constexpr (LOG) {
+        if (rp_armed) {
+            rp.st[env].cursor = rp_cur;
+            if (!rp_on) rp.st[env].flags |= SF_REPLAY_EXHAUSTED;
+        }
     }
     int r = 0;
     if (e.on) r = sf_rand(e, t) & 1;
@@ -1845,7 +1932,7 @@ SF_FN void sf_eval_end(const SfDev &d, const SfConst &k, int env, SfEnv &e)
  * portal_damage (:1444-1456), round 1 = human_action (:1464). */
 template <bool LOG = false>
 SF_FN void sf_step_halves(const SfDev &d, const SfConst &k, const SfTabs &t, int env, SfEnv &e,
-                          const uint8_t *actions, int first, int last, SfLog lg = SfLog{})
+                          const uint8_t *actions, int first, int last, SfLog lg = SfLog{}, SfReplay rp = SfReplay{})
 {
 #pragma unroll 1
     for (int ph = first; ph <= last; ++ph) {
@@ -1857,7 +1944,7 @@ SF_FN void sf_step_halves(const SfDev &d, const SfConst &k, const SfTabs &t, int
             SF_PHASE_SYNC(2);
             sf_portal_damage(d, k, t, env, e);
         } else {
-            sf_human_action<LOG>(d, k, t, env, e, actions, lg);
+            sf_human_action<LOG>(d, k, t, env, e, actions, lg, rp);
         }
         SF_PHASE_SYNC(3);
         sf_resolve_bullets(d, k, t, env, e);
@@ -1935,9 +2022,11 @@ struct SfStatDelta {
     int32_t kills, tkills, loot;
 };
 
-/* reset one arena for episode `episode` with explicit seeds */
+/* reset one arena for episode `episode` with explicit seeds.  kLevel (sf_replay_load): the arena plays `level`
+ * instead of the level its global id gives (the reset itself reads no level: it only sets it) */
+template <bool kLevel = false>
 SF_FN void sf_reset_body(const SfDev &d, const SfConst &k, const SfTabs &t, int env, int64_t tb, int64_t serial,
-                         uint32_t episode)
+                         uint32_t episode, int level = 0)
 {
     SfEnv e;
     e.episode = episode;
@@ -1945,6 +2034,7 @@ SF_FN void sf_reset_body(const SfDev &d, const SfConst &k, const SfTabs &t, int 
     e.bank = (d.misc[env] >> 25) & 1u;
     sf_seed_pending(d, t, env, e.bank ? 0 : 1, tb, serial);
     sf_reset_env(d, k, t, env, e);
+    if constexpr (kLevel) e.level = level;
     sf_store_env(d, env, e);
     sf_step_out o;
     o.status = SF_RUNNING, o.d_kills = o.d_teams_kills = o.d_loot = o.d_hp = o.d_damage = o.d_effect = 0;
@@ -1985,11 +2075,15 @@ SF_FN void sf_reset_finished_body(const SfDev &d, const SfConst &k, const SfTabs
  *   driven slot, half B (or the whole step) adds the values at exit and DIED, before any auto-reset.
  * - Match logs (sf_enable_log, DESIGN.md section 7h): `lg` holds the handle's tapes.  Half A (or the
  *   whole step) restarts the tape of an arena at step count 0, sf_human_action appends, and the half
- *   that ran writes the status and step count, before any auto-reset. */
+ *   that ran writes the status and step count, before any auto-reset.
+ * - Replay (sf_enable_replay, DESIGN.md section 7i): `rp` holds the handle's replay tapes and states.  Half A (or
+ *   the whole step) clears the arena's dealt row, sf_human_action deals from an armed tape, and the half that ran
+ *   ends or disarms the replay (sf_replay_exit), before any auto-reset. */
 #define SF_AO(field, a) ao[((size_t)(field) * (size_t)k.n_agents + (size_t)(a)) * (size_t)d.n_envs + (size_t)env]
 template <bool EXTRAS = false>
 SF_FN void sf_step_body(const SfDev &d, const SfConst &k, const SfTabs &t, int env, bool valid,
-                        const uint8_t *actions, int half, SfStatDelta &sd, int32_t *ao = nullptr, SfLog lg = SfLog{})
+                        const uint8_t *actions, int half, SfStatDelta &sd, int32_t *ao = nullptr, SfLog lg = SfLog{},
+                        SfReplay rp = SfReplay{})
 {
     if (half != SF_HALF_B) {
         sf_advance_pending(d, t, env, valid, SF_WARM_PER_STEP);
@@ -2019,11 +2113,15 @@ SF_FN void sf_step_body(const SfDev &d, const SfConst &k, const SfTabs &t, int e
                 }
             }
             if (lg.rows && half != SF_HALF_B && e.on && e.steps == 0) sf_log_restart(d, k, t, lg, env, e);
+            if (rp.st && half != SF_HALF_B) {
+#pragma unroll 1
+                for (int a = 0; a < k.n_agents; ++a) rp.dealt[(size_t)a * (size_t)d.n_envs + (size_t)env] = 0;
+            }
         }
     }
     if (half != SF_HALF_B && e.on) sd.algo_bytes += sf_algo_bytes(k, e);
     sf_bt_rebuild(d, t, env, e);
-    sf_step_halves<EXTRAS>(d, k, t, env, e, actions, half == SF_HALF_B ? 1 : 0, half == SF_HALF_A ? 0 : 1, lg);
+    sf_step_halves<EXTRAS>(d, k, t, env, e, actions, half == SF_HALF_B ? 1 : 0, half == SF_HALF_A ? 0 : 1, lg, rp);
     if (valid) {
         /* a terminal arena that is not auto-reset waits for sf_reset: report, change nothing */
         sf_step_out o = d.out[env];
@@ -2047,6 +2145,7 @@ SF_FN void sf_step_body(const SfDev &d, const SfConst &k, const SfTabs &t, int e
                 }
             }
             if (lg.rows && was_on) sf_log_exit(lg, env, e);
+            if (rp.st) sf_replay_exit(rp, env, e);
         }
     }
     /* Auto-reset happens at the end of the whole step: an episode that ends in half A (an overflow or

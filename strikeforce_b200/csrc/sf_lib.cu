@@ -14,6 +14,7 @@
 
 #include <cstdio>
 #include <cstdlib>
+#include <algorithm>
 #include <cstring>
 #include <new>
 #include <string>
@@ -109,13 +110,13 @@ __device__ __forceinline__ void sf_flush_stats(const SfDev &d, const SfStatDelta
  * EXTRAS: the opt-in outputs, each written when its buffer is set -- agent outputs (sf_enable_agent_out, DESIGN.md
  * section 7g): the stepped arenas write their rows of the handle's agent-output buffer agent_out ([field][slot][n_envs]:
  * the lanes of a warp store neighbouring words); match logs (sf_enable_log, section 7h): they restart and append to
- * their tapes in log.  The buffers are the last parameters, so that the parameters the other instantiations read keep
- * their offsets. */
+ * their tapes in log; replay (sf_enable_replay, section 7i): they deal from armed tapes in replay.  The buffers are the
+ * last parameters, so that the parameters the other instantiations read keep their offsets. */
 template <int HALF, bool LIST, bool EXTRAS>
 __global__ void __launch_bounds__(SF_CTA, 1)
 sf_step_kernel(const SfDev d, const __grid_constant__ SfConst k, const uint8_t *__restrict__ actions, int lpw,
                const int32_t *__restrict__ env_ids, const int32_t *__restrict__ list_n, int n_max,
-               const int32_t *__restrict__ claim, int32_t *__restrict__ agent_out, const SfLog log)
+               const int32_t *__restrict__ claim, int32_t *__restrict__ agent_out, const SfLog log, const SfReplay replay)
 {
     SfTabs t;
     sf_stage_tables(d, t);
@@ -149,10 +150,10 @@ sf_step_kernel(const SfDev d, const __grid_constant__ SfConst k, const uint8_t *
             const int id = valid ? env_ids[env] : -1;
             const uint8_t *row = actions + (size_t)env * k.n_agents;
             valid = id >= 0 && id < d.n_envs && claim[id] == env;
-            sf_step_body<EXTRAS>(d, k, t, valid ? id : lane, valid, valid ? row : nullptr, HALF, sd, agent_out, log);
+            sf_step_body<EXTRAS>(d, k, t, valid ? id : lane, valid, valid ? row : nullptr, HALF, sd, agent_out, log, replay);
         } else {
             sf_step_body<EXTRAS>(d, k, t, env, valid, (actions && valid) ? actions + (size_t)env * k.n_agents : nullptr, HALF,
-                                 sd, agent_out, log);
+                                 sd, agent_out, log, replay);
         }
         __syncwarp();
         sf_flush_stats(d, sd);
@@ -1084,6 +1085,71 @@ __global__ void sf_log_unload_kernel(uint8_t *__restrict__ tapes, int row_bytes,
     }
 }
 
+/* sf_reset / sf_load / sf_load_list on a replay handle: disarm the tapes of the arenas they overwrite -- entry
+ * i < min(*list_n, n) (list_n NULL: n) with an id in range (ids NULL: arena i), unless the load was refused
+ * (refused NULL: a reset, never refused; else *refused != 0, read here on the device). */
+__global__ void sf_replay_disarm_kernel(sf_replay_state *__restrict__ st, int n_envs, const int32_t *__restrict__ ids,
+                                        const int32_t *__restrict__ list_n, int n, const int32_t *__restrict__ refused)
+{
+    if (refused && *refused != 0) return;
+    const int m = list_n ? min(max(*list_n, 0), n) : n;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < m; i += gridDim.x * blockDim.x) {
+        const int id = ids ? ids[i] : i;
+        if (id >= 0 && id < n_envs) st[id].flags &= ~SF_REPLAY_ARMED;
+    }
+}
+
+/* sf_replay_load, check: count the owning entries whose head sf_replay_refused refuses into *status */
+__global__ void sf_replay_check_kernel(const uint8_t *__restrict__ rows, int row_bytes,
+                                       int32_t cap, int mode, const int32_t *__restrict__ ids, const int32_t *__restrict__ list_n,
+                                       int n_max, int n_envs, const int32_t *__restrict__ claim, int32_t *__restrict__ status)
+{
+    const int n = list_n ? min(max(*list_n, 0), n_max) : n_max;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const int id = ids[i];
+        if (id < 0 || id >= n_envs || claim[id] != i) continue;
+        const sf_log_head hd = *reinterpret_cast<const sf_log_head *>(rows + (size_t)i * row_bytes);
+        if (sf_replay_refused(hd, cap, mode)) atomicAdd(status, 1);
+    }
+}
+
+/* sf_replay_load, apply (only if *status == 0): every owning entry resets its arena as sf_reset_kernel does, with the
+ * head's seeds, episode and level, and arms the tape; then the grid copies the rows into the tapes, one 16-byte word
+ * per thread and step of the loop.  The tables are staged as in sf_reset_kernel. */
+__global__ void __launch_bounds__(SF_CTA, 1)
+sf_replay_apply_kernel(const SfDev d, const __grid_constant__ SfConst k, const SfReplay rp, const uint8_t *__restrict__ rows,
+                       const int32_t *__restrict__ ids, const int32_t *__restrict__ list_n, int n_max,
+                       const int32_t *__restrict__ claim, const int32_t *__restrict__ status)
+{
+    if (*status != 0) return; /* the same value in every thread: no barrier is skipped by some threads only */
+    SfTabs t;
+    sf_stage_tables(d, t);
+    const int n = list_n ? min(max(*list_n, 0), n_max) : n_max;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const int id = ids[i];
+        if (id < 0 || id >= d.n_envs || claim[id] != i) continue;
+        const sf_log_head hd = *reinterpret_cast<const sf_log_head *>(rows + (size_t)i * rp.row_bytes);
+        sf_reset_body<true>(d, k, t, id, hd.tb, hd.serial, hd.episode, hd.level);
+        sf_replay_arm(rp, id, hd.n_symbols);
+    }
+    const int row_words = rp.row_bytes / 16;
+    const long words = (long)n * row_words;
+    for (long w = (long)blockIdx.x * blockDim.x + threadIdx.x; w < words; w += (long)gridDim.x * blockDim.x) {
+        const long i = w / row_words;
+        const int id = ids[i];
+        if (id < 0 || id >= d.n_envs || claim[id] != (int)i) continue;
+        reinterpret_cast<uint4 *>(rp.tapes)[(long)id * row_words + (w - i * row_words)] = reinterpret_cast<const uint4 *>(rows)[w];
+    }
+}
+
+/* sf_get(SF_FIELD_REPLAY_DEALT): the dealt rows, [slot][n_envs], as uint8 [n_envs][slot], one thread per output byte */
+__global__ void sf_replay_dealt_kernel(const uint8_t *__restrict__ dealt, int n_envs, int n_agents, uint8_t *__restrict__ out)
+{
+    const long n = (long)n_envs * n_agents;
+    for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x)
+        out[i] = dealt[(i % n_agents) * n_envs + i / n_agents];
+}
+
 /* ====================================================================== host side */
 
 struct sf_handle {
@@ -1106,6 +1172,7 @@ struct sf_handle {
     int32_t *d_claim = nullptr;   /* sf_step_list: the list entry that steps each arena; INT32_MAX between calls */
     int32_t *d_agent_out = nullptr; /* sf_enable_agent_out: [field][slot][n_envs] (its own allocation), or NULL */
     SfLog log = {nullptr, 0, 0};    /* sf_enable_log: the tapes, [n_envs][row_bytes] (their own allocation) */
+    SfReplay replay = {nullptr, nullptr, nullptr, 0, 0}; /* sf_enable_replay: tapes, states and dealt rows (one allocation) */
     SfSnapLayout snap;           /* the record layout of sf_save / sf_load (sf_snapshot.cuh) */
     int device = 0, n_sm = 0;
     bool between_halves = false; /* sf_step_a has run, sf_step_b has not: the P2 observation point */
@@ -1315,6 +1382,7 @@ int sf_create(const sf_config *cfg, sf_handle **out)
     SF_STEP_SMEM_ATTRS(true);
 #undef SF_STEP_SMEM_ATTRS
     SF_CREATE_CUDA(cudaFuncSetAttribute(sf_reset_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
+    SF_CREATE_CUDA(cudaFuncSetAttribute(sf_replay_apply_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
     SF_CREATE_CUDA(cudaFuncSetAttribute(sf_rng_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SF_SMEM_BYTES));
 #define SF_OBS_SMEM_ATTR(NHWC, LIST, T) \
     SF_CREATE_CUDA(cudaFuncSetAttribute(sf_observe_kernel<NHWC, LIST, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, sf_obs_smem<T, NHWC>()))
@@ -1350,6 +1418,7 @@ int sf_destroy(sf_handle *h)
         cudaFree(h->arena);
         if (h->d_agent_out) cudaFree(h->d_agent_out);
         if (h->log.rows) cudaFree(h->log.rows);
+        if (h->replay.tapes) cudaFree(h->replay.tapes);
     }
     delete h;
     return SF_OK;
@@ -1376,6 +1445,12 @@ int sf_reset(sf_handle *h, const int32_t *env_ids, int32_t n, const int64_t *tb,
     }
     int rc = sf_launch_reset(h, env_ids ? h->d_ids : nullptr, n, tb ? h->d_tb : nullptr, tb ? h->d_serial : nullptr, s);
     if (rc) return rc;
+    if (h->replay.st) {
+        sf_replay_disarm_kernel<<<(n + 255) / 256, 256, 0, s>>>(h->replay.st, h->d.n_envs, env_ids ? h->d_ids : nullptr,
+                                                                nullptr, n, nullptr);
+        h->launches += 1;
+        SF_CUDA(h, cudaGetLastError());
+    }
     h->between_halves = false;
     /* the staging buffers are reused by the next call */
     SF_CUDA(h, cudaStreamSynchronize(s));
@@ -1400,15 +1475,16 @@ static int sf_launch_step(sf_handle *h, int half, const uint8_t *d_actions, cuda
     int grid = nchunks < h->n_sm ? nchunks : h->n_sm; /* one persistent CTA per SM; warps take chunks round-robin over the CTAs */
     int32_t *ao = h->d_agent_out;
     const SfLog lg = h->log;
+    const SfReplay rp = h->replay;
 #define SF_STEP_LAUNCH(EXTRAS)                                                                                                  \
     do {                                                                                                                        \
         if (half == SF_HALF_BOTH)                                                                                               \
-            sf_step_kernel<SF_HALF_BOTH, false, EXTRAS><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, d_actions, lpw, nullptr, nullptr, 0, nullptr, ao, lg); \
+            sf_step_kernel<SF_HALF_BOTH, false, EXTRAS><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, d_actions, lpw, nullptr, nullptr, 0, nullptr, ao, lg, rp); \
         else if (half == SF_HALF_A)                                                                                             \
-            sf_step_kernel<SF_HALF_A, false, EXTRAS><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, nullptr, lpw, nullptr, nullptr, 0, nullptr, ao, lg); \
-        else sf_step_kernel<SF_HALF_B, false, EXTRAS><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, d_actions, lpw, nullptr, nullptr, 0, nullptr, ao, lg); \
+            sf_step_kernel<SF_HALF_A, false, EXTRAS><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, nullptr, lpw, nullptr, nullptr, 0, nullptr, ao, lg, rp); \
+        else sf_step_kernel<SF_HALF_B, false, EXTRAS><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, d_actions, lpw, nullptr, nullptr, 0, nullptr, ao, lg, rp); \
     } while (0)
-    if (ao || lg.rows) SF_STEP_LAUNCH(true);
+    if (ao || lg.rows || rp.st) SF_STEP_LAUNCH(true);
     else SF_STEP_LAUNCH(false);
 #undef SF_STEP_LAUNCH
     h->launches += 1;
@@ -1435,12 +1511,12 @@ int sf_step_list(sf_handle *h, const uint8_t *actions, const int32_t *env_ids, c
     int cgrid = (n_max + 255) / 256;
     if (cgrid > 4 * h->n_sm) cgrid = 4 * h->n_sm;
     sf_claim_kernel<false><<<cgrid, 256, 0, s>>>(env_ids, count, n_max, h->d.n_envs, h->d_claim);
-    if (h->d_agent_out || h->log.rows)
+    if (h->d_agent_out || h->log.rows || h->replay.st)
         sf_step_kernel<SF_HALF_BOTH, true, true><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, actions, lpw, env_ids, count, n_max,
-                                                                                   h->d_claim, h->d_agent_out, h->log);
+                                                                                   h->d_claim, h->d_agent_out, h->log, h->replay);
     else
         sf_step_kernel<SF_HALF_BOTH, true, false><<<grid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, actions, lpw, env_ids, count, n_max,
-                                                                                    h->d_claim, nullptr, h->log);
+                                                                                    h->d_claim, nullptr, h->log, h->replay);
     sf_claim_kernel<true><<<cgrid, 256, 0, s>>>(env_ids, count, n_max, h->d.n_envs, h->d_claim);
     h->launches += 3;
     SF_CUDA(h, cudaGetLastError());
@@ -1711,6 +1787,67 @@ int sf_log_list(sf_handle *h, void *rows, const int32_t *env_ids, const int32_t 
     return SF_OK;
 }
 
+int sf_enable_replay(sf_handle *h, int32_t cap_symbols)
+{
+    if (!h) return SF_ERR_ARG;
+    if (h->between_halves) return sf_fail(h, SF_ERR_ARG, "sf_enable_replay: the step opened by sf_step_a is still waiting for sf_step_b");
+    if (cap_symbols < 1 || cap_symbols > SF_LOG_CAP_MAX)
+        return sf_fail(h, SF_ERR_ARG, "sf_enable_replay: cap_symbols must be in [1, SF_LOG_CAP_MAX]");
+    if (h->replay.st)
+        return cap_symbols == h->replay.cap ? SF_OK : sf_fail(h, SF_ERR_ARG, "sf_enable_replay: replay is on with another capacity");
+    SfDeviceGuard guard(h);
+    /* one allocation: the tapes (the load rows' layout), the states, the dealt rows ([slot][n_envs]) */
+    const int32_t row_bytes = (int32_t)sizeof(sf_log_head) + ((cap_symbols + 15) & ~15);
+    const size_t n = (size_t)h->d.n_envs, tape_bytes = n * (size_t)row_bytes;
+    const size_t st_bytes = (n * sizeof(sf_replay_state) + 15) & ~(size_t)15;
+    const size_t bytes = tape_bytes + st_bytes + n * (size_t)h->k.n_agents;
+    uint8_t *p = nullptr;
+    SF_CUDA(h, cudaMalloc(&p, bytes));
+    /* zeroed before any stream of the caller can step with it: no tape is armed */
+    cudaError_t e = cudaMemset(p, 0, bytes);
+    if (e == cudaSuccess) e = cudaDeviceSynchronize();
+    if (e != cudaSuccess) {
+        cudaFree(p);
+        return sf_fail(h, SF_ERR_CUDA, std::string("sf_enable_replay: ") + cudaGetErrorString(e));
+    }
+    h->replay = SfReplay{p, reinterpret_cast<sf_replay_state *>(p + tape_bytes), p + tape_bytes + st_bytes, row_bytes, cap_symbols};
+    h->arena_bytes += bytes;
+    return SF_OK;
+}
+
+int32_t sf_replay_row_bytes(const sf_handle *h) { return h ? h->replay.row_bytes : 0; }
+
+int sf_replay_load(sf_handle *h, const void *rows, const int32_t *env_ids, const int32_t *count, int32_t n_max,
+                   int32_t *status, void *stream)
+{
+    if (!h) return SF_ERR_ARG;
+    if (!h->replay.st) return sf_fail(h, SF_ERR_ARG, "sf_replay_load: needs sf_enable_replay first");
+    if (h->between_halves) return sf_fail(h, SF_ERR_ARG, "sf_replay_load: the step opened by sf_step_a is still waiting for sf_step_b");
+    if (!rows || !env_ids || !status) return sf_fail(h, SF_ERR_ARG, "sf_replay_load: null buffer");
+    if (n_max < 1 || n_max > h->d.n_envs) return sf_fail(h, SF_ERR_ARG, "sf_replay_load: n_max must be in [1, n_envs]");
+    if (reinterpret_cast<uintptr_t>(rows) & 15u) return sf_fail(h, SF_ERR_ARG, "sf_replay_load: rows must be 16-byte aligned");
+    if ((reinterpret_cast<uintptr_t>(env_ids) | reinterpret_cast<uintptr_t>(count) | reinterpret_cast<uintptr_t>(status)) & 3u)
+        return sf_fail(h, SF_ERR_ARG, "sf_replay_load: env_ids, count and status must be 4-byte aligned");
+    SfDeviceGuard guard(h);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const uint8_t *r = static_cast<const uint8_t *>(rows);
+    /* claim, check (counts the refused owners into *status), apply (returns at once unless *status == 0), release.
+       The apply grid has a thread per entry for the resets and up to a thread per 16-byte word of the copy. */
+    int cgrid = (n_max + 255) / 256;
+    if (cgrid > 4 * h->n_sm) cgrid = 4 * h->n_sm;
+    const long words = (long)n_max * (h->replay.row_bytes / 16);
+    const int agrid = (int)std::min<long>((words + SF_CTA - 1) / SF_CTA, (long)h->n_sm);
+    SF_CUDA(h, cudaMemsetAsync(status, 0, sizeof(int32_t), s));
+    sf_claim_kernel<false><<<cgrid, 256, 0, s>>>(env_ids, count, n_max, h->d.n_envs, h->d_claim);
+    sf_replay_check_kernel<<<cgrid, 256, 0, s>>>(r, h->replay.row_bytes, h->replay.cap, h->k.mode, env_ids, count, n_max,
+                                                 h->d.n_envs, h->d_claim, status);
+    sf_replay_apply_kernel<<<agrid, SF_CTA, SF_SMEM_BYTES, s>>>(h->d, h->k, h->replay, r, env_ids, count, n_max, h->d_claim, status);
+    sf_claim_kernel<true><<<cgrid, 256, 0, s>>>(env_ids, count, n_max, h->d.n_envs, h->d_claim);
+    h->launches += 4;
+    SF_CUDA(h, cudaGetLastError());
+    return SF_OK;
+}
+
 int sf_get(sf_handle *h, int32_t field, void *dev_out, void *stream)
 {
     if (!h || !dev_out) return h ? sf_fail(h, SF_ERR_ARG, "sf_get: null buffer") : SF_ERR_ARG;
@@ -1739,6 +1876,18 @@ int sf_get(sf_handle *h, int32_t field, void *dev_out, void *stream)
         long ag = (words + 255) / 256;
         if (ag > 8L * h->n_sm) ag = 8L * h->n_sm;
         sf_agent_out_kernel<<<(int)ag, 256, 0, s>>>(h->d_agent_out, n, h->k.n_agents, static_cast<int32_t *>(dev_out));
+        break;
+    }
+    case SF_FIELD_REPLAY:
+        if (!h->replay.st) return sf_fail(h, SF_ERR_ARG, "sf_get: SF_FIELD_REPLAY needs sf_enable_replay first");
+        SF_CUDA(h, cudaMemcpyAsync(dev_out, h->replay.st, (size_t)n * sizeof(sf_replay_state), cudaMemcpyDeviceToDevice, s));
+        return SF_OK;
+    case SF_FIELD_REPLAY_DEALT: {
+        if (!h->replay.st) return sf_fail(h, SF_ERR_ARG, "sf_get: SF_FIELD_REPLAY_DEALT needs sf_enable_replay first");
+        const long bytes = (long)n * h->k.n_agents;
+        long dg = (bytes + 255) / 256;
+        if (dg > 8L * h->n_sm) dg = 8L * h->n_sm;
+        sf_replay_dealt_kernel<<<(int)dg, 256, 0, s>>>(h->replay.dealt, n, h->k.n_agents, static_cast<uint8_t *>(dev_out));
         break;
     }
     default:
@@ -1868,6 +2017,10 @@ int sf_load(sf_handle *h, const int32_t *env_ids, int32_t n, const void *records
                                                              h->d_refused);
         h->launches += 1;
     }
+    if (h->replay.st) {
+        sf_replay_disarm_kernel<<<(n + 255) / 256, 256, 0, s>>>(h->replay.st, h->d.n_envs, d_ids, nullptr, n, h->d_refused);
+        h->launches += 1;
+    }
     SF_CUDA(h, cudaGetLastError());
     int refused = 0;
     SF_CUDA(h, cudaMemcpyAsync(&refused, h->d_refused, sizeof refused, cudaMemcpyDeviceToHost, s));
@@ -1936,6 +2089,10 @@ int sf_load_list(sf_handle *h, const void *records, int32_t n_records, const int
     h->launches += 5;
     if (h->log.rows) {
         sf_log_unload_kernel<<<cgrid, 256, 0, s>>>(h->log.rows, h->log.row_bytes, h->d.n_envs, env_ids, count, n_max, st);
+        h->launches += 1;
+    }
+    if (h->replay.st) {
+        sf_replay_disarm_kernel<<<cgrid, 256, 0, s>>>(h->replay.st, h->d.n_envs, env_ids, count, n_max, st);
         h->launches += 1;
     }
     SF_CUDA(h, cudaGetLastError());

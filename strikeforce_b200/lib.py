@@ -20,7 +20,8 @@ EXPORTS = [
     "sf_step_host", "sf_step_list", "sf_synth_actions", "sf_observe", "sf_list_finished", "sf_reset_finished", "sf_observe_list",
     "sf_get", "sf_export_env", "sf_snapshot_bytes", "sf_save", "sf_load", "sf_save_list", "sf_load_list",
     "sf_rng_stream", "sf_agents_per_env", "sf_num_envs", "sf_launch_count", "sf_device_bytes", "sf_action_mask",
-    "sf_enable_agent_out", "sf_enable_log", "sf_log_row_bytes", "sf_log_list",
+    "sf_enable_agent_out", "sf_enable_log", "sf_log_row_bytes", "sf_log_list", "sf_enable_replay", "sf_replay_row_bytes",
+    "sf_replay_load",
 ]
 
 _lib = None
@@ -80,6 +81,9 @@ def lib():
         L.sf_enable_log.argtypes = [vp, i32]
         L.sf_log_row_bytes.argtypes = [vp]
         L.sf_log_list.argtypes = [vp, vp, vp, vp, i32, vp]
+        L.sf_enable_replay.argtypes = [vp, i32]
+        L.sf_replay_row_bytes.argtypes = [vp]
+        L.sf_replay_load.argtypes = [vp, vp, vp, vp, i32, vp, vp]
         L.sf_rng_stream.argtypes = [vp, vp, vp, i32, i32, vp]
         L.sf_agents_per_env.argtypes = [vp]
         L.sf_num_envs.argtypes = [vp]

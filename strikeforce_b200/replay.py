@@ -175,6 +175,49 @@ def write_device_log(path, row, cfg, name="1"):
     return int(head["level"])
 
 
+def tape_rows(logs, cfg, cap, levels=1):
+    """Load rows for ``BatchedArena.replay_load`` (uint8 numpy [len(logs), config.replay_row_bytes(cap)]) from
+    ``MatchLog`` / ``RoyaleLog`` objects (``read`` / ``read_royale``) for a handle created with configuration ``cfg``
+    and ``replay=cap``.  ``levels``: the level of each offline log, or one level for all (the offline format does not
+    carry it); Battle Royale plays level 1.  The head holds the log's seeds, the level, episode 0 and the number of
+    symbols.  Rows exported by ``BatchedArena.match_logs()`` are already load rows.
+
+    The device never sees character sheets, so a log the handle cannot replay raises ValueError: an offline log on a
+    Battle Royale handle or the reverse, a player sheet, teams, ``ind`` or sheets other than what ``write_device_log``
+    writes for ``cfg``, or more symbols than ``cap``."""
+    from . import config as sfcfg
+    logs = list(logs)
+    levels = list(levels) if np.ndim(levels) else [int(levels)] * len(logs)
+    assert len(levels) == len(logs)
+    rows = np.zeros((len(logs), sfcfg.replay_row_bytes(cap)), dtype=np.uint8)
+    royale = cfg.mode == sfcfg.MODE_ROYALE
+    for i, (log, level) in enumerate(zip(logs, levels)):
+        if royale:
+            if not isinstance(log, RoyaleLog):
+                raise ValueError("log %d: an offline match log cannot be replayed on a Battle Royale handle" % i)
+            n = cfg.royale_players
+            sheets = np.array([list(cfg.royale_sheets[j]) for j in range(n)], dtype=np.int32)
+            if (log.ind != cfg.royale_ind or list(log.teams) != [cfg.royale_teams[j] for j in range(n)]
+                    or log.sheets.shape != sheets.shape or (log.sheets != sheets).any()):
+                raise ValueError("log %d: players, ind, teams or sheets differ from the handle's" % i)
+            level = 1
+        else:
+            if not isinstance(log, MatchLog):
+                raise ValueError("log %d: a Battle Royale match log needs a Battle Royale handle" % i)
+            if (log.players, log.ind, log.team) != (1, 0, 1):
+                raise ValueError("log %d: not an offline match of one player (players %d, ind %d, team %d)"
+                                 % (i, log.players, log.ind, log.team))
+            if (log.sheet != logged_sheet(list(cfg.player_sheet))).any():
+                raise ValueError("log %d: the player sheet differs from the handle's" % i)
+        if len(log.commands) > cap:
+            raise ValueError("log %d: %d symbols do not fit tapes of %d" % (i, len(log.commands), cap))
+        head = np.zeros(1, dtype=sfcfg.LOG_HEAD)
+        head["level"], head["n_symbols"], head["tb"], head["serial"] = level, len(log.commands), log.tb, log.serial
+        rows[i, :sfcfg.LOG_HEAD.itemsize] = head.view(np.uint8)
+        rows[i, sfcfg.LOG_HEAD.itemsize:sfcfg.LOG_HEAD.itemsize + len(log.commands)] = np.frombuffer(log.commands, np.uint8)
+    return rows
+
+
 def commands_per_step(log: MatchLog, n_agents_alive):
     """Split the command stream into steps: ``n_agents_alive(step)`` = number of logged humans that
     step (1 offline without squad agents)."""

@@ -25,10 +25,11 @@ _OBS_FORMAT = {torch.float32: 0, torch.float16: sfcfg.OBS_F16, torch.bfloat16: s
 class BatchedArena:
     def __init__(self, n_envs, mode="Solo", level=1, level_max=None, squad_agents=False, auto_reset=True,
                  max_steps=0, env_id_base=0, player="account1", caps=None, arena=None, device=None, teams=None, sheets=None,
-                 ind=0, agent_out=False, match_log=0):
+                 ind=0, agent_out=False, match_log=0, replay=0):
         """``agent_out=True`` turns on the per-agent step outputs (sf_enable_agent_out, read with ``agent_out()``)
         from the first step on.  ``match_log`` > 0 turns on match logs (sf_enable_log, read with ``match_logs()``)
-        with tapes of that many command symbols."""
+        with tapes of that many command symbols.  ``replay`` > 0 turns on replay (sf_enable_replay, loaded with
+        ``replay_load()``) with tapes of that many command symbols."""
         if not torch.cuda.is_available():
             # fail loudly: there is no CPU path (sf_create would report SF_ERR_NO_DEVICE as well)
             raise RuntimeError("strikeforce_b200 needs a CUDA device; it has no CPU fallback")
@@ -49,6 +50,8 @@ class BatchedArena:
             self._chk(lib().sf_enable_agent_out(self._h))
         if match_log:
             self._chk(lib().sf_enable_log(self._h, match_log))
+        if replay:
+            self._chk(lib().sf_enable_replay(self._h, replay))
 
     # ------------------------------------------------------------------ lifetime
     def close(self):
@@ -271,6 +274,37 @@ class BatchedArena:
         assert out.is_cuda and out.dtype == torch.uint8 and out.is_contiguous() and out.numel() == rows * row_bytes
         self._chk(lib().sf_log_list(self._h, C.c_void_p(out.data_ptr()), ids, cnt, rows, self._stream()))
         return out
+
+    def replay_load(self, rows, env_ids, count=None, status=None):
+        """Load replay tapes (sf_replay_load, DESIGN.md section 7i): ``rows`` a uint8 CUDA tensor [n, row_bytes]
+        in the layout ``match_logs()`` exports (``replay.tape_rows`` builds them from .sf_sample logs), ``env_ids``
+        an int32 CUDA tensor [n]; row i resets arena env_ids[i] to the head's seeds, level and episode and arms its
+        tape, and every later step deals the recorded commands from it in place of the action rows.  ``count`` (int32
+        CUDA scalar) limits the live entries; an id outside [0, n_envs) is skipped, a repeated id loads from its
+        lowest entry.  Returns the int32 CUDA ``status`` tensor, the number of refused entries (nothing is loaded
+        unless it is 0), without reading it: no host synchronisation.  Needs ``replay`` at construction."""
+        row_bytes = lib().sf_replay_row_bytes(self._h)
+        n = env_ids.numel()
+        assert rows.is_cuda and rows.dtype == torch.uint8 and rows.is_contiguous() and rows.numel() == n * row_bytes, \
+            "rows: a uint8 CUDA tensor [n, sf_replay_row_bytes]"
+        ids = self._device_list(env_ids, "env_ids")
+        if status is None:
+            status = torch.empty((), dtype=torch.int32, device=self.device)
+        assert status.is_cuda and status.dtype == torch.int32 and status.numel() == 1
+        self._chk(lib().sf_replay_load(self._h, C.c_void_p(rows.data_ptr()), ids, self._device_count(count), n,
+                                       C.c_void_p(status.data_ptr()), self._stream()))
+        return status
+
+    def replay_state(self):
+        """int32 CUDA tensor [n_envs, 5]: the ``config.REPLAY_STATE`` fields (flags cursor n_symbols steps status) of
+        every arena's replay (sf_get(SF_FIELD_REPLAY)); no host synchronisation"""
+        return self._get(sfcfg.FIELD_REPLAY, (self.n_envs, 5), torch.int32)
+
+    def replay_dealt(self):
+        """uint8 CUDA tensor [n_envs, n_agents]: the symbol each human slot took from its arena's tape in the arena's
+        last step, as delivered to obey, 0 where none (sf_get(SF_FIELD_REPLAY_DEALT)) -- the action labels of a
+        replayed step; no host synchronisation"""
+        return self._get(sfcfg.FIELD_REPLAY_DEALT, (self.n_envs, self.n_agents), torch.uint8)
 
     def state_hash(self):
         return self._get(sfcfg.FIELD_STATE_HASH, (self.n_envs,), torch.int64)
